@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 \
            --master-port P bench.py --gpus N --steps K --warmup W     # N GPUs, one rank per GPU (NCCL)
     python bench.py --impl reference --steps 3 --warmup 1             # reference arm: CPU port on the host cores
+    python bench.py --gpus 1 --steps 10 --warmup 3 --dump-outputs D   # + the last timed step's outputs as D/*.npy
 
 A "step" is one training step of the drop-in UniDefenseModelEb4 (EfficientNet-B4, 380x380, per-GPU
 batch 32, bf16 autocast + channels_last for the stock-torch backbone and dense convs, fp32 hot-path kernels)
@@ -529,6 +530,44 @@ def run_microbench(args):
 # ---------------------------------------------------------------------------------------------
 # our arm
 # ---------------------------------------------------------------------------------------------
+DUMP_LIMIT = 64 * 10 ** 6          # bytes of all files written by --dump-outputs together
+
+
+def dump_outputs(outdir, last, params):
+    """Writes what the last timed step computed as <outdir>/<name>.npy (float32; float64 stays float64): the loss, every
+    tensor of the model's output dict (`cls_out`, `rec`, `loss_dict.<key>`, `loss_dict.triplet.<i>`), and the gradients
+    and updated values of the trained parameters, each flattened and concatenated in model.parameters() order.  An
+    array larger than its equal share of DUMP_LIMIT is replaced by the same seeded sample of its flattened elements
+    (sorted indices) on every run, so two builds run with the same arguments can be compared file by file.  Inputs and
+    initial weights are seeded and the step is deterministic (see run_ours), so two runs of one build write the same
+    files."""
+    import numpy as np
+    arrays = {"loss": last["loss"]}
+
+    def add(name, v):
+        if torch.is_tensor(v):
+            arrays[name] = v
+        elif isinstance(v, dict):
+            for k, x in v.items():
+                add(f"{name}.{k}" if name else k, x)
+        elif isinstance(v, (list, tuple)):
+            for i, x in enumerate(v):
+                add(f"{name}.{i}", x)
+    add("", last["out"])
+    arrays["param_grads"] = torch.cat([(p.grad if p.grad is not None else torch.zeros_like(p)).flatten() for p in params])
+    arrays["params"] = torch.cat([p.detach().flatten() for p in params])
+    os.makedirs(outdir, exist_ok=True)
+    share = DUMP_LIMIT // len(arrays) - 4096                  # (room for the .npy header)
+    for name, t in arrays.items():
+        t = t.detach()
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        keep = share // t.element_size()
+        if t.numel() > keep:
+            idx = torch.randint(t.numel(), (keep,), generator=torch.Generator().manual_seed(0)).sort().values
+            t = t.flatten()[idx.to(t.device)]
+        np.save(os.path.join(outdir, f"{name}.npy"), t.cpu().numpy())
+
+
 def run_ours(args):
     world = int(os.environ.get("WORLD_SIZE", "1"))
     rank = int(os.environ.get("RANK", "0"))
@@ -551,7 +590,12 @@ def run_ours(args):
     name, kw, res, nb = ARCH[arch]
     res, nb = args.res or res, args.batch or nb
     torch.manual_seed(0)
-    torch.backends.cudnn.benchmark = True                     # engine/abstract_engine.py:120
+    # Same arguments, same result: the reference engines time cuDNN's algorithms per process (cudnn.benchmark,
+    # engine/abstract_engine.py:120), which picks differently from run to run, and some of those algorithms add with
+    # atomics; either makes two runs of one build train to different weights.  Deterministic algorithms, chosen by
+    # cuDNN's heuristics, make the step bit-reproducible (our kernels reduce in a fixed order).
+    torch.backends.cudnn.benchmark = False
+    torch.backends.cudnn.deterministic = True
     model = init_live(load_model(name)(**kw)).to(dev).train()
     if args.channels_last == "all":
         model = model.to(memory_format=torch.channels_last)
@@ -594,6 +638,9 @@ def run_ours(args):
     nr = nb // 2
     amp = args.dtype == "bf16"
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)     # > 126 MB L2
+    # --dump-outputs: loss and model outputs of the one step recorded (the capture, whose static outputs every replay
+    # rewrites, or the last timed eager step); no other step keeps its outputs alive, so memory use matches a plain run
+    last = {"record": False}
 
     def body(x, labels):
         with torch.autocast("cuda", dtype=torch.bfloat16, enabled=amp):
@@ -607,6 +654,8 @@ def run_ours(args):
         if flat is not None:
             flat.all_reduce()                       # one NCCL all-reduce (avg) of every gradient
         opt.step()
+        if last["record"]:
+            last.update(loss=loss, out=out)
         return loss
 
     def second_pass(x, labels, gt):
@@ -629,6 +678,8 @@ def run_ours(args):
         if flat is not None:
             flat.all_reduce()
         opt.step()
+        if last["record"]:
+            last.update(loss=loss, out=out)
         return loss
 
     def two_pass_step(x, labels):
@@ -683,6 +734,7 @@ def run_ours(args):
                 opt.zero_grad(set_to_none=True)
             l0 = L.lib().ud_launch_count()
             err = None
+            last["record"] = bool(args.dump_outputs)
             try:
                 with torch.cuda.graph(graph, capture_error_mode="thread_local"):
                     if flat is not None:
@@ -690,6 +742,7 @@ def run_ours(args):
                     static_loss = body(x_dev, l_dev)
             except Exception as e:                   # noqa: BLE001
                 err = e
+            last["record"] = False
             graph_launches = L.lib().ud_launch_count() - l0
             if world > 1:                            # every rank replays, or none does (else the collectives dead-lock)
                 flag = torch.tensor([0.0 if err is not None else 1.0], device=dev)
@@ -737,14 +790,19 @@ def run_ours(args):
     launches0 = L.lib().ud_launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(args.steps):
+    for i in range(args.steps):
         flush.zero_()                                          # L2 flush between timed iterations
+        if args.dump_outputs and not graphed and i == args.steps - 1:
+            last["record"] = True
         step(x_dev, l_dev)
     e1.record()
+    last["record"] = False
     barrier()
     launches = graph_launches * args.steps if graphed else L.lib().ud_launch_count() - launches0
     ms = e0.elapsed_time(e1) / args.steps
     clocks = sampler.summary() if sampler is not None else None
+    if args.dump_outputs and rank == 0:          # before the steps below move the weights on
+        dump_outputs(args.dump_outputs, last, params)
     # per-op device times behind `roofline` / `hot_path`: the same step issued eagerly right after the timed region
     # (same inputs, same kernels, L2 flushed), kernel durations taken from CUPTI records; host-recorded events (the
     # round-1 method) are only the fallback because in a host-bound eager stream they include the launch gaps
@@ -928,7 +986,14 @@ def main():
                     help="time the reference's full engine iteration (clean + perturbed pass, config C4) instead of one pass")
     ap.add_argument("--microbench", action="store_true",
                     help="C5 (BASELINE.json configs[4]): frequency-branch sweep R in {224,299,380} x B in {16..256}")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps write what the last one computed to DIR/<name>.npy (seeded inputs: "
+                         "runs with the same arguments compare output for output; at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.microbench or args.recon_only):
+        ap.error("--dump-outputs applies to the timed training step of --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.microbench:

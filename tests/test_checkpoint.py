@@ -1,17 +1,14 @@
 """Checkpoint interchange with the reference engines (SURVEY.md §8f row 4): unidefense_b200.checkpoint.
 
-CPU tests.  The cross-load cases build the LIVE reference classes (tests/golden/ref_loader.py) and are skipped where
-/root/reference does not exist (the GPU box); the self round trip runs everywhere."""
+CPU tests.  The cross-load cases check against the reference classes' state_dict layout recorded in
+tests/golden/full_<arch>.pt."""
 import io
 import os
-import sys
 
 import pytest
 import torch
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-sys.path.insert(0, GOLDEN)
-import ref_loader  # noqa: E402
 
 CTOR = {"r18": ("UDR18", dict(num_classes=2, drop_rate=0.5)),
         "r50": ("UDR50", dict(extractor="resnet50", num_classes=2, drop_rate=0.5)),
@@ -83,32 +80,42 @@ def test_ddp_prefix_bare_state_dict_and_errors():
         CK.load_reference_checkpoint(b, buf)
 
 
-@pytest.mark.skipif(not ref_loader.available(), reason="needs the live reference at /root/reference")
+def _reference_state_dict(arch, seed):
+    """A state_dict laid out as the reference class's: the key order and shapes make_golden.py recorded from it
+    (tests/golden/full_<arch>.pt), BatchNorm counters int64 as torch keeps them, seeded values."""
+    shapes = torch.load(os.path.join(GOLDEN, f"full_{arch}.pt"), weights_only=False)["state_dict_shapes"]
+    g = torch.Generator().manual_seed(seed)
+    sd = {}
+    for k, shape in shapes.items():
+        if k.endswith("num_batches_tracked"):
+            sd[k] = torch.full(shape, seed, dtype=torch.int64)
+        else:
+            sd[k] = torch.randn(shape, generator=g)
+    return sd
+
+
 @pytest.mark.parametrize("arch", ["r18", "r50", "eb4"])
-def test_cross_load_with_the_live_reference_classes(arch, tmp_path):
+def test_cross_load_with_the_reference_layout(arch, tmp_path):
     """A file written the way the reference engine writes it loads strictly into the drop-in, and a file written by
-    the drop-in loads strictly into the reference class (forgery_engine.py:200-209), tensors bit-identical."""
+    the drop-in passes the reference's strict load (forgery_engine.py:200-209: same keys, same shapes), keys in the
+    reference order, tensors bit-identical."""
     from unidefense_b200 import checkpoint as CK
-    ref = ref_loader.load()
-    name, kw = CTOR[arch]
-    kw = dict(kw)
-    torch.manual_seed(11)
-    rmodel = ref.model.load_model(name)(**kw)
-    _randomise(rmodel, 5)
+    ref_sd = _reference_state_dict(arch, 5)
     path = os.path.join(tmp_path, "best_model.bin")
-    torch.save({"step": 12, "best_step": 10, "best_auc": 0.97, "best_acc": 0.93, "model": rmodel.state_dict()}, path)
+    torch.save({"step": 12, "best_step": 10, "best_auc": 0.97, "best_acc": 0.93, "model": ref_sd}, path)
     ours = _ours(arch)
     meta = CK.load_reference_checkpoint(ours, path)
     assert meta["best_step"] == 10
-    for (k, u), (k2, v) in zip(rmodel.state_dict().items(), ours.state_dict().items()):
-        assert k == k2 and u.shape == v.shape and torch.equal(u, v), k
-    assert CK.verify(ours, path)[1] == len(rmodel.state_dict())
-    # and back: the drop-in's file through the reference's own loading code
+    assert list(ours.state_dict()) == list(ref_sd)
+    for (k, u), (k2, v) in zip(ref_sd.items(), ours.state_dict().items()):
+        assert k == k2 and u.shape == v.shape and u.dtype == v.dtype and torch.equal(u, v), k
+    assert CK.verify(ours, path)[1] == len(ref_sd)
+    # and back: the drop-in's file against the reference's strict load_state_dict
     _randomise(ours, 9)
     back = os.path.join(tmp_path, "latest_model.bin")
     CK.save_reference_checkpoint(ours, back, step=13, best_step=10, best_auc=0.97, best_acc=0.93)
     ckpt = torch.load(back, map_location="cpu")
-    rmodel.load_state_dict(ckpt["model"])                                               # strict, as the engine does
-    for u, v in zip(rmodel.state_dict().values(), ours.state_dict().values()):
-        assert torch.equal(u, v)
+    assert list(ckpt["model"]) == list(ref_sd)
+    for (k, u), v in zip(ckpt["model"].items(), ours.state_dict().values()):
+        assert u.shape == ref_sd[k].shape and u.dtype == ref_sd[k].dtype and torch.equal(u, v), k
     assert round(ckpt.get("best_auc", -1), 4) == 0.97                                   # the engine's print statement

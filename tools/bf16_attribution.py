@@ -1,5 +1,6 @@
 import os, sys, torch, torch.nn.functional as F
-sys.path.insert(0, "/root/repo"); sys.path.insert(0, "/root/repo/tests"); sys.path.insert(0, "/root/repo/tests/golden")
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "tests")); sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
 import procedural as P
 F.dropout = lambda t, p=0.5, training=True, inplace=False: t * 1.0
 torch.backends.cudnn.deterministic = True

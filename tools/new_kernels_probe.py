@@ -1,5 +1,5 @@
-import sys, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from unidefense_b200 import ops
 g = torch.Generator().manual_seed(0)
 x = (torch.rand(32, 3, 380, 380, generator=g) * 2 - 1).cuda()
