@@ -18,8 +18,10 @@
  *  - workspaces are passed in by the caller; *_workspace_bytes() say how large.
  *  - the first call for a new FFT length / resize pair builds its table with cudaMalloc + a synchronous copy:
  *    warm every shape up once before capturing calls into a CUDA graph (all later calls are capture-safe).
- *  - reductions are fixed-order (bitwise reproducible) except ud_recon_tail_bwd and ud_bilinear_ac_bwd, whose
- *    transposed resize accumulates with float atomics.
+ *  - reductions are fixed-order (bitwise reproducible) except ud_recon_tail_bwd(2)'s g_dec and ud_bilinear_ac_bwd,
+ *    whose transposed resize accumulates with float atomics.  The input-gradient outputs (g_x of ud_recon_tail_bwd2,
+ *    ud_attn_prep_bwd, ud_gaussian_blur5_bwd, ud_downscale_nearest_bwd; g_diff of ud_dyfi_mask_bwd2) are gathers
+ *    written once per element: bitwise reproducible.
  */
 #ifndef UNIDEFENSE_B200_H
 #define UNIDEFENSE_B200_H
@@ -75,6 +77,14 @@ UD_API int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, float
 UD_API int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
                              const float* g_freq, float* g_dec, void* ws, size_t ws_bytes, int N, int C, int h,
                              int w, int H, int W, int norm_ortho, cudaStream_t stream);
+/* The same backward with the input-image gradient (x is differentiated in the reference: rec - x at
+ * model/unidefense.py:245 and rfft2(x) at :247):
+ *   g_x [N,C,H,W] = -(g_spatial[n]*sign(d)/(C*H*W) + fft_r2c_backward(g_freq[n]*sign(dF)/(C*H*Wh)))   (d = rec - x),
+ * stored at full resolution by the pass that holds it before the transposed resize.  g_dec and g_x are each nullable
+ * (not both); samples with g_spatial[n]==g_freq[n]==0 get g_x = 0.                                                   */
+UD_API int ud_recon_tail_bwd2(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
+                              const float* g_freq, float* g_dec, float* g_x, void* ws, size_t ws_bytes, int N, int C,
+                              int h, int w, int H, int W, int norm_ortho, cudaStream_t stream);
 
 /* ---- a2: decoder epilogues ------------------------------------------------------------------
  * nn.InstanceNorm2d(C, affine) + MemoryEfficientSwish / nn.ReLU after every decoder conv
@@ -116,6 +126,14 @@ UD_API int ud_bilinear_ac_bwd(const float* gy, float* gx, int planes, int h, int
  * to (h,w); spat_diff [N,C,h,w] = |p-xs|; freq_diff [N,2C,h,w/2+1] = |cat(re,im) rfft2(p-xs)|.      */
 UD_API int ud_attn_prep(const float* pred, const float* x, float* spat_diff, float* freq_diff, int N, int C, int hp,
                         int wp, int Hx, int Wx, int h, int w, int norm_ortho, cudaStream_t stream);
+/* Its gradient w.r.t. x (model/unidefense.py:127-134: x is resized and enters p - xs; pred is detached by the caller,
+ * :213/:393/:586): d = down(pred) - down(x) is recomputed at (h,w),
+ *   g_d = sign(d)*g_spat_diff + fft_r2c_backward(sign(cat(re,im) rfft2(d)) * g_freq_diff),
+ *   g_x [N,C,Hx,Wx] = -(transposed align-corners resize)(g_d), evaluated as a gather (no atomics, fully written).
+ * g_spat_diff [N,C,h,w] and g_freq_diff [N,2C,h,w/2+1] are each nullable.  Same shapes as ud_attn_prep; N*C <= 65535. */
+UD_API int ud_attn_prep_bwd(const float* pred, const float* x, const float* g_spat_diff, const float* g_freq_diff,
+                            float* g_x, int N, int C, int hp, int wp, int Hx, int Wx, int h, int w, int norm_ortho,
+                            cudaStream_t stream);
 /* torch.fft.rfft2 + cat([re,im],1) of feature maps (model/unidefense.py:135-136): x [N,C,h,w] ->
  * xf [N,2C,h,w/2+1]; h,w <= 64.  adjoint_of_inverse=1 gives irfft2's backward (fft_c2r_backward:
  * interior columns doubled, inverse normalisation; SURVEY App. B.3).                               */
@@ -199,6 +217,13 @@ UD_API int ud_dyfi_mask_bwd(const float* proj, const float* bn_mean, const float
                             const float* pmean, const float* pmax, const int* argmax, const float* g_mask,
                             const float* g_out, float* g_x, float* dz, float* g_w2, void* ws, size_t ws_bytes, int N,
                             int Cp, int D, int Cx, int HW, int act, cudaStream_t stream);
+/* ud_dyfi_mask_bwd plus g_diff [N,D,HW] (nullable) = w2[2+k] * d loss / d logit: the gradient of the guide channels
+ * cat'ed into layer2's input (model/modules.py:101-103, :130-132), through which the error maps carry x's gradient. */
+UD_API int ud_dyfi_mask_bwd2(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
+                             const float* beta, const float* diff, const float* w2, const float* x, const float* mask,
+                             const float* pmean, const float* pmax, const int* argmax, const float* g_mask,
+                             const float* g_out, float* g_x, float* dz, float* g_w2, float* g_diff, void* ws,
+                             size_t ws_bytes, int N, int Cp, int D, int Cx, int HW, int act, cudaStream_t stream);
 
 /* ---- a9-a11: losses; each also returns d loss / d input for upstream gradient 1 ------------------
  * AsymmetricalWeightedTripletLoss.forward (loss/triplet_loss.py:75-82): feat [N,c], labels int64 [N]
@@ -254,12 +279,18 @@ UD_API size_t ud_coral_workspace_bytes(int N, int HW);
 UD_API int ud_coral(const float* source, const float* target, float* out, void* ws, size_t ws_bytes, int N, int HW,
                     cudaStream_t stream);
 
-/* ---- a16: stencil / resampling perturbations (no grad) ---------------------------------------------
+/* ---- a16: stencil / resampling perturbations ---------------------------------------------------------
  * random_blur (model/modules.py:15-16): torchvision gaussian_blur 5x5, sigma 1.1, reflect padding.   */
 UD_API int ud_gaussian_blur5(const float* x, float* y, int planes, int H, int W, cudaStream_t stream);
 /* downscale (model/modules.py:19-21): nearest by `bottleneck_scale`, then nearest back to HxW.       */
 UD_API int ud_downscale_nearest(const float* x, float* y, int planes, int H, int W, float bottleneck_scale,
                                 cudaStream_t stream);
+/* Their adjoints (torch autograd of model/modules.py:16 and :20-21; pass 2 of training applies them to x):
+ * gx [planes,H,W] from gy [planes,H,W].  Blur: the reflected border taps fold back onto the border pixels;
+ * downscale: each input pixel sums the gradient of its nearest-index preimage (H + W + 2 ints of shared memory). */
+UD_API int ud_gaussian_blur5_bwd(const float* gy, float* gx, int planes, int H, int W, cudaStream_t stream);
+UD_API int ud_downscale_nearest_bwd(const float* gy, float* gx, int planes, int H, int W, float bottleneck_scale,
+                                    cudaStream_t stream);
 
 /* ---- a17 (next row, first step): glue of the SFConv frequency branch ----------------------------------
  * (model/efficientnet/exp.py:55-65, model/resnet/exp.py:44-54).  spec: interleaved complex64 [N,C,P]

@@ -31,6 +31,7 @@ SIGNATURES = {
     "ud_recon_tail_signs_bytes": (c_sz, [c_i] * 4),
     "ud_recon_tail_fwd": (c_i, [c_p] * 7 + [c_sz] + [c_i] * 7 + [c_p]),
     "ud_recon_tail_bwd": (c_i, [c_p] * 7 + [c_sz] + [c_i] * 7 + [c_p]),
+    "ud_recon_tail_bwd2": (c_i, [c_p] * 8 + [c_sz] + [c_i] * 7 + [c_p]),
     "ud_in_act_fwd": (c_i, [c_p] * 7 + [c_i] * 3 + [c_f, c_i, c_p]),
     "ud_in_act_bwd_workspace_bytes": (c_sz, [c_i, c_i]),
     "ud_in_act_bwd": (c_i, [c_p] * 11 + [c_sz] + [c_i] * 4 + [c_p]),
@@ -41,6 +42,7 @@ SIGNATURES = {
     "ud_bilinear_ac_fwd": (c_i, [c_p, c_p] + [c_i] * 5 + [c_p]),
     "ud_bilinear_ac_bwd": (c_i, [c_p, c_p] + [c_i] * 5 + [c_p]),
     "ud_attn_prep": (c_i, [c_p] * 4 + [c_i] * 9 + [c_p]),
+    "ud_attn_prep_bwd": (c_i, [c_p] * 5 + [c_i] * 9 + [c_p]),
     "ud_rfft2_cat": (c_i, [c_p, c_p] + [c_i] * 6 + [c_p]),
     "ud_irfft2_cat": (c_i, [c_p, c_p, c_p] + [c_i] * 6 + [c_p]),
     "ud_rfft2_workspace_bytes": (c_sz, [c_i] * 4),
@@ -63,6 +65,7 @@ SIGNATURES = {
     "ud_dyfi_mask_fwd": (c_i, [c_p] * 13 + [c_i] * 6 + [c_p]),
     "ud_dyfi_mask_bwd_workspace_bytes": (c_sz, [c_i, c_i]),
     "ud_dyfi_mask_bwd": (c_i, [c_p] * 18 + [c_sz] + [c_i] * 6 + [c_p]),
+    "ud_dyfi_mask_bwd2": (c_i, [c_p] * 19 + [c_sz] + [c_i] * 6 + [c_p]),
     "ud_triplet_fwd": (c_i, [c_p] * 4 + [c_i, c_i, c_p]),
     "ud_factorization_workspace_bytes": (c_sz, [c_i, c_i]),
     "ud_factorization_fwd": (c_i, [c_p] * 5 + [c_sz, c_i, c_i, c_f, c_f, c_p]),
@@ -78,6 +81,8 @@ SIGNATURES = {
     "ud_coral": (c_i, [c_p] * 4 + [c_sz, c_i, c_i, c_p]),
     "ud_gaussian_blur5": (c_i, [c_p, c_p, c_i, c_i, c_i, c_p]),
     "ud_downscale_nearest": (c_i, [c_p, c_p, c_i, c_i, c_i, c_f, c_p]),
+    "ud_gaussian_blur5_bwd": (c_i, [c_p, c_p, c_i, c_i, c_i, c_p]),
+    "ud_downscale_nearest_bwd": (c_i, [c_p, c_p, c_i, c_i, c_i, c_f, c_p]),
     "ud_sf_pack": (c_i, [c_p, c_p] + [c_i] * 5 + [c_p]),
     "ud_sf_unpack": (c_i, [c_p, c_p] + [c_i] * 5 + [c_p]),
     "ud_sf_mix_fwd": (c_i, [c_p] * 4 + [c_i] * 5 + [c_p]),

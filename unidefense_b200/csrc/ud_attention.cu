@@ -321,6 +321,20 @@ extern "C" int ud_irfft2_cat(const float* xf, const float* mask, float* y, int N
 }
 
 // ---------------------------------------------------------------- a4: error maps
+// d = down(pred) - down(x) at small-plane pixel (r, cc) for the backward: the expression of at_prep_kernel below, so
+// that the backward sees the forward's fp32 value (and so its signs)
+__device__ __forceinline__ float at_prep_d(const float* __restrict__ pp, const float* __restrict__ xp, int r, int cc,
+                                           int hp, int wp, int Hx, int Wx, float syp, float sxp, float syx, float sxx) {
+  UdLerp yr = ud_lerp_ac(r, hp, syp), xc = ud_lerp_ac(cc, wp, sxp);
+  const float pv = yr.l0 * (xc.l0 * __ldg(pp + yr.i0 * wp + xc.i0) + xc.l1 * __ldg(pp + yr.i0 * wp + xc.i1)) +
+                   yr.l1 * (xc.l0 * __ldg(pp + yr.i1 * wp + xc.i0) + xc.l1 * __ldg(pp + yr.i1 * wp + xc.i1));
+  yr = ud_lerp_ac(r, Hx, syx);
+  xc = ud_lerp_ac(cc, Wx, sxx);
+  const float xv = yr.l0 * (xc.l0 * __ldg(xp + (long long)yr.i0 * Wx + xc.i0) + xc.l1 * __ldg(xp + (long long)yr.i0 * Wx + xc.i1)) +
+                   yr.l1 * (xc.l0 * __ldg(xp + (long long)yr.i1 * Wx + xc.i0) + xc.l1 * __ldg(xp + (long long)yr.i1 * Wx + xc.i1));
+  return pv - xv;
+}
+
 // pred [N,C,hp,wp], x [N,C,Hx,Wx] -> spat_diff [N,C,h,w] = |p - xs|, freq_diff [N,2C,h,wh] = |cat rfft2(p - xs)|
 // (model/unidefense.py:126-134,:148; one FFT by linearity).  One CTA per (n,c) plane.
 __global__ void __launch_bounds__(AT_THREADS)
@@ -375,6 +389,110 @@ extern "C" int ud_attn_prep(const float* pred, const float* x, float* spat_diff,
                                                       ud_ac_scale(hp, h), ud_ac_scale(wp, w), ud_ac_scale(Hx, h),
                                                       ud_ac_scale(Wx, w), at_scale(h, w, norm_ortho, false));
   return ud_check_launch("attn_prep");
+}
+
+// ---------------------------------------------------------------- a4 backward: error maps -> x
+// g_d = sign(d) * g_sd + fft_r2c_backward(sign(F) * g_fd) at (h, w); g_x = -(transposed align-corners resize)(g_d).
+// grid (row tiles of the x plane, N*C planes).  Every CTA recomputes d and the small-plane transforms of its plane
+// (<= 64x64, the same code and thread mapping as at_prep_kernel, so the signs are the forward's), then GATHERS its
+// rows of g_x: output pixel (R, Q) reads the small pixels whose bilinear taps include it, in a fixed order.  g_x is
+// written once, coalesced, without atomics: bitwise reproducible.
+#define AT_BWD_ROWS 8   // x rows per CTA
+
+// small-plane index range [lo, hi] whose align-corners taps (scale s = (in-1)/(out-1), in = big, out = small) can
+// include big index R; the weights are then evaluated exactly with ud_lerp_ac
+__device__ __forceinline__ void at_tap_range(int R, int out, float s, int& lo, int& hi) {
+  if (s <= 0.f) {                     // out == 1 (s = 0): every small index samples big index 0
+    lo = 0;
+    hi = out - 1;
+    return;
+  }
+  lo = max(0, (int)floorf((float)(R - 1) / s) - 1);
+  hi = min(out - 1, (int)ceilf((float)(R + 1) / s) + 1);
+}
+__device__ __forceinline__ float at_tap_weight(int r, int R, int in, float s) {
+  const UdLerp l = ud_lerp_ac(r, in, s);
+  return (l.i0 == R ? l.l0 : 0.f) + (l.i1 == R ? l.l1 : 0.f);
+}
+
+__global__ void __launch_bounds__(AT_THREADS)
+at_prep_bwd_kernel(const float* __restrict__ pred, const float* __restrict__ x, const float* __restrict__ g_sd,
+                   const float* __restrict__ g_fd, float* __restrict__ g_x, int C, int hp, int wp, int Hx, int Wx, int h,
+                   int w, float syp, float sxp, float syx, float sxx, float scale) {
+  extern __shared__ float2 sm2[];
+  const int wh = w / 2 + 1;
+  float2* twW = sm2;
+  float2* twH = twW + w;
+  float* gd = reinterpret_cast<float*>(twH + h);               // d, then g_d [h][w]
+  float2* tmp = reinterpret_cast<float2*>(gd + ((h * w + 1) & ~1));
+  float2* spec = tmp + h * wh;
+  at_fill_tw(twW, w, threadIdx.x, AT_THREADS);
+  at_fill_tw(twH, h, threadIdx.x, AT_THREADS);
+  const int plane = blockIdx.y;
+  const int n = plane / C, c = plane % C;
+  const float* pp = pred + (long long)plane * hp * wp;
+  const float* xp = x + (long long)plane * Hx * Wx;
+  for (int i = threadIdx.x; i < h * w; i += AT_THREADS) {
+    const int r = i / w, cc = i - r * w;
+    gd[i] = at_prep_d(pp, xp, r, cc, hp, wp, Hx, Wx, syp, sxp, syx, sxx);
+  }
+  __syncthreads();
+  const float* gsp = g_sd ? g_sd + (long long)plane * h * w : nullptr;
+  if (g_fd != nullptr) {
+    const float* gre = g_fd + ((long long)n * 2 * C + c) * h * wh;
+    const float* gim = g_fd + ((long long)n * 2 * C + C + c) * h * wh;
+    at_r2c_plane(gd, tmp, twW, twH, h, w, scale, false, threadIdx.x, AT_THREADS, [&](int j, int k, float re, float im) {
+      const int o = j * wh + k;
+      spec[o] = make_float2(ud_sign(re) * __ldg(gre + o), ud_sign(im) * __ldg(gim + o));
+    });
+    __syncthreads();                  // tmp is reused by the inverse
+    at_c2r_plane(spec, tmp, twW, twH, h, w, scale, false, threadIdx.x, AT_THREADS, [&](int r, int cc, float v) {
+      const int i = r * w + cc;
+      gd[i] = gsp ? fmaf(ud_sign(gd[i]), __ldg(gsp + i), v) : v;
+    });
+  } else {
+    for (int i = threadIdx.x; i < h * w; i += AT_THREADS) gd[i] = gsp ? ud_sign(gd[i]) * __ldg(gsp + i) : 0.f;
+  }
+  __syncthreads();
+  float* gxp = g_x + (long long)plane * Hx * Wx;
+  const int R0 = blockIdx.x * AT_BWD_ROWS, R1 = min(Hx, R0 + AT_BWD_ROWS);
+  for (int Q = threadIdx.x; Q < Wx; Q += AT_THREADS) {
+    int clo, chi;
+    at_tap_range(Q, w, sxx, clo, chi);
+    for (int R = R0; R < R1; ++R) {
+      int rlo, rhi;
+      at_tap_range(R, h, syx, rlo, rhi);
+      float acc = 0.f;
+      for (int r = rlo; r <= rhi; ++r) {
+        const float wr = at_tap_weight(r, R, Hx, syx);
+        if (wr == 0.f) continue;
+        float row = 0.f;
+        for (int cc = clo; cc <= chi; ++cc) {
+          const float wc = at_tap_weight(cc, Q, Wx, sxx);
+          if (wc != 0.f) row = fmaf(wc, gd[r * w + cc], row);
+        }
+        acc = fmaf(wr, row, acc);
+      }
+      gxp[(long long)R * Wx + Q] = -acc;
+    }
+  }
+}
+
+extern "C" int ud_attn_prep_bwd(const float* pred, const float* x, const float* g_spat_diff, const float* g_freq_diff,
+                                float* g_x, int N, int C, int hp, int wp, int Hx, int Wx, int h, int w, int norm_ortho,
+                                cudaStream_t stream) {
+  int rc = at_check_small("attn_prep_bwd", N, C, h, w);
+  if (rc != UD_OK) return rc;
+  UD_REQUIRE(hp >= 1 && wp >= 1 && Hx >= 1 && Wx >= 1, UD_ERR_INVALID, "attn_prep_bwd: bad source shape");
+  UD_REQUIRE((long long)N * C <= 65535, UD_ERR_UNSUPPORTED, "attn_prep_bwd: too many planes (%lld)", (long long)N * C);
+  if (N == 0) return UD_OK;
+  UD_REQUIRE(pred && x && g_x, UD_ERR_INVALID, "attn_prep_bwd: null pointer");
+  const size_t smem = sizeof(float2) * (size_t)(w + h) + sizeof(float) * (size_t)at_slot_floats(h, w);
+  if ((rc = at_set_smem(at_prep_bwd_kernel, smem)) != UD_OK) return rc;
+  at_prep_bwd_kernel<<<dim3(ud_cdiv(Hx, AT_BWD_ROWS), N * C), AT_THREADS, smem, stream>>>(
+      pred, x, g_spat_diff, g_freq_diff, g_x, C, hp, wp, Hx, Wx, h, w, ud_ac_scale(hp, h), ud_ac_scale(wp, w),
+      ud_ac_scale(Hx, h), ud_ac_scale(Wx, w), at_scale(h, w, norm_ortho, false));
+  return ud_check_launch("attn_prep_bwd");
 }
 
 // ---------------------------------------------------------------- a7: fuse

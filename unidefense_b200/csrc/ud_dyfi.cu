@@ -210,14 +210,16 @@ extern "C" int ud_dyfi_mask_fwd(const float* proj, const float* bn_mean, const f
 // ---------------------------------------------------------------- fused mask stage, backward
 // d_s = (g_mask + sum_c g_out*x) * m(1-m);  g_x = m*g_out;  g_w2[i] = sum d_s*pre_i;
 // dz[c] = d_s * (w2[0]/Cp + [c==argmax] w2[1]) * act'(z_c)      (grad w.r.t. the BN output)
+// GD: also g_diff[n,k,p] = w2[2+k] * d_s (the guide maps' gradient; nullable).  GD = false is the training path.
+template <bool GD>
 __global__ void __launch_bounds__(DF_GROUPS * 32)
 df_mask_bwd_kernel(const float* __restrict__ proj, const float* __restrict__ bn_mean, const float* __restrict__ bn_rstd,
                    const float* __restrict__ gamma, const float* __restrict__ beta, const float* __restrict__ diff,
                    const float* __restrict__ w2, const float* __restrict__ x, const float* __restrict__ mask,
                    const float* __restrict__ pmean, const float* __restrict__ pmax, const int* __restrict__ argmax,
                    const float* __restrict__ g_mask, const float* __restrict__ g_out, float* __restrict__ g_x,
-                   float* __restrict__ dz, float* __restrict__ w2_part, int Cp, int D, int Cx, int HW, int tiles,
-                   int act) {
+                   float* __restrict__ dz, float* __restrict__ w2_part, float* __restrict__ g_diff, int Cp, int D,
+                   int Cx, int HW, int tiles, int act) {
   __shared__ float s_t[DF_GROUPS][33];
   __shared__ float s_ds[32];
   const int n = blockIdx.x / tiles, tile = blockIdx.x % tiles;
@@ -272,6 +274,9 @@ df_mask_bwd_kernel(const float* __restrict__ proj, const float* __restrict__ bn_
       v = ud_warp_sum(v);
       if (lane == 0) w2_part[(long long)blockIdx.x * DF_MAX_PRE + i] = v;
     }
+    if (GD && g_diff != nullptr && live) {
+      for (int k = 0; k < D; ++k) g_diff[((long long)n * D + k) * HW + pos] = __ldg(w2 + 2 + k) * ds;
+    }
   }
 }
 
@@ -288,11 +293,11 @@ extern "C" size_t ud_dyfi_mask_bwd_workspace_bytes(int N, int HW) {
   return sizeof(float) * (size_t)N * ud_cdiv(HW, 32) * DF_MAX_PRE;
 }
 
-extern "C" int ud_dyfi_mask_bwd(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
-                                const float* beta, const float* diff, const float* w2, const float* x,
-                                const float* mask, const float* pmean, const float* pmax, const int* argmax,
-                                const float* g_mask, const float* g_out, float* g_x, float* dz, float* g_w2, void* ws,
-                                size_t ws_bytes, int N, int Cp, int D, int Cx, int HW, int act, cudaStream_t stream) {
+static int df_mask_bwd(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
+                       const float* beta, const float* diff, const float* w2, const float* x, const float* mask,
+                       const float* pmean, const float* pmax, const int* argmax, const float* g_mask, const float* g_out,
+                       float* g_x, float* dz, float* g_w2, float* g_diff, void* ws, size_t ws_bytes, int N, int Cp, int D,
+                       int Cx, int HW, int act, cudaStream_t stream) {
   UD_REQUIRE(N >= 0 && Cp >= 1 && D >= 0 && Cx >= 1 && HW >= 1 && 2 + D <= DF_MAX_PRE, UD_ERR_INVALID,
              "dyfi_mask_bwd: bad shape");
   UD_REQUIRE(g_w2, UD_ERR_INVALID, "dyfi_mask_bwd: null pointer");
@@ -306,10 +311,30 @@ extern "C" int ud_dyfi_mask_bwd(const float* proj, const float* bn_mean, const f
   UD_REQUIRE(ws_bytes >= ud_dyfi_mask_bwd_workspace_bytes(N, HW), UD_ERR_WORKSPACE, "dyfi_mask_bwd: workspace too small");
   const int tiles = ud_cdiv(HW, 32);
   float* part = static_cast<float*>(ws);
-  df_mask_bwd_kernel<<<N * tiles, DF_GROUPS * 32, 0, stream>>>(proj, bn_mean, bn_rstd, gamma, beta, diff, w2, x, mask, pmean, pmax,
-                                                    argmax, g_mask, g_out, g_x, dz, part, Cp, D, Cx, HW, tiles, act);
+  auto k = g_diff ? df_mask_bwd_kernel<true> : df_mask_bwd_kernel<false>;
+  k<<<N * tiles, DF_GROUPS * 32, 0, stream>>>(proj, bn_mean, bn_rstd, gamma, beta, diff, w2, x, mask, pmean, pmax, argmax,
+                                              g_mask, g_out, g_x, dz, part, g_diff, Cp, D, Cx, HW, tiles, act);
   int rc = ud_check_launch("dyfi_mask_bwd");
   if (rc != UD_OK) return rc;
   df_w2_reduce_kernel<<<2 + D, 128, 0, stream>>>(part, g_w2, N * tiles, 2 + D);
   return ud_check_launch("dyfi_w2_reduce");
+}
+
+extern "C" int ud_dyfi_mask_bwd(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
+                                const float* beta, const float* diff, const float* w2, const float* x,
+                                const float* mask, const float* pmean, const float* pmax, const int* argmax,
+                                const float* g_mask, const float* g_out, float* g_x, float* dz, float* g_w2, void* ws,
+                                size_t ws_bytes, int N, int Cp, int D, int Cx, int HW, int act, cudaStream_t stream) {
+  return df_mask_bwd(proj, bn_mean, bn_rstd, gamma, beta, diff, w2, x, mask, pmean, pmax, argmax, g_mask, g_out, g_x, dz,
+                     g_w2, nullptr, ws, ws_bytes, N, Cp, D, Cx, HW, act, stream);
+}
+
+extern "C" int ud_dyfi_mask_bwd2(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
+                                 const float* beta, const float* diff, const float* w2, const float* x,
+                                 const float* mask, const float* pmean, const float* pmax, const int* argmax,
+                                 const float* g_mask, const float* g_out, float* g_x, float* dz, float* g_w2,
+                                 float* g_diff, void* ws, size_t ws_bytes, int N, int Cp, int D, int Cx, int HW, int act,
+                                 cudaStream_t stream) {
+  return df_mask_bwd(proj, bn_mean, bn_rstd, gamma, beta, diff, w2, x, mask, pmean, pmax, argmax, g_mask, g_out, g_x, dz,
+                     g_w2, D > 0 ? g_diff : nullptr, ws, ws_bytes, N, Cp, D, Cx, HW, act, stream);
 }

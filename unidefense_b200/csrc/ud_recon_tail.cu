@@ -30,7 +30,7 @@ size_t ud_rt2_workspace_plane_bytes(int H, int W);
 int ud_rt2_fwd(const float* dec, const float* x, float* rec, float2* Z, float* part_sp, float* part_fr, uint8_t* signs,
                int plane0, int planes, int h, int w, int H, int W, int row_tiles, int col_tiles, cudaStream_t stream);
 int ud_rt2_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial, const float* g_freq,
-               float* g_dec, float2* T, int plane0, int planes, int C, int h, int w, int H, int W, int row_tiles,
+               float* g_dec, float* g_x, float2* T, int plane0, int planes, int C, int h, int w, int H, int W, int row_tiles,
                int col_tiles, float gscale, float sp_scale, cudaStream_t stream);
 // row pairs per rows-CTA of ud_recon_tail2.cu = its RT2_LPC (16) x the steps a CTA walks.  Measured at N=32, 380^2: one
 // step per CTA (12 row tiles per plane, ~4 waves) and two (6 tiles, ~2 waves) take the same time (101 / 89 us fwd / bwd),
@@ -330,12 +330,14 @@ rt_cols_bwd_kernel(Plan plan, const uint8_t* __restrict__ signs, const float* __
 // first (gather through xtab, both rows of a pair at once, results staged in registers and written back
 // over the line), then vertically: one thread per dec column walks the tile's rows in order carrying two
 // running sums (rows i and i+1) and flushes each finished dec row with one atomicAdd.
+// GX: also g_x = -g_rec at full resolution from the finished lines (zeros for planes whose sample has gs == gf == 0);
+// g_dec may then be NULL.  GX = false is the training path.
 // ------------------------------------------------------------------------------------------
-template <class Plan>
+template <class Plan, bool GX>
 __global__ void __launch_bounds__(RT_ROW_T)
 rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __restrict__ x,
                    const float2* __restrict__ T, const float* __restrict__ g_spatial,
-                   const float* __restrict__ g_freq, float* __restrict__ g_dec,
+                   const float* __restrict__ g_freq, float* __restrict__ g_dec, float* __restrict__ g_x,
                    const float2* __restrict__ tw_g, const float2* __restrict__ ytab_g,
                    const float2* __restrict__ xtab_g, const int2* __restrict__ jtab_g, int plane0, int C, int h,
                    int w, int H, int W, float sp_scale) {
@@ -355,8 +357,15 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
   const int smp = (int)(plane / C);
   const float gs = g_spatial[smp] * sp_scale;
   const bool has_f = g_freq[smp] != 0.f;
-  if (gs == 0.f && !has_f) return;
   const int r0 = tile * (2 * RT_ROW_L);
+  if (gs == 0.f && !has_f) {
+    if (GX) {                            // the tile's rows of g_x are zero
+      float* gxp = g_x + plane * (long long)H * n;
+      const long long e = (long long)min(H, r0 + 2 * RT_ROW_L) * n;
+      for (long long i = (long long)r0 * n + threadIdx.x; i < e; i += RT_ROW_T) gxp[i] = 0.f;
+    }
+    return;
+  }
   W = n;
   const int Wh = n / 2 + 1;
   const int WhP = (Wh + 15) & ~15;
@@ -461,6 +470,15 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
     __syncthreads();
   }
 
+  if (GX) {                              // g_x = -g_rec; res[p][c] = (g_b[c], g_a[c])
+    float* gxp = g_x + (plane * H + r0) * (long long)n;
+    for (int t = threadIdx.x; t < nrows * n; t += RT_ROW_T) {
+      const int rr = t / n, c = t - rr * n;
+      const float2 g2 = res[(rr >> 1) * LS + c];
+      __stcs(gxp + t, (rr & 1) ? -g2.x : -g2.y);
+    }
+    if (g_dec == nullptr) return;        // g_x only: no transposed resize
+  }
   float* gd = g_dec + plane * (long long)h * w;
   const int items = RT_ROW_L * w;
   if (items <= RT_HSTAGE * RT_ROW_T && w <= n) {   // staged results are written back over the line (n slots)
@@ -690,13 +708,14 @@ extern "C" int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, f
   return ud_check_launch("rt_finalize");
 }
 
-extern "C" int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
-                                 const float* g_freq, float* g_dec, void* ws, size_t ws_bytes, int N, int C,
-                                 int h, int w, int H, int W, int norm_ortho, cudaStream_t stream) {
+// g_dec and g_x are each nullable (not both): ud_recon_tail_bwd passes g_x = NULL, which selects the GX = false kernels
+static int rt_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial, const float* g_freq,
+                  float* g_dec, float* g_x, void* ws, size_t ws_bytes, int N, int C, int h, int w, int H, int W,
+                  int norm_ortho, cudaStream_t stream) {
   int rc = rt_validate(N, C, h, w, H, W);
   if (rc != UD_OK) return rc;
   if (N == 0) return UD_OK;
-  UD_REQUIRE(dec && x && signs && g_spatial && g_freq && g_dec && ws, UD_ERR_INVALID,
+  UD_REQUIRE(dec && x && signs && g_spatial && g_freq && (g_dec || g_x) && ws, UD_ERR_INVALID,
              "recon_tail_bwd: null pointer");
   UD_REQUIRE(ws_bytes >= ud_recon_tail_workspace_bytes(N, C, h, w, H, W), UD_ERR_WORKSPACE,
              "recon_tail_bwd: workspace too small");
@@ -722,12 +741,12 @@ extern "C" int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t
   const float nrm = norm_ortho ? 1.f / sqrtf((float)H * (float)W) : 1.f;
   const float gscale = nrm / ((float)C * H * Wh);
   const float sp_scale = 1.f / ((float)C * H * W);
-  UD_CUDA(cudaMemsetAsync(g_dec, 0, sizeof(float) * (size_t)N * C * h * w, stream));
+  if (g_dec) UD_CUDA(cudaMemsetAsync(g_dec, 0, sizeof(float) * (size_t)N * C * h * w, stream));
   for (int s0 = 0; s0 < N; s0 += chunk) {
     const int ns = (N - s0 < chunk) ? (N - s0) : chunk;
     const int planes = ns * C, plane0 = s0 * C;
     if (v2) {
-      if ((rc = ud_rt2_bwd(dec, x, signs, g_spatial, g_freq, g_dec, T, plane0, planes, C, h, w, H, W, row_tiles, col_tiles,
+      if ((rc = ud_rt2_bwd(dec, x, signs, g_spatial, g_freq, g_dec, g_x, T, plane0, planes, C, h, w, H, W, row_tiles, col_tiles,
                            gscale, sp_scale, stream)) != UD_OK) return rc;
       continue;
     }
@@ -738,12 +757,25 @@ extern "C" int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t
     });
     if ((rc = ud_check_launch("rt_cols_bwd")) != UD_OK) return rc;
     RT_DISPATCH_PLAN(W, RT_ROW_L, RT_ROW_T, plan, {
-      auto k = rt_rows_bwd_kernel<decltype(plan)>;
+      auto k = g_x ? rt_rows_bwd_kernel<decltype(plan), true> : rt_rows_bwd_kernel<decltype(plan), false>;
       if ((rc = rt_set_smem(k, smW)) != UD_OK) return rc;
-      k<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(plan, dec, x, T, g_spatial, g_freq, g_dec, twW, ytab,
+      k<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(plan, dec, x, T, g_spatial, g_freq, g_dec, g_x, twW, ytab,
                                                              xtab, jtab, plane0, C, h, w, H, W, sp_scale);
     });
     if ((rc = ud_check_launch("rt_rows_bwd")) != UD_OK) return rc;
   }
   return UD_OK;
+}
+
+extern "C" int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
+                                 const float* g_freq, float* g_dec, void* ws, size_t ws_bytes, int N, int C,
+                                 int h, int w, int H, int W, int norm_ortho, cudaStream_t stream) {
+  UD_REQUIRE(N == 0 || g_dec, UD_ERR_INVALID, "recon_tail_bwd: null pointer");
+  return rt_bwd(dec, x, signs, g_spatial, g_freq, g_dec, nullptr, ws, ws_bytes, N, C, h, w, H, W, norm_ortho, stream);
+}
+
+extern "C" int ud_recon_tail_bwd2(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
+                                  const float* g_freq, float* g_dec, float* g_x, void* ws, size_t ws_bytes, int N, int C,
+                                  int h, int w, int H, int W, int norm_ortho, cudaStream_t stream) {
+  return rt_bwd(dec, x, signs, g_spatial, g_freq, g_dec, g_x, ws, ws_bytes, N, C, h, w, H, W, norm_ortho, stream);
 }

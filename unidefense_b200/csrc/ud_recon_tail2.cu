@@ -305,14 +305,17 @@ rt2_cols_bwd_kernel(const uint8_t* __restrict__ signs, const float* __restrict__
 // ------------------------------------------------------------------------------------------
 // backward rows: grid (row_tiles, planes_in_chunk)
 //   g_rec[r,c] = gs*sign(d[r,c]) + Re sum_{k<Wh} T[r,k] e^{+2 pi i k c / W}; transposed bilinear into g_dec.
+//   GX: also g_x = -g_rec at full resolution, straight from the registers that hold g_rec (zeros for planes whose
+//   sample has gs == gf == 0); g_dec may then be NULL (no transposed resize).  GX = false is the training path.
 //   shared: tw2[R1*P] | xtab[N] | S[LPC*LS] | V[LPC*w] (aliased by Hb[2*LPC][w] floats)
 // ------------------------------------------------------------------------------------------
-template <class PL>
+template <class PL, bool GX>
 __global__ void __launch_bounds__(PL::TL* RT2_RLPC, 2)
 rt2_rows_bwd_kernel(const float* __restrict__ dec, const float* __restrict__ x, const float2* __restrict__ T,
                     const float* __restrict__ g_spatial, const float* __restrict__ g_freq, float* __restrict__ g_dec,
-                    const float2* __restrict__ tw_g, const float2* __restrict__ ytab_g, const float2* __restrict__ xtab_g,
-                    const int2* __restrict__ jtab_g, int plane0, int C, int h, int w, int H, float sp_scale, int iters) {
+                    float* __restrict__ g_x, const float2* __restrict__ tw_g, const float2* __restrict__ ytab_g,
+                    const float2* __restrict__ xtab_g, const int2* __restrict__ jtab_g, int plane0, int C, int h, int w,
+                    int H, float sp_scale, int iters) {
   constexpr int N = PL::N, R1 = PL::R1, R2 = PL::R2, TL = PL::TL, P = PL::P, LS = PL::LS;
   constexpr int NT = TL * RT2_RLPC;
   extern __shared__ float2 smem[];
@@ -327,11 +330,18 @@ rt2_rows_bwd_kernel(const float* __restrict__ dec, const float* __restrict__ x, 
   const int smp = (int)(plane / C);
   const float gs = __ldg(g_spatial + smp) * sp_scale;
   const bool has_f = __ldg(g_freq + smp) != 0.f;
-  if (gs == 0.f && !has_f) return;
   const int Hp = (H + 1) >> 1;
+  const int pair0 = blockIdx.x * (RT2_RLPC * iters);
+  if (gs == 0.f && !has_f) {
+    if (GX) {                              // the tile's rows of g_x are zero
+      const int r0 = 2 * pair0, r1 = min(H, 2 * (pair0 + RT2_RLPC * iters));
+      float* gxp = g_x + plane * (long long)H * N;
+      for (long long i = (long long)r0 * N + tid; i < (long long)r1 * N; i += NT) gxp[i] = 0.f;
+    }
+    return;
+  }
   const int Wh = N / 2 + 1;
   const int WhP = (Wh + 15) & ~15;
-  const int pair0 = blockIdx.x * (RT2_RLPC * iters);
 
   ud2s_build_tw<PL>(tw2, tw_g);
   for (int t = tid; t < N; t += NT) xtab[t] = __ldg(xtab_g + t);
@@ -399,7 +409,17 @@ rt2_rows_bwd_kernel(const float* __restrict__ dec, const float* __restrict__ x, 
         }
       }
     }
+    if (GX && live && ln < R1) {           // g_x = -g_rec: u[k2] = (g_b[c], g_a[c])
+      float* qa = g_x + (plane * H + ra) * (long long)N;
+#pragma unroll
+      for (int k2 = 0; k2 < R2; ++k2) {
+        const int c = ln + R1 * k2;
+        __stcs(qa + c, -u[k2].y);
+        if (has_b) __stcs(qa + N + c, -u[k2].x);
+      }
+    }
     __syncthreads();                       // all reads of S (stage B) and V (signs) done
+    if (GX && g_dec == nullptr) continue;  // g_x only: no transposed resize
     if (ln < R1) {
       float2* Gg = S + g * LS;             // G[c] = (g_b[c], g_a[c]); dead lines hold zeros
 #pragma unroll
@@ -446,6 +466,7 @@ rt2_rows_bwd_kernel(const float* __restrict__ dec, const float* __restrict__ x, 
     }
     __syncthreads();                       // Hb (== V) and S are rewritten by the next step
   }
+  if (GX && g_dec == nullptr) return;
   if (tid < w) {
     if (acc0 != 0.f) atomicAdd(gd + (long long)cur * w + tid, acc0);
     if (acc1 != 0.f && cur + 1 < h) atomicAdd(gd + (long long)(cur + 1) * w + tid, acc1);
@@ -519,7 +540,7 @@ int ud_rt2_fwd(const float* dec, const float* x, float* rec, float2* Z, float* p
 }
 
 int ud_rt2_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial, const float* g_freq,
-               float* g_dec, float2* T, int plane0, int planes, int C, int h, int w, int H, int W, int row_tiles,
+               float* g_dec, float* g_x, float2* T, int plane0, int planes, int C, int h, int w, int H, int W, int row_tiles,
                int col_tiles, float gscale, float sp_scale, cudaStream_t stream) {
   const float2* twW = ud_twiddles(W);
   const float2* twH = ud_twiddles(H);
@@ -537,11 +558,12 @@ int ud_rt2_bwd(const float* dec, const float* x, const uint8_t* signs, const flo
   });
   if ((rc = ud_check_launch("rt2_cols_bwd")) != UD_OK) return rc;
   RT2_DISPATCH(W, PLW, {
-    auto k = rt2_rows_bwd_kernel<PLW>;
+    auto k = g_x ? rt2_rows_bwd_kernel<PLW, true> : rt2_rows_bwd_kernel<PLW, false>;
     const size_t sm = sizeof(float2) * ((size_t)PLW::R1 * PLW::P + W + (size_t)RT2_RLPC * PLW::LS + (size_t)RT2_RLPC * w);
     if ((rc = rt2_set_smem(k, sm)) != UD_OK) return rc;
-    k<<<dim3(row_tiles, planes), PLW::TL * RT2_RLPC, sm, stream>>>(dec, x, T, g_spatial, g_freq, g_dec, twW, ytab, xtab,
-                                                                    jtab, plane0, C, h, w, H, sp_scale, rt2_iters(H, row_tiles));
+    k<<<dim3(row_tiles, planes), PLW::TL * RT2_RLPC, sm, stream>>>(dec, x, T, g_spatial, g_freq, g_dec, g_x, twW, ytab,
+                                                                    xtab, jtab, plane0, C, h, w, H, sp_scale,
+                                                                    rt2_iters(H, row_tiles));
   });
   return ud_check_launch("rt2_rows_bwd");
 }

@@ -1,9 +1,10 @@
-"""Input perturbations of the second training pass (no grad)      (SURVEY.md §8a rows a13-a16).
+"""Input perturbations of the second training pass               (SURVEY.md §8a rows a13-a16).
 
 Reference: model/modules.py:7-21 (random_noise, random_blur, downscale), :35-76
 (FrequencyStyleTransfer, SpatialStyleTransfer) and utils/operation.py:15-45 (coral).  Control-flow
 randomness comes from torch's CPU generator exactly as in the reference (Appendix D) so that a
-shared seed reproduces the same augmentation choices.
+shared seed reproduces the same augmentation choices.  random_noise, random_blur and downscale pass the gradient
+on to the input as in the reference; the style transfers and coral run under no_grad there and here.
 """
 import torch
 

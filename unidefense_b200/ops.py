@@ -16,7 +16,8 @@ def norm_flag(norm):
 
 
 class _ReconTail(torch.autograd.Function):
-    """a1: model/unidefense.py:244-253 / :423-433 / :618-628."""
+    """a1: model/unidefense.py:244-253 / :423-433 / :618-628.  Differentiable in dec and in x (rec - x and rfft2(x) are
+    differentiated in the reference); the x gradient is only computed when x requires one."""
 
     @staticmethod
     def forward(ctx, dec, x, norm_ortho):
@@ -31,7 +32,7 @@ class _ReconTail(torch.autograd.Function):
         rec = torch.empty_like(x)
         spatial = torch.empty(N, device=x.device, dtype=torch.float32)
         freq = torch.empty(N, device=x.device, dtype=torch.float32)
-        need_grad = ctx.needs_input_grad[0]
+        need_grad = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
         signs = (torch.empty(lib.ud_recon_tail_signs_bytes(N, C, H, W), dtype=torch.uint8, device=x.device)
                  if need_grad else None)
         nws = lib.ud_recon_tail_workspace_bytes(N, C, h, w, H, W)
@@ -51,28 +52,35 @@ class _ReconTail(torch.autograd.Function):
         N, C, h, w = dec.shape
         H, W = x.shape[-2:]
         lib = L.lib()
-        g_dec = None
+        need_dec, need_x = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        g_dec = g_x = None
         if g_spatial is not None or g_freq is not None:
             gs = (g_spatial if g_spatial is not None else torch.zeros(N, device=x.device)).contiguous().float()
             gf = (g_freq if g_freq is not None else torch.zeros(N, device=x.device)).contiguous().float()
-            g_dec = torch.empty_like(dec)
+            g_dec = torch.empty_like(dec) if need_dec else None
             nws = lib.ud_recon_tail_workspace_bytes(N, C, h, w, H, W)
             ws = L.workspace(nws, x.device)
-            L.check(lib.ud_recon_tail_bwd(L.ptr(dec), L.ptr(x), L.ptr(signs), L.ptr(gs), L.ptr(gf), L.ptr(g_dec),
-                                          L.ptr(ws), ws.numel(), N, C, h, w, H, W, ctx.norm_ortho, L.stream()),
-                    "recon_tail_bwd")
-        if g_rec is not None:
+            if need_x:
+                g_x = torch.empty_like(x)
+                L.check(lib.ud_recon_tail_bwd2(L.ptr(dec), L.ptr(x), L.ptr(signs), L.ptr(gs), L.ptr(gf), L.ptr(g_dec),
+                                               L.ptr(g_x), L.ptr(ws), ws.numel(), N, C, h, w, H, W, ctx.norm_ortho,
+                                               L.stream()), "recon_tail_bwd2")
+            else:
+                L.check(lib.ud_recon_tail_bwd(L.ptr(dec), L.ptr(x), L.ptr(signs), L.ptr(gs), L.ptr(gf), L.ptr(g_dec),
+                                              L.ptr(ws), ws.numel(), N, C, h, w, H, W, ctx.norm_ortho, L.stream()),
+                        "recon_tail_bwd")
+        if g_rec is not None and need_dec:
             # rec = interpolate(dec) is differentiable in the reference (model/unidefense.py:244); the shipped engines
             # never use that gradient, but a loss on out['rec'] gets the transposed resize, not silent zeros
             g_up = torch.empty_like(dec)
             L.check(lib.ud_bilinear_ac_bwd(L.ptr(g_rec.contiguous().float()), L.ptr(g_up), N * C, h, w, H, W, L.stream()),
                     "bilinear_bwd")
             g_dec = g_up if g_dec is None else g_dec + g_up
-        return g_dec, None, None
+        return g_dec, g_x, None
 
 
 def recon_tail(dec, x, norm="ortho"):
-    """-> (rec [N,C,H,W], spatial [N], freq [N]), all differentiable w.r.t. dec (x is data)."""
+    """-> (rec [N,C,H,W], spatial [N], freq [N]); rec is differentiable w.r.t. dec, spatial and freq w.r.t. dec and x."""
     return _ReconTail.apply(dec, x, norm_flag(norm))
 
 
@@ -186,18 +194,46 @@ def bilinear_ac(x, size):
     return _BilinearAC.apply(x, int(size[0]), int(size[1]))
 
 
+class _AttnPrep(torch.autograd.Function):
+    """Error maps (model/unidefense.py:126-134,:148).  Differentiable in x only: the reference passes pred detached
+    (dec_out.clone().detach(), :213 / :393 / :586), so no gradient is ever returned for it."""
+
+    @staticmethod
+    def forward(ctx, pred, x, h, w, norm_ortho):
+        pred = pred.detach().contiguous()
+        x = x.detach().contiguous()
+        L.require_cuda_f32(pred, x)
+        N, C = x.shape[:2]
+        sd = torch.empty(N, C, h, w, device=x.device, dtype=torch.float32)
+        fd = torch.empty(N, 2 * C, h, w // 2 + 1, device=x.device, dtype=torch.float32)
+        L.check(L.lib().ud_attn_prep(L.ptr(pred), L.ptr(x), L.ptr(sd), L.ptr(fd), N, C, pred.shape[-2], pred.shape[-1],
+                                     x.shape[-2], x.shape[-1], h, w, norm_ortho, L.stream()), "attn_prep")
+        if ctx.needs_input_grad[1]:
+            ctx.save_for_backward(pred, x)
+        ctx.hw = (h, w)
+        ctx.norm_ortho = norm_ortho
+        ctx.set_materialize_grads(False)
+        return sd, fd
+
+    @staticmethod
+    def backward(ctx, g_sd, g_fd):
+        if not ctx.needs_input_grad[1] or (g_sd is None and g_fd is None):
+            return None, None, None, None, None
+        pred, x = ctx.saved_tensors
+        N, C = x.shape[:2]
+        h, w = ctx.hw
+        g_sd = None if g_sd is None else g_sd.contiguous()
+        g_fd = None if g_fd is None else g_fd.contiguous()
+        g_x = torch.empty_like(x)
+        L.check(L.lib().ud_attn_prep_bwd(L.ptr(pred), L.ptr(x), L.ptr(g_sd), L.ptr(g_fd), L.ptr(g_x), N, C,
+                                         pred.shape[-2], pred.shape[-1], x.shape[-2], x.shape[-1], h, w, ctx.norm_ortho,
+                                         L.stream()), "attn_prep_bwd")
+        return None, g_x, None, None, None
+
+
 def attn_prep(pred, x, size, norm="ortho"):
-    """Error maps (no grad; model/unidefense.py:126-134,:148) -> (spat_diff [N,C,h,w], freq_diff [N,2C,h,w/2+1])."""
-    pred = pred.detach().contiguous()
-    x = x.detach().contiguous()
-    L.require_cuda_f32(pred, x)
-    N, C = x.shape[:2]
-    h, w = int(size[0]), int(size[1])
-    sd = torch.empty(N, C, h, w, device=x.device, dtype=torch.float32)
-    fd = torch.empty(N, 2 * C, h, w // 2 + 1, device=x.device, dtype=torch.float32)
-    L.check(L.lib().ud_attn_prep(L.ptr(pred), L.ptr(x), L.ptr(sd), L.ptr(fd), N, C, pred.shape[-2], pred.shape[-1],
-                                 x.shape[-2], x.shape[-1], h, w, norm_flag(norm), L.stream()), "attn_prep")
-    return sd, fd
+    """Error maps -> (spat_diff [N,C,h,w], freq_diff [N,2C,h,w/2+1]); differentiable w.r.t. x (pred is data)."""
+    return _AttnPrep.apply(pred, x, int(size[0]), int(size[1]), norm_flag(norm))
 
 
 def _rfft2_raw(x, norm_ortho, adjoint):
@@ -501,10 +537,18 @@ class _DyfiMask(torch.autograd.Function):
         dz = torch.empty_like(proj)
         g_w2 = torch.empty(2 + D, device=dev, dtype=torch.float32)
         ws = L.workspace(lib.ud_dyfi_mask_bwd_workspace_bytes(N, HW), dev)
-        L.check(lib.ud_dyfi_mask_bwd(L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(gamma), L.ptr(beta), L.ptr(diff),
-                                     L.ptr(w2f), L.ptr(x), L.ptr(mask), L.ptr(pmean), L.ptr(pmax), L.ptr(argmax),
-                                     L.ptr(g_mask), L.ptr(g_out), L.ptr(g_x), L.ptr(dz), L.ptr(g_w2), L.ptr(ws),
-                                     ws.numel(), N, Cp, D, Cx, HW, ctx.act, L.stream()), "dyfi_mask_bwd")
+        g_diff = None
+        if ctx.needs_input_grad[5]:          # the error maps carry x's gradient (model/modules.py:101-103, :130-132)
+            g_diff = torch.empty_like(diff)
+            L.check(lib.ud_dyfi_mask_bwd2(L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(gamma), L.ptr(beta), L.ptr(diff),
+                                          L.ptr(w2f), L.ptr(x), L.ptr(mask), L.ptr(pmean), L.ptr(pmax), L.ptr(argmax),
+                                          L.ptr(g_mask), L.ptr(g_out), L.ptr(g_x), L.ptr(dz), L.ptr(g_w2), L.ptr(g_diff),
+                                          L.ptr(ws), ws.numel(), N, Cp, D, Cx, HW, ctx.act, L.stream()), "dyfi_mask_bwd2")
+        else:
+            L.check(lib.ud_dyfi_mask_bwd(L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(gamma), L.ptr(beta), L.ptr(diff),
+                                         L.ptr(w2f), L.ptr(x), L.ptr(mask), L.ptr(pmean), L.ptr(pmax), L.ptr(argmax),
+                                         L.ptr(g_mask), L.ptr(g_out), L.ptr(g_x), L.ptr(dz), L.ptr(g_w2), L.ptr(ws),
+                                         ws.numel(), N, Cp, D, Cx, HW, ctx.act, L.stream()), "dyfi_mask_bwd")
         sums = torch.empty(2, Cp, device=dev, dtype=torch.float32)
         L.check(lib.ud_bn_bwd_reduce(L.ptr(dz), L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(sums[0]), L.ptr(sums[1]),
                                      N, Cp, HW, L.stream()), "bn_bwd_reduce")
@@ -522,7 +566,7 @@ class _DyfiMask(torch.autograd.Function):
         L.check(lib.ud_bn_bwd_apply(L.ptr(dz), L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(gamma), L.ptr(sums[0]),
                                     L.ptr(sums[1]), inv_count, L.ptr(g_proj), N, Cp, HW, L.stream()), "bn_bwd_apply")
         return (g_proj, None, None, g_gamma if gamma is not None else None, g_beta if beta is not None else None,
-                None, g_w2.reshape(ctx.w2_shape), g_x, None, None, None, None)
+                g_diff, g_w2.reshape(ctx.w2_shape), g_x, None, None, None, None)
 
 
 def dyfi_mask(proj, mean, rstd, gamma, beta, diff, w2, x, act="swish", count=0, want_out=True, stat_reduce=None):
@@ -674,27 +718,63 @@ def bce_with_logits(logits, target):
 
 
 # ------------------------------------------------------------------------------------------
-# a13-a16: perturbations (no grad)
+# a13-a16: perturbations (blur and downscale are differentiable, as in the reference; the style transfers and coral
+# run under no_grad there, model/unidefense.py:181-193, and here)
 # ------------------------------------------------------------------------------------------
+class _Blur5(torch.autograd.Function):
+    """random_blur (model/modules.py:15-16); backward = the adjoint 5x5 stencil with the reflected taps folded back."""
+
+    @staticmethod
+    def forward(ctx, x):
+        x = x.detach().contiguous()
+        L.require_cuda_f32(x)
+        H, W = x.shape[-2:]
+        y = torch.empty_like(x)
+        L.check(L.lib().ud_gaussian_blur5(L.ptr(x), L.ptr(y), x.numel() // (H * W), H, W, L.stream()), "gaussian_blur5")
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        gy = gy.contiguous()
+        H, W = gy.shape[-2:]
+        gx = torch.empty_like(gy)
+        L.check(L.lib().ud_gaussian_blur5_bwd(L.ptr(gy), L.ptr(gx), gy.numel() // (H * W), H, W, L.stream()),
+                "gaussian_blur5_bwd")
+        return gx
+
+
 def gaussian_blur5(x):
     """random_blur (model/modules.py:15-16)."""
-    x = x.detach().contiguous()
-    L.require_cuda_f32(x)
-    H, W = x.shape[-2:]
-    y = torch.empty_like(x)
-    L.check(L.lib().ud_gaussian_blur5(L.ptr(x), L.ptr(y), x.numel() // (H * W), H, W, L.stream()), "gaussian_blur5")
-    return y
+    return _Blur5.apply(x)
+
+
+class _Downscale(torch.autograd.Function):
+    """downscale (model/modules.py:19-21); backward = sum over each input pixel's nearest-index preimage."""
+
+    @staticmethod
+    def forward(ctx, x, bottleneck_scale):
+        x = x.detach().contiguous()
+        L.require_cuda_f32(x)
+        H, W = x.shape[-2:]
+        y = torch.empty_like(x)
+        L.check(L.lib().ud_downscale_nearest(L.ptr(x), L.ptr(y), x.numel() // (H * W), H, W, bottleneck_scale,
+                                             L.stream()), "downscale")
+        ctx.scale = bottleneck_scale
+        return y
+
+    @staticmethod
+    def backward(ctx, gy):
+        gy = gy.contiguous()
+        H, W = gy.shape[-2:]
+        gx = torch.empty_like(gy)
+        L.check(L.lib().ud_downscale_nearest_bwd(L.ptr(gy), L.ptr(gx), gy.numel() // (H * W), H, W, ctx.scale,
+                                                 L.stream()), "downscale_bwd")
+        return gx, None
 
 
 def downscale_nearest(x, bottleneck_scale=0.75):
     """downscale (model/modules.py:19-21)."""
-    x = x.detach().contiguous()
-    L.require_cuda_f32(x)
-    H, W = x.shape[-2:]
-    y = torch.empty_like(x)
-    L.check(L.lib().ud_downscale_nearest(L.ptr(x), L.ptr(y), x.numel() // (H * W), H, W, float(bottleneck_scale),
-                                         L.stream()), "downscale")
-    return y
+    return _Downscale.apply(x, float(bottleneck_scale))
 
 
 def freq_style_transfer(content, style, lmda):
