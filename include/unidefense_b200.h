@@ -18,9 +18,9 @@
  *  - workspaces are passed in by the caller; *_workspace_bytes() say how large.
  *  - the first call for a new FFT length / resize pair builds its table with cudaMalloc + a synchronous copy:
  *    warm every shape up once before capturing calls into a CUDA graph (all later calls are capture-safe).
- *  - reductions are fixed-order (bitwise reproducible) except ud_recon_tail_bwd(2)'s g_dec and ud_bilinear_ac_bwd,
- *    whose transposed resize accumulates with float atomics.  The input-gradient outputs (g_x of ud_recon_tail_bwd2,
- *    ud_attn_prep_bwd, ud_gaussian_blur5_bwd, ud_downscale_nearest_bwd; g_diff of ud_dyfi_mask_bwd2) are gathers
+ *  - reductions are fixed-order (bitwise reproducible) except ud_recon_tail_bwd's g_dec and ud_bilinear_ac_bwd,
+ *    whose transposed resize accumulates with float atomics.  The input-gradient outputs (g_x of ud_recon_tail_bwd,
+ *    ud_attn_prep_bwd, ud_gaussian_blur5_bwd, ud_downscale_nearest_bwd; g_diff of ud_dyfi_mask_bwd) are gathers
  *    written once per element: bitwise reproducible.
  */
 #ifndef UNIDEFENSE_B200_H
@@ -43,7 +43,7 @@ typedef struct CUstream_st* cudaStream_t;
 #define UD_API
 #endif
 
-#define UD_B200_VERSION 100
+#define UD_B200_VERSION 101
 #define UD_FFT_MAX_N 1024
 
 #define UD_ACT_NONE 0
@@ -73,18 +73,15 @@ UD_API int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, float
 /* g_dec [N,C,h,w] = d(sum_n g_spatial[n]*spatial[n] + g_freq[n]*freq[n]) / d dec
  * (torch autograd of the lines above: abs -> sgn, fft_r2c_backward, upsample_bilinear2d_backward).
  * Samples with g_spatial[n]==g_freq[n]==0 (the engine's fake rows, abstract_engine.py:241,249)
- * cost nothing.                                                                              */
-UD_API int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
-                             const float* g_freq, float* g_dec, void* ws, size_t ws_bytes, int N, int C, int h,
-                             int w, int H, int W, int norm_ortho, cudaStream_t stream);
-/* The same backward with the input-image gradient (x is differentiated in the reference: rec - x at
+ * cost nothing.
+ * g_x [N,C,H,W] is the input-image gradient (x is differentiated in the reference: rec - x at
  * model/unidefense.py:245 and rfft2(x) at :247):
- *   g_x [N,C,H,W] = -(g_spatial[n]*sign(d)/(C*H*W) + fft_r2c_backward(g_freq[n]*sign(dF)/(C*H*Wh)))   (d = rec - x),
- * stored at full resolution by the pass that holds it before the transposed resize.  g_dec and g_x are each nullable
- * (not both); samples with g_spatial[n]==g_freq[n]==0 get g_x = 0.                                                   */
-UD_API int ud_recon_tail_bwd2(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
-                              const float* g_freq, float* g_dec, float* g_x, void* ws, size_t ws_bytes, int N, int C,
-                              int h, int w, int H, int W, int norm_ortho, cudaStream_t stream);
+ *   g_x = -(g_spatial[n]*sign(d)/(C*H*W) + fft_r2c_backward(g_freq[n]*sign(dF)/(C*H*Wh)))   (d = rec - x),
+ * stored at full resolution by the pass that holds it before the transposed resize; samples with
+ * g_spatial[n]==g_freq[n]==0 get g_x = 0.  g_dec and g_x are each nullable (not both).         */
+UD_API int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
+                             const float* g_freq, float* g_dec, float* g_x, void* ws, size_t ws_bytes, int N, int C,
+                             int h, int w, int H, int W, int norm_ortho, cudaStream_t stream);
 
 /* ---- a2: decoder epilogues ------------------------------------------------------------------
  * nn.InstanceNorm2d(C, affine) + MemoryEfficientSwish / nn.ReLU after every decoder conv
@@ -134,21 +131,16 @@ UD_API int ud_attn_prep(const float* pred, const float* x, float* spat_diff, flo
 UD_API int ud_attn_prep_bwd(const float* pred, const float* x, const float* g_spat_diff, const float* g_freq_diff,
                             float* g_x, int N, int C, int hp, int wp, int Hx, int Wx, int h, int w, int norm_ortho,
                             cudaStream_t stream);
-/* torch.fft.rfft2 + cat([re,im],1) of feature maps (model/unidefense.py:135-136): x [N,C,h,w] ->
- * xf [N,2C,h,w/2+1]; h,w <= 64.  adjoint_of_inverse=1 gives irfft2's backward (fft_c2r_backward:
- * interior columns doubled, inverse normalisation; SURVEY App. B.3).                               */
-UD_API int ud_rfft2_cat(const float* x, float* xf, int N, int C, int h, int w, int norm_ortho,
-                        int adjoint_of_inverse, cudaStream_t stream);
-/* torch.complex(*tensor_split(xf,2,1)) + irfft2(s=(h,w)) (model/unidefense.py:142-145): xf [N,2C,h,w/2+1]
- * (optionally multiplied on load by mask [N,h*(w/2+1)]) -> y [N,C,h,w].  adjoint_of_forward=1 gives
- * rfft2's backward (fft_r2c_backward: zero-padded half spectrum, no mirroring; SURVEY App. B.2).    */
-UD_API int ud_irfft2_cat(const float* xf, const float* mask, float* y, int N, int C, int h, int w, int norm_ortho,
-                         int adjoint_of_forward, cudaStream_t stream);
-/* Generic forms of the two calls above for ANY 1 <= h, w <= UD_FFT_MAX_N (torch.fft.rfft2 / irfft2 as called at
- * model/unidefense.py:135-145, :246-249, model/modules.py:43-54, model/efficientnet/exp.py:55-65,
- * model/resnet/exp.py:44-54): mixed radix when every prime factor is <= 23, Bluestein otherwise.  Planes with
- * h, w <= 64 take the workspace-free small-plane path; larger planes need ws of ud_rfft2_workspace_bytes()
- * (the row-transformed half spectrum, [N*C][h][w/2+1] complex).  Same flags and layouts as the _cat calls.  */
+/* ud_rfft2: torch.fft.rfft2 + cat([re,im],1) (model/unidefense.py:135-136): x [N,C,h,w] -> xf [N,2C,h,w/2+1].
+ * adjoint_of_inverse=1 gives irfft2's backward (fft_c2r_backward: interior columns doubled, inverse normalisation;
+ * SURVEY App. B.3).
+ * ud_irfft2: torch.complex(*tensor_split(xf,2,1)) + irfft2(s=(h,w)) (model/unidefense.py:142-145): xf [N,2C,h,w/2+1]
+ * (optionally multiplied on load by mask [N,h*(w/2+1)]) -> y [N,C,h,w].  adjoint_of_forward=1 gives rfft2's backward
+ * (fft_r2c_backward: zero-padded half spectrum, no mirroring; SURVEY App. B.2).
+ * Both take ANY 1 <= h, w <= UD_FFT_MAX_N (torch.fft.rfft2 / irfft2 as also called at model/unidefense.py:246-249,
+ * model/modules.py:43-54, model/efficientnet/exp.py:55-65, model/resnet/exp.py:44-54): mixed radix when every prime
+ * factor is <= 23, Bluestein otherwise.  Planes with h, w <= 64 take the workspace-free small-plane path; larger planes
+ * need ws of ud_rfft2_workspace_bytes() (the row-transformed half spectrum, [N*C][h][w/2+1] complex).             */
 UD_API size_t ud_rfft2_workspace_bytes(int N, int C, int h, int w);
 UD_API int ud_rfft2(const float* x, float* xf, void* ws, size_t ws_bytes, int N, int C, int h, int w, int norm_ortho,
                     int adjoint_of_inverse, cudaStream_t stream);
@@ -211,19 +203,14 @@ UD_API int ud_dyfi_mask_fwd(const float* proj, const float* bn_mean, const float
                             int act, cudaStream_t stream);
 UD_API size_t ud_dyfi_mask_bwd_workspace_bytes(int N, int HW);
 /* g_mask [N,HW] / g_out [N,Cx,HW] (either nullable) -> g_x = mask*g_out, dz [N,Cp,HW] (gradient w.r.t.
- * the BN output, to be finished by ud_bn_bwd_*), g_w2 [2+D].                                          */
+ * the BN output, to be finished by ud_bn_bwd_*), g_w2 [2+D], and g_diff [N,D,HW] (nullable) = w2[2+k] * d loss / d logit:
+ * the gradient of the guide channels cat'ed into layer2's input (model/modules.py:101-103, :130-132), through which the
+ * error maps carry x's gradient.                                                                                   */
 UD_API int ud_dyfi_mask_bwd(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
                             const float* beta, const float* diff, const float* w2, const float* x, const float* mask,
                             const float* pmean, const float* pmax, const int* argmax, const float* g_mask,
-                            const float* g_out, float* g_x, float* dz, float* g_w2, void* ws, size_t ws_bytes, int N,
-                            int Cp, int D, int Cx, int HW, int act, cudaStream_t stream);
-/* ud_dyfi_mask_bwd plus g_diff [N,D,HW] (nullable) = w2[2+k] * d loss / d logit: the gradient of the guide channels
- * cat'ed into layer2's input (model/modules.py:101-103, :130-132), through which the error maps carry x's gradient. */
-UD_API int ud_dyfi_mask_bwd2(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
-                             const float* beta, const float* diff, const float* w2, const float* x, const float* mask,
-                             const float* pmean, const float* pmax, const int* argmax, const float* g_mask,
-                             const float* g_out, float* g_x, float* dz, float* g_w2, float* g_diff, void* ws,
-                             size_t ws_bytes, int N, int Cp, int D, int Cx, int HW, int act, cudaStream_t stream);
+                            const float* g_out, float* g_x, float* dz, float* g_w2, float* g_diff, void* ws,
+                            size_t ws_bytes, int N, int Cp, int D, int Cx, int HW, int act, cudaStream_t stream);
 
 /* ---- a9-a11: losses; each also returns d loss / d input for upstream gradient 1 ------------------
  * AsymmetricalWeightedTripletLoss.forward (loss/triplet_loss.py:75-82): feat [N,c], labels int64 [N]

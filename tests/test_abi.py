@@ -26,7 +26,7 @@ def test_every_declared_symbol_is_exported_and_bound():
 def test_status_calls_without_gpu():
     from unidefense_b200 import _lib
     L = _lib.lib()
-    assert L.ud_version() >= 100
+    assert L.ud_version() >= 101
     assert L.ud_fft_size_supported(380) == 1 and L.ud_fft_size_supported(299) == 1
     assert L.ud_fft_size_supported(58) == 0          # 29 is not a mixed-radix factor ...
     assert L.ud_fft_size_any(58) == 1                # ... such sizes run Bluestein

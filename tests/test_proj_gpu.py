@@ -81,8 +81,8 @@ def test_filter_modules_use_the_tensor_core_path(golden_ops_r2):
     import torch.nn as nn
 
     from unidefense_b200 import _lib as L
+    from unidefense_b200 import ops
     from unidefense_b200.model import modules as M
-    assert M.PROJ_BACKEND == "tcgen05"
     for c in golden_ops_r2["dyfi_wide"]:
         depth = c["x"].shape[1] // (2 if c["kind"] == "freq" else 1)
         act = M.MemoryEfficientSwish if c["act"] == "swish" else nn.ReLU
@@ -90,6 +90,7 @@ def test_filter_modules_use_the_tensor_core_path(golden_ops_r2):
         mod = cls(depth, act, nn.BatchNorm2d, True, False).cuda().train()
         mod.load_state_dict(c["sd0"])
         x = c["x"].cuda().requires_grad_()
+        assert ops.proj_supported(x, mod.layer1[0])             # the module selects the tcgen05 projection
         before = L.lib().ud_launch_count()
         out = mod(x, c["diff"].cuda())
         assert x.shape[1] >= 32 and x.shape[1] % 4 == 0

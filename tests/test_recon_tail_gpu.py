@@ -25,6 +25,8 @@ SHAPES = [
     (1, 2, 31, 40, 62, 80),      # Bluestein columns (62 = 2*31), mixed-radix rows
     (1, 3, 124, 124, 248, 248),  # the ADVICE example: 248 = 8*31
     (1, 1, 20, 37, 40, 37),      # prime 37 rows
+    (1, 3, 128, 150, 256, 300),  # first-generation kernels with 256-point columns (300 is no second-generation size)
+    (1, 3, 150, 190, 300, 380),  # first-generation kernels with 380-point rows
 ]
 
 

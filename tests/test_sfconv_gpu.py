@@ -69,21 +69,8 @@ def test_mix(shape, dtype, cl):
           atol=(2e-2 if dtype == torch.bfloat16 else 1e-4) * float(ref[2].grad.abs()) + 1e-4)
 
 
-@pytest.mark.parametrize("own_fft", [False, True])
 @pytest.mark.parametrize("cl", [False, True])
-def test_sfconv_modules_reference_fixture(golden_ops, cl, own_fft):
-    """own_fft: the fp32 path on this repo's transforms (ud_rfft2 / ud_irfft2 with their autograd adjoints) instead of
-    cuFFT -- same reference fixtures, same tolerances."""
-    from unidefense_b200.model import sfconv as SF
-    old = SF.USE_OWN_FFT
-    SF.USE_OWN_FFT = own_fft
-    try:
-        _sfconv_fixture_body(golden_ops, cl)
-    finally:
-        SF.USE_OWN_FFT = old
-
-
-def _sfconv_fixture_body(golden_ops, cl):
+def test_sfconv_modules_reference_fixture(golden_ops, cl):
     from unidefense_b200.model.sfconv import SFConv2d, SFSamePadConv2d
     for c in golden_ops["sfconv"]:
         C, hw, s = c["x"].shape[1], c["x"].shape[-1], c["stride"]
@@ -119,18 +106,17 @@ def test_sfconv_paths_agree_bf16(cfg):
     m = m.to(memory_format=torch.channels_last)
     x = torch.randn(4, C, hw, hw, device="cuda").contiguous(memory_format=torch.channels_last)
     outs = {}
-    try:
-        for mode, (gemm, glue) in {"gemm": (True, True), "glue": (False, True), "plain": (False, False)}.items():
-            sfconv.USE_DFT_GEMM, sfconv.USE_GLUE_KERNELS = gemm, glue
-            xi = x.clone().requires_grad_()
-            m.zero_grad()
-            with torch.autocast("cuda", dtype=torch.bfloat16):
-                y = m(xi)
-            y.float().square().mean().backward()
-            outs[mode] = (y.float(), xi.grad.float(), m.freq_conv.weight.grad.clone(), m.sf_coef.grad.clone().reshape(1),
-                          m.weight.grad.clone())
-    finally:
-        sfconv.USE_DFT_GEMM, sfconv.USE_GLUE_KERNELS = True, True
+    paths = {"gemm": sfconv._sf_forward_gemm, "glue": sfconv._sf_forward_glue, "plain": sfconv._sf_forward_plain}
+    for mode, sf_forward in paths.items():
+        xi = x.clone().requires_grad_()
+        m.zero_grad()
+        with torch.autocast("cuda", dtype=torch.bfloat16):
+            assert sfconv._dft_gemm_ok(xi)          # the module itself takes the GEMM path here
+            spat = m._conv_forward(m.static_padding(xi), m.weight, m.bias)
+            y = sf_forward(xi, spat, m.freq_conv, m.sf_coef, m.freq_norm)
+        y.float().square().mean().backward()
+        outs[mode] = (y.float(), xi.grad.float(), m.freq_conv.weight.grad.clone(), m.sf_coef.grad.clone().reshape(1),
+                      m.weight.grad.clone())
     for mode in ("gemm", "glue"):
         for a, b in zip(outs[mode], outs["plain"]):
             torch.testing.assert_close(a, b, rtol=5e-2, atol=3e-2 * float(b.abs().max()) + 1e-6)

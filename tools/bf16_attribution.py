@@ -6,6 +6,7 @@ F.dropout = lambda t, p=0.5, training=True, inplace=False: t * 1.0
 torch.backends.cudnn.deterministic = True
 from unidefense_b200.model import load_model, sfconv
 from unidefense_b200 import ops
+dft_gemm_ok = sfconv._dft_gemm_ok
 
 def build(arch):
     name, kw = {"eb4": ("UDEB4", dict(extractor="efficientnet-b4", num_classes=2, drop_rate=0.0, drop_connect_rate=0.0)),
@@ -26,7 +27,7 @@ for arch in ("eb4", "r18"):
     ref = build(arch)(x)
     for tag, dft, cl, tf32 in (("bench config", True, True, True), ("DFT-GEMM off (cuFFT fp32)", False, True, True),
                                ("DFT-GEMM off, NCHW", False, False, True), ("bench config, 3xTF32 projections", True, True, False)):
-        sfconv.USE_DFT_GEMM = dft
+        sfconv._dft_gemm_ok = dft_gemm_ok if dft else (lambda x: False)      # "DFT-GEMM off": the cuFFT glue path
         m = build(arch)
         if cl:
             for part in ("backbone", "extractor", "emb_block1", "emb_block2"):
@@ -41,4 +42,4 @@ for arch in ("eb4", "r18"):
               f"fmask {rel2(a['freq_mask'], b['freq_mask']):.3f} smask {rel2(a['spat_mask'], b['spat_mask']):.3f} "
               f"tri0 {rel2(a['triplet'][0], b['triplet'][0]):.3f} fac {rel2(a['factorization'], b['factorization']):.3f} "
               f"spatial {rel2(a['spatial'], b['spatial']):.4f}", flush=True)
-    sfconv.USE_DFT_GEMM = True
+    sfconv._dft_gemm_ok = dft_gemm_ok

@@ -72,12 +72,12 @@ def kernels(iters, flush):
     g_dec, g_x = torch.empty_like(dec), torch.empty_like(x)
     img, small, sb = N * C * R * R * 4, N * C * h * h * 4, signs.numel()
     row("recon_tail_bwd (g_dec)", lambda: L.check(lib.ud_recon_tail_bwd(
-        L.ptr(dec), L.ptr(x), L.ptr(signs), L.ptr(gs), L.ptr(gf), L.ptr(g_dec), L.ptr(ws), nws, N, C, h, h, R, R, 1, s)),
-        small + img + sb + small, "reads dec, x, signs; writes g_dec")
-    row("recon_tail_bwd2 (g_dec + g_x)", lambda: L.check(lib.ud_recon_tail_bwd2(
+        L.ptr(dec), L.ptr(x), L.ptr(signs), L.ptr(gs), L.ptr(gf), L.ptr(g_dec), None, L.ptr(ws), nws, N, C, h, h, R, R, 1,
+        s)), small + img + sb + small, "reads dec, x, signs; writes g_dec")
+    row("recon_tail_bwd (g_dec + g_x)", lambda: L.check(lib.ud_recon_tail_bwd(
         L.ptr(dec), L.ptr(x), L.ptr(signs), L.ptr(gs), L.ptr(gf), L.ptr(g_dec), L.ptr(g_x), L.ptr(ws), nws, N, C, h, h, R,
         R, 1, s)), small + img + sb + small + img, "+ 3R^2*4 B written per sample")
-    row("recon_tail_bwd2 (g_x only)", lambda: L.check(lib.ud_recon_tail_bwd2(
+    row("recon_tail_bwd (g_x only)", lambda: L.check(lib.ud_recon_tail_bwd(
         L.ptr(dec), L.ptr(x), L.ptr(signs), L.ptr(gs), L.ptr(gf), None, L.ptr(g_x), L.ptr(ws), nws, N, C, h, h, R, R, 1,
         s)), small + img + sb + img, "dec detached")
     # error maps -> x
@@ -108,9 +108,9 @@ def kernels(iters, flush):
         base = (3 * proj.numel() + 3 * xx.numel() + 4 * N * hw + D * N * hw) * 4
         row(f"dyfi_mask_bwd ({kind})", lambda: L.check(lib.ud_dyfi_mask_bwd(
             L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(gam), L.ptr(bet), L.ptr(diff), L.ptr(w2), L.ptr(xx), L.ptr(mask),
-            L.ptr(pm), L.ptr(px), L.ptr(am), None, L.ptr(go), L.ptr(gxx), L.ptr(dz), L.ptr(gw2), L.ptr(wsd), wsd.numel(),
-            N, Cp, D, Cp, hw, 2, s)), base, "training path")
-        row(f"dyfi_mask_bwd2 ({kind}, + g_diff)", lambda: L.check(lib.ud_dyfi_mask_bwd2(
+            L.ptr(pm), L.ptr(px), L.ptr(am), None, L.ptr(go), L.ptr(gxx), L.ptr(dz), L.ptr(gw2), None, L.ptr(wsd),
+            wsd.numel(), N, Cp, D, Cp, hw, 2, s)), base, "training path")
+        row(f"dyfi_mask_bwd ({kind}, + g_diff)", lambda: L.check(lib.ud_dyfi_mask_bwd(
             L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(gam), L.ptr(bet), L.ptr(diff), L.ptr(w2), L.ptr(xx), L.ptr(mask),
             L.ptr(pm), L.ptr(px), L.ptr(am), None, L.ptr(go), L.ptr(gxx), L.ptr(dz), L.ptr(gw2), L.ptr(gd), L.ptr(wsd),
             wsd.numel(), N, Cp, D, Cp, hw, 2, s)), base + gd.numel() * 4, "+ D*HW*4 B written per sample")

@@ -30,8 +30,7 @@ SIGNATURES = {
     "ud_recon_tail_workspace_bytes": (c_sz, [c_i] * 6),
     "ud_recon_tail_signs_bytes": (c_sz, [c_i] * 4),
     "ud_recon_tail_fwd": (c_i, [c_p] * 7 + [c_sz] + [c_i] * 7 + [c_p]),
-    "ud_recon_tail_bwd": (c_i, [c_p] * 7 + [c_sz] + [c_i] * 7 + [c_p]),
-    "ud_recon_tail_bwd2": (c_i, [c_p] * 8 + [c_sz] + [c_i] * 7 + [c_p]),
+    "ud_recon_tail_bwd": (c_i, [c_p] * 8 + [c_sz] + [c_i] * 7 + [c_p]),
     "ud_in_act_fwd": (c_i, [c_p] * 7 + [c_i] * 3 + [c_f, c_i, c_p]),
     "ud_in_act_bwd_workspace_bytes": (c_sz, [c_i, c_i]),
     "ud_in_act_bwd": (c_i, [c_p] * 11 + [c_sz] + [c_i] * 4 + [c_p]),
@@ -43,8 +42,6 @@ SIGNATURES = {
     "ud_bilinear_ac_bwd": (c_i, [c_p, c_p] + [c_i] * 5 + [c_p]),
     "ud_attn_prep": (c_i, [c_p] * 4 + [c_i] * 9 + [c_p]),
     "ud_attn_prep_bwd": (c_i, [c_p] * 5 + [c_i] * 9 + [c_p]),
-    "ud_rfft2_cat": (c_i, [c_p, c_p] + [c_i] * 6 + [c_p]),
-    "ud_irfft2_cat": (c_i, [c_p, c_p, c_p] + [c_i] * 6 + [c_p]),
     "ud_rfft2_workspace_bytes": (c_sz, [c_i] * 4),
     "ud_rfft2": (c_i, [c_p] * 3 + [c_sz] + [c_i] * 6 + [c_p]),
     "ud_irfft2": (c_i, [c_p] * 4 + [c_sz] + [c_i] * 6 + [c_p]),
@@ -64,8 +61,7 @@ SIGNATURES = {
     "ud_bn_merge_partials": (c_i, [c_p] * 5 + [c_i] * 2 + [c_p]),
     "ud_dyfi_mask_fwd": (c_i, [c_p] * 13 + [c_i] * 6 + [c_p]),
     "ud_dyfi_mask_bwd_workspace_bytes": (c_sz, [c_i, c_i]),
-    "ud_dyfi_mask_bwd": (c_i, [c_p] * 18 + [c_sz] + [c_i] * 6 + [c_p]),
-    "ud_dyfi_mask_bwd2": (c_i, [c_p] * 19 + [c_sz] + [c_i] * 6 + [c_p]),
+    "ud_dyfi_mask_bwd": (c_i, [c_p] * 19 + [c_sz] + [c_i] * 6 + [c_p]),
     "ud_triplet_fwd": (c_i, [c_p] * 4 + [c_i, c_i, c_p]),
     "ud_factorization_workspace_bytes": (c_sz, [c_i, c_i]),
     "ud_factorization_fwd": (c_i, [c_p] * 5 + [c_sz, c_i, c_i, c_f, c_f, c_p]),

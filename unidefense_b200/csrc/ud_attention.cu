@@ -287,15 +287,6 @@ int ud_rfft2_small(const float* x, float* xf, int N, int C, int h, int w, int no
   return ud_check_launch("rfft2_cat");
 }
 
-extern "C" int ud_rfft2_cat(const float* x, float* xf, int N, int C, int h, int w, int norm_ortho, int adjoint_of_inverse,
-                            cudaStream_t stream) {
-  int rc = at_check_small("rfft2_cat", N, C, h, w);
-  if (rc != UD_OK) return rc;
-  if (N == 0) return UD_OK;
-  UD_REQUIRE(x && xf, UD_ERR_INVALID, "rfft2_cat: null pointer");
-  return ud_rfft2_small(x, xf, N, C, h, w, norm_ortho, adjoint_of_inverse, stream);
-}
-
 // mode 0: inverse transform irfft2(s=(h,w)) (column multipliers m_k, scale per norm);
 // mode 1: adjoint of the forward transform (rfft2 backward: zero-padded, no multipliers)
 int ud_irfft2_small(const float* xf, const float* mask, float* y, int N, int C, int h, int w, int norm_ortho,
@@ -309,15 +300,6 @@ int ud_irfft2_small(const float* xf, const float* mask, float* y, int N, int C, 
   at_c2r_kernel<<<ud_cdiv(planes, P), AT_THREADS, smem, stream>>>(xf, mask, y, planes, C, h, w, scale,
                                                                    adjoint_of_forward ? 0 : 1, P);
   return ud_check_launch("irfft2_cat");
-}
-
-extern "C" int ud_irfft2_cat(const float* xf, const float* mask, float* y, int N, int C, int h, int w, int norm_ortho,
-                             int adjoint_of_forward, cudaStream_t stream) {
-  int rc = at_check_small("irfft2_cat", N, C, h, w);
-  if (rc != UD_OK) return rc;
-  if (N == 0) return UD_OK;
-  UD_REQUIRE(xf && y, UD_ERR_INVALID, "irfft2_cat: null pointer");
-  return ud_irfft2_small(xf, mask, y, N, C, h, w, norm_ortho, adjoint_of_forward, stream);
 }
 
 // ---------------------------------------------------------------- a4: error maps

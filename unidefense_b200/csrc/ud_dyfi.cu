@@ -293,11 +293,12 @@ extern "C" size_t ud_dyfi_mask_bwd_workspace_bytes(int N, int HW) {
   return sizeof(float) * (size_t)N * ud_cdiv(HW, 32) * DF_MAX_PRE;
 }
 
-static int df_mask_bwd(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
-                       const float* beta, const float* diff, const float* w2, const float* x, const float* mask,
-                       const float* pmean, const float* pmax, const int* argmax, const float* g_mask, const float* g_out,
-                       float* g_x, float* dz, float* g_w2, float* g_diff, void* ws, size_t ws_bytes, int N, int Cp, int D,
-                       int Cx, int HW, int act, cudaStream_t stream) {
+extern "C" int ud_dyfi_mask_bwd(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
+                                const float* beta, const float* diff, const float* w2, const float* x,
+                                const float* mask, const float* pmean, const float* pmax, const int* argmax,
+                                const float* g_mask, const float* g_out, float* g_x, float* dz, float* g_w2, float* g_diff,
+                                void* ws, size_t ws_bytes, int N, int Cp, int D, int Cx, int HW, int act,
+                                cudaStream_t stream) {
   UD_REQUIRE(N >= 0 && Cp >= 1 && D >= 0 && Cx >= 1 && HW >= 1 && 2 + D <= DF_MAX_PRE, UD_ERR_INVALID,
              "dyfi_mask_bwd: bad shape");
   UD_REQUIRE(g_w2, UD_ERR_INVALID, "dyfi_mask_bwd: null pointer");
@@ -309,6 +310,7 @@ static int df_mask_bwd(const float* proj, const float* bn_mean, const float* bn_
                  (!g_out || (x && g_x)),
              UD_ERR_INVALID, "dyfi_mask_bwd: null pointer");
   UD_REQUIRE(ws_bytes >= ud_dyfi_mask_bwd_workspace_bytes(N, HW), UD_ERR_WORKSPACE, "dyfi_mask_bwd: workspace too small");
+  if (D == 0) g_diff = nullptr;
   const int tiles = ud_cdiv(HW, 32);
   float* part = static_cast<float*>(ws);
   auto k = g_diff ? df_mask_bwd_kernel<true> : df_mask_bwd_kernel<false>;
@@ -318,23 +320,4 @@ static int df_mask_bwd(const float* proj, const float* bn_mean, const float* bn_
   if (rc != UD_OK) return rc;
   df_w2_reduce_kernel<<<2 + D, 128, 0, stream>>>(part, g_w2, N * tiles, 2 + D);
   return ud_check_launch("dyfi_w2_reduce");
-}
-
-extern "C" int ud_dyfi_mask_bwd(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
-                                const float* beta, const float* diff, const float* w2, const float* x,
-                                const float* mask, const float* pmean, const float* pmax, const int* argmax,
-                                const float* g_mask, const float* g_out, float* g_x, float* dz, float* g_w2, void* ws,
-                                size_t ws_bytes, int N, int Cp, int D, int Cx, int HW, int act, cudaStream_t stream) {
-  return df_mask_bwd(proj, bn_mean, bn_rstd, gamma, beta, diff, w2, x, mask, pmean, pmax, argmax, g_mask, g_out, g_x, dz,
-                     g_w2, nullptr, ws, ws_bytes, N, Cp, D, Cx, HW, act, stream);
-}
-
-extern "C" int ud_dyfi_mask_bwd2(const float* proj, const float* bn_mean, const float* bn_rstd, const float* gamma,
-                                 const float* beta, const float* diff, const float* w2, const float* x,
-                                 const float* mask, const float* pmean, const float* pmax, const int* argmax,
-                                 const float* g_mask, const float* g_out, float* g_x, float* dz, float* g_w2,
-                                 float* g_diff, void* ws, size_t ws_bytes, int N, int Cp, int D, int Cx, int HW, int act,
-                                 cudaStream_t stream) {
-  return df_mask_bwd(proj, bn_mean, bn_rstd, gamma, beta, diff, w2, x, mask, pmean, pmax, argmax, g_mask, g_out, g_x, dz,
-                     g_w2, D > 0 ? g_diff : nullptr, ws, ws_bytes, N, Cp, D, Cx, HW, act, stream);
 }

@@ -18,7 +18,6 @@
 // HBM traffic per sample (fp32): fwd reads dec+x, writes rec (+1 B/bin signs);
 // bwd reads dec+x(+signs), writes g_dec.
 #include "../../include/unidefense_b200.h"
-#include <stdlib.h>
 
 #include "ud_fft.cuh"
 #include "ud_fft_any.cuh"
@@ -32,24 +31,10 @@ int ud_rt2_fwd(const float* dec, const float* x, float* rec, float2* Z, float* p
 int ud_rt2_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial, const float* g_freq,
                float* g_dec, float* g_x, float2* T, int plane0, int planes, int C, int h, int w, int H, int W, int row_tiles,
                int col_tiles, float gscale, float sp_scale, cudaStream_t stream);
-// row pairs per rows-CTA of ud_recon_tail2.cu = its RT2_LPC (16) x the steps a CTA walks.  Measured at N=32, 380^2: one
+// Each rows-CTA of ud_recon_tail2.cu walks one step of ud_rt2_rows_lpc() (16) row pairs.  Measured at N=32, 380^2: one
 // step per CTA (12 row tiles per plane, ~4 waves) and two (6 tiles, ~2 waves) take the same time (101 / 89 us fwd / bwd),
 // three is 10-30 % slower: the kernels are bound per SM (issue + L2 latency at 20 resident warps), not by wave shape.
-// UD_RT2_ITER overrides (profiling aid).
-static int rt2_pairs_per_tile() {
-  static const int iters = [] {
-    const char* e = getenv("UD_RT2_ITER");
-    const int v = e ? atoi(e) : 1;
-    return v >= 1 && v <= 8 ? v : 1;
-  }();
-  return ud_rt2_rows_lpc() * iters;
-}
-#define RT2_PAIRS_PER_TILE rt2_pairs_per_tile()
 #define RT2_COLS_PER_TILE 16
-static bool rt_use_v2(int h, int w, int H, int W) {
-  static const bool force_v1 = getenv("UD_RT_V1") != nullptr;      // A/B switch for profiling
-  return !force_v1 && ud_rt2_supported(h, w, H, W);
-}
 
 #define RT_ROW_T 256   // threads of the rows kernels
 #define RT_ROW_L 12    // row PAIRS (complex lines) per CTA of the rows kernels  -> 24 image rows
@@ -570,21 +555,14 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-static bool rt_static_size(int n) { return n == 380 || n == 256 || n == 224 || n == 299; }
-// points per line buffer / staged twiddles: n, or the Bluestein length for sizes with a prime factor > 23 (0 = error)
-static int rt_line_len(int n) {
-  if (rt_static_size(n)) return n;
-  UdAnyPlan p;
-  return ud_make_any_plan(n, &p) ? p.m : 0;
-}
+// m: points per line buffer / staged twiddles (UdAnyPlan::m: n, or the Bluestein length for sizes with a prime factor
+// > 23).  The plans are not in place, so the kernels keep two line buffers.
 static size_t rt_rows_smem(int n, int m, int w) {
-  const size_t bufs = rt_static_size(n) ? 1 : 2;
-  return sizeof(float2) * ((size_t)m + n + bufs * RT_ROW_L * (size_t)(m | 1)) + sizeof(float) * 4ull * RT_VGRP * w +
+  return sizeof(float2) * ((size_t)m + n + 2ull * RT_ROW_L * (size_t)(m | 1)) + sizeof(float) * 4ull * RT_VGRP * w +
          (size_t)RT_ROW_L * n;   // + sign bytes of the tile (rows_bwd)
 }
-static size_t rt_cols_smem(int n, int m) {
-  const size_t bufs = rt_static_size(n) ? 1 : 2;
-  return sizeof(float2) * ((size_t)m + bufs * RT_COL_L * (size_t)(m | 1));
+static size_t rt_cols_smem(int m) {
+  return sizeof(float2) * ((size_t)m + 2ull * RT_COL_L * (size_t)(m | 1));
 }
 
 static size_t rt_plane_bytes(int H, int W) {
@@ -614,17 +592,6 @@ extern "C" size_t ud_recon_tail_workspace_bytes(int N, int C, int h, int w, int 
 extern "C" size_t ud_recon_tail_signs_bytes(int N, int C, int H, int W) {
   return (size_t)N * C * (W / 2 + 1) * H;
 }
-
-// Runs the body with PLANVAR bound to the in-place static plan for n when one exists, else a run-time plan (mixed radix,
-// or Bluestein for sizes with a prime factor > 23).
-#define RT_DISPATCH_PLAN(n, L, THREADS, PLANVAR, ...)                                                    \
-  do {                                                                                                   \
-    if ((n) == 380) { UdStaticPlanIP<380, L, THREADS, 19, 5, 4> PLANVAR; __VA_ARGS__; }                  \
-    else if ((n) == 256) { UdStaticPlanIP<256, L, THREADS, 4, 4, 4, 4> PLANVAR; __VA_ARGS__; }           \
-    else if ((n) == 224) { UdStaticPlanIP<224, L, THREADS, 7, 4, 4, 2> PLANVAR; __VA_ARGS__; }           \
-    else if ((n) == 299) { UdStaticPlanIP<299, L, THREADS, 23, 13> PLANVAR; __VA_ARGS__; }               \
-    else { UdAnyPlan PLANVAR; if (!ud_make_any_plan((n), &PLANVAR)) return UD_ERR_UNSUPPORTED; __VA_ARGS__; } \
-  } while (0)
 
 template <class K>
 static int rt_set_smem(K kernel, size_t bytes) {
@@ -662,8 +629,8 @@ extern "C" int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, f
   int chunk = rt_chunk_samples(N, C, H, W);
   if (chunk * C > 65535) chunk = 65535 / C;
   const int Wh = W / 2 + 1;
-  const bool v2 = rt_use_v2(h, w, H, W);
-  const int row_tiles = v2 ? ud_cdiv((H + 1) / 2, RT2_PAIRS_PER_TILE) : ud_cdiv(H, 2 * RT_ROW_L);
+  const bool v2 = ud_rt2_supported(h, w, H, W);
+  const int row_tiles = v2 ? ud_cdiv((H + 1) / 2, ud_rt2_rows_lpc()) : ud_cdiv(H, 2 * RT_ROW_L);
   const int col_tiles = v2 ? ud_cdiv(Wh, RT2_COLS_PER_TILE) : ud_cdiv(Wh, RT_COL_L);
   char* p = static_cast<char*>(ws);
   float2* Y = reinterpret_cast<float2*>(p);
@@ -671,14 +638,12 @@ extern "C" int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, f
   float* part_sp = reinterpret_cast<float*>(p);
   p += ud_align_up((size_t)N * C * row_tiles * sizeof(float), 256);
   float* part_fr = reinterpret_cast<float*>(p);
-  const int mW = rt_line_len(W), mH = rt_line_len(H);
-  if (!mW || !mH) return UD_ERR_UNSUPPORTED;
-  const float2* twW = ud_twiddles(mW);
-  const float2* twH = ud_twiddles(mH);
+  UdAnyPlan pW, pH;   // line FFTs of the first-generation kernels: mixed radix, or Bluestein for a prime factor > 23
+  if (!ud_make_any_plan(W, &pW) || !ud_make_any_plan(H, &pH)) return UD_ERR_UNSUPPORTED;
   const float2* ytab = ud_lerp_table(h, H);
   const float2* xtab = ud_lerp_table(w, W);
-  if (!twW || !twH || !ytab || !xtab) return UD_ERR_CUDA;
-  const size_t smW = rt_rows_smem(W, mW, w), smH = rt_cols_smem(H, mH);
+  if (!ytab || !xtab) return UD_ERR_CUDA;
+  const size_t smW = rt_rows_smem(W, pW.m, w), smH = rt_cols_smem(pH.m);
 
   for (int s0 = 0; s0 < N; s0 += chunk) {
     const int ns = (N - s0 < chunk) ? (N - s0) : chunk;
@@ -688,18 +653,13 @@ extern "C" int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, f
                            stream)) != UD_OK) return rc;
       continue;
     }
-    RT_DISPATCH_PLAN(W, RT_ROW_L, RT_ROW_T, plan, {
-      auto k = rt_rows_fwd_kernel<decltype(plan)>;
-      if ((rc = rt_set_smem(k, smW)) != UD_OK) return rc;
-      k<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(plan, dec, x, rec, Y, part_sp, twW, ytab, xtab, plane0,
-                                                             h, w, H, W, row_tiles);
-    });
+    if ((rc = rt_set_smem(rt_rows_fwd_kernel<UdAnyPlan>, smW)) != UD_OK) return rc;
+    rt_rows_fwd_kernel<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(pW, dec, x, rec, Y, part_sp, pW.tw, ytab, xtab,
+                                                                           plane0, h, w, H, W, row_tiles);
     if ((rc = ud_check_launch("rt_rows_fwd")) != UD_OK) return rc;
-    RT_DISPATCH_PLAN(H, RT_COL_L, RT_COL_T, plan, {
-      auto k = rt_cols_fwd_kernel<decltype(plan)>;
-      if ((rc = rt_set_smem(k, smH)) != UD_OK) return rc;
-      k<<<dim3(col_tiles, planes), RT_COL_T, smH, stream>>>(plan, Y, part_fr, signs, twH, plane0, H, W, col_tiles);
-    });
+    if ((rc = rt_set_smem(rt_cols_fwd_kernel<UdAnyPlan>, smH)) != UD_OK) return rc;
+    rt_cols_fwd_kernel<<<dim3(col_tiles, planes), RT_COL_T, smH, stream>>>(pH, Y, part_fr, signs, pH.tw, plane0, H, W,
+                                                                           col_tiles);
     if ((rc = ud_check_launch("rt_cols_fwd")) != UD_OK) return rc;
   }
   const float nrm = norm_ortho ? 1.f / sqrtf((float)H * (float)W) : 1.f;
@@ -708,10 +668,10 @@ extern "C" int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, f
   return ud_check_launch("rt_finalize");
 }
 
-// g_dec and g_x are each nullable (not both): ud_recon_tail_bwd passes g_x = NULL, which selects the GX = false kernels
-static int rt_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial, const float* g_freq,
-                  float* g_dec, float* g_x, void* ws, size_t ws_bytes, int N, int C, int h, int w, int H, int W,
-                  int norm_ortho, cudaStream_t stream) {
+// g_dec and g_x are each nullable (not both); g_x = NULL selects the GX = false kernels (the training path)
+extern "C" int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
+                                 const float* g_freq, float* g_dec, float* g_x, void* ws, size_t ws_bytes, int N, int C,
+                                 int h, int w, int H, int W, int norm_ortho, cudaStream_t stream) {
   int rc = rt_validate(N, C, h, w, H, W);
   if (rc != UD_OK) return rc;
   if (N == 0) return UD_OK;
@@ -722,20 +682,18 @@ static int rt_bwd(const float* dec, const float* x, const uint8_t* signs, const 
   int chunk = rt_chunk_samples(N, C, H, W);
   if (chunk * C > 65535) chunk = 65535 / C;
   const int Wh = W / 2 + 1;
-  const bool v2 = rt_use_v2(h, w, H, W);
-  const int row_tiles = v2 ? ud_cdiv((H + 1) / 2, RT2_PAIRS_PER_TILE) : ud_cdiv(H, 2 * RT_ROW_L);
+  const bool v2 = ud_rt2_supported(h, w, H, W);
+  const int row_tiles = v2 ? ud_cdiv((H + 1) / 2, ud_rt2_rows_lpc()) : ud_cdiv(H, 2 * RT_ROW_L);
   const int col_tiles = v2 ? ud_cdiv(Wh, RT2_COLS_PER_TILE) : ud_cdiv(Wh, RT_COL_L);
   float2* T = reinterpret_cast<float2*>(ws);
-  const int mW = rt_line_len(W), mH = rt_line_len(H);
-  if (!mW || !mH) return UD_ERR_UNSUPPORTED;
-  const float2* twW = ud_twiddles(mW);
-  const float2* twH = ud_twiddles(mH);
+  UdAnyPlan pW, pH;   // line FFTs of the first-generation kernels: mixed radix, or Bluestein for a prime factor > 23
+  if (!ud_make_any_plan(W, &pW) || !ud_make_any_plan(H, &pH)) return UD_ERR_UNSUPPORTED;
   const float2* ytab = ud_lerp_table(h, H);
   const float2* xtab = ud_lerp_table(w, W);
-  if (!twW || !twH || !ytab || !xtab) return UD_ERR_CUDA;
+  if (!ytab || !xtab) return UD_ERR_CUDA;
   const int2* jtab = ud_lerp_ranges(w, W);
   if (!jtab) return UD_ERR_CUDA;
-  const size_t smH = rt_cols_smem(H, mH), smW = rt_rows_smem(W, mW, w);
+  const size_t smH = rt_cols_smem(pH.m), smW = rt_rows_smem(W, pW.m, w);
   // freq[n] = nrm/(C*H*Wh) * sum |D'| with D' the unnormalised spectrum, so the sign spectrum
   // carries nrm/(C*H*Wh) and the adjoint of the unnormalised forward is the unnormalised inverse.
   const float nrm = norm_ortho ? 1.f / sqrtf((float)H * (float)W) : 1.f;
@@ -750,32 +708,15 @@ static int rt_bwd(const float* dec, const float* x, const uint8_t* signs, const 
                            gscale, sp_scale, stream)) != UD_OK) return rc;
       continue;
     }
-    RT_DISPATCH_PLAN(H, RT_COL_L, RT_COL_T, plan, {
-      auto k = rt_cols_bwd_kernel<decltype(plan)>;
-      if ((rc = rt_set_smem(k, smH)) != UD_OK) return rc;
-      k<<<dim3(col_tiles, planes), RT_COL_T, smH, stream>>>(plan, signs, g_freq, T, twH, plane0, C, H, W, gscale);
-    });
+    if ((rc = rt_set_smem(rt_cols_bwd_kernel<UdAnyPlan>, smH)) != UD_OK) return rc;
+    rt_cols_bwd_kernel<<<dim3(col_tiles, planes), RT_COL_T, smH, stream>>>(pH, signs, g_freq, T, pH.tw, plane0, C, H, W,
+                                                                           gscale);
     if ((rc = ud_check_launch("rt_cols_bwd")) != UD_OK) return rc;
-    RT_DISPATCH_PLAN(W, RT_ROW_L, RT_ROW_T, plan, {
-      auto k = g_x ? rt_rows_bwd_kernel<decltype(plan), true> : rt_rows_bwd_kernel<decltype(plan), false>;
-      if ((rc = rt_set_smem(k, smW)) != UD_OK) return rc;
-      k<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(plan, dec, x, T, g_spatial, g_freq, g_dec, g_x, twW, ytab,
-                                                             xtab, jtab, plane0, C, h, w, H, W, sp_scale);
-    });
+    auto k = g_x ? rt_rows_bwd_kernel<UdAnyPlan, true> : rt_rows_bwd_kernel<UdAnyPlan, false>;
+    if ((rc = rt_set_smem(k, smW)) != UD_OK) return rc;
+    k<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(pW, dec, x, T, g_spatial, g_freq, g_dec, g_x, pW.tw, ytab, xtab,
+                                                           jtab, plane0, C, h, w, H, W, sp_scale);
     if ((rc = ud_check_launch("rt_rows_bwd")) != UD_OK) return rc;
   }
   return UD_OK;
-}
-
-extern "C" int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
-                                 const float* g_freq, float* g_dec, void* ws, size_t ws_bytes, int N, int C,
-                                 int h, int w, int H, int W, int norm_ortho, cudaStream_t stream) {
-  UD_REQUIRE(N == 0 || g_dec, UD_ERR_INVALID, "recon_tail_bwd: null pointer");
-  return rt_bwd(dec, x, signs, g_spatial, g_freq, g_dec, nullptr, ws, ws_bytes, N, C, h, w, H, W, norm_ortho, stream);
-}
-
-extern "C" int ud_recon_tail_bwd2(const float* dec, const float* x, const uint8_t* signs, const float* g_spatial,
-                                  const float* g_freq, float* g_dec, float* g_x, void* ws, size_t ws_bytes, int N, int C,
-                                  int h, int w, int H, int W, int norm_ortho, cudaStream_t stream) {
-  return rt_bwd(dec, x, signs, g_spatial, g_freq, g_dec, g_x, ws, ws_bytes, N, C, h, w, H, W, norm_ortho, stream);
 }

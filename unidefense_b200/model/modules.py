@@ -13,7 +13,6 @@ nn.Conv2d / nn.BatchNorm2d / nn.InstanceNorm2d child as the parameter holder so 
 SyncBatchNorm.convert_sync_batchnorm, DDP, weight-decay grouping and strict state_dict loading
 (engine/forgery_engine.py:142-154,:208) see the same tree as with the reference.
 """
-import os
 
 import torch
 import torch.distributed as dist
@@ -171,17 +170,13 @@ def bn_forward_stats(bn, proj, local=None):
     return mean, torch.rsqrt(var + bn.eps), (count if torch.is_tensor(count) else int(count)), reduce_fn
 
 
-# "tcgen05": our implicit-GEMM kernel (csrc/ud_proj.cu); "cudnn": the library convolution (A/B timing, UD_PROJ=cudnn)
-PROJ_BACKEND = os.environ.get("UD_PROJ", "tcgen05")
-
-
 class _DynamicFilter(nn.Module):
     def _mask(self, x, diff, want_out):
         conv, bn, act = self.layer1[0], self.layer1[1], self.layer1[2]
         x = x.float()
         use_batch = bn.training or bn.running_mean is None
         local = None
-        if PROJ_BACKEND == "tcgen05" and ops.proj_supported(x, conv):
+        if ops.proj_supported(x, conv):
             # layer1[0] on the tensor cores (tcgen05 implicit GEMM); its epilogue already holds the batch statistics
             proj, pm, p2 = ops.proj_conv(x, conv.weight, want_stats=use_batch)
             local = (pm, p2) if use_batch else None

@@ -11,18 +11,10 @@ The north star keeps the backbone on stock torch, so this file is plain PyTorch;
 computed in fp32 even under bf16 autocast (torch.complex rejects bf16, SURVEY.md §0).
 """
 import math
-import os
 
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
-
-
-# SURVEY.md §8(f) #1, first step: on CUDA the ~10 elementwise / layout / dtype passes torch makes around the two
-# FFTs and the 1x1 convolution (x.float, real, imag, cat, cast, tensor_split, complex, two muls, add and their
-# backward twins) are replaced by three single-pass kernels (ops.sf_pack / sf_unpack / sf_mix); cuFFT and the
-# convolution stay library calls.  UD_SFCONV_GLUE=0 restores the plain composition (used by the CPU oracle arm).
-USE_GLUE_KERNELS = os.environ.get("UD_SFCONV_GLUE", "1") != "0"
 
 
 # Under bf16 autocast with channels-last activations (the benchmark configuration) the two small 2-D transforms are
@@ -35,14 +27,9 @@ USE_GLUE_KERNELS = os.environ.get("UD_SFCONV_GLUE", "1") != "0"
 #     y = A  @ G.view(N*h, 4wh, C)         A [w x 4wh]  folds the complex product and the Hermitian weights m_k
 # Four batched library GEMMs replace copy->fp32, R2C, C2C, pack, unpack, C2R and their backward twins; autograd
 # differentiates the matmuls.  Exact fp32 runs keep the cuFFT path (bf16 twiddles carry ~3 significant digits).
-USE_DFT_GEMM = os.environ.get("UD_SFCONV_DFT_GEMM", "1") != "0"
 # largest side evaluated as DFT-by-GEMM: 96 covers every SFConv layer of the shipped configs (95^2 at EB4@380 is the
 # biggest: with it on the GEMM path the step went 77.2 -> 74.0 ms on a B200; 64 was the round-1 setting)
-_DFT_MAX = int(os.environ.get("UD_SFCONV_DFT_MAX", "96"))
-# fp32 path on this repo's own transforms instead of cuFFT (opt-in): ud_rfft2 emits the cat([re, im], 1) planar spectrum
-# the 1x1 convolution consumes and ud_irfft2 takes it back, so the pack / unpack passes disappear as well; any plane size,
-# autograd through the kernels' adjoint modes.  Off by default: the library path is what the timings were taken on.
-USE_OWN_FFT = os.environ.get("UD_SFCONV_OWN_FFT", "0") == "1"
+_DFT_MAX = 96
 _dft_cache = {}
 
 
@@ -77,10 +64,10 @@ def _dft_mats(h, w, norm, device):
     return mats
 
 
-def _dft_gemm_ok(x, spat):
+def _dft_gemm_ok(x):
     h, w = x.shape[-2:]
     # bf16 autocast only: under fp16 autocast (or none) the transforms stay on the fp32 cuFFT path (ADVICE r1)
-    return (USE_DFT_GEMM and x.is_cuda and torch.is_autocast_enabled() and torch.get_autocast_dtype("cuda") == torch.bfloat16
+    return (x.is_cuda and torch.is_autocast_enabled() and torch.get_autocast_dtype("cuda") == torch.bfloat16
             and x.dim() == 4 and h <= _DFT_MAX and w <= _DFT_MAX
             and x.is_contiguous(memory_format=torch.channels_last) and not x.is_contiguous())
 
@@ -104,37 +91,28 @@ def _sf_forward_gemm(x, spat, freq_conv, sf_coef, norm):
     return torch.lerp(spat, y.to(spat.dtype), torch.sigmoid(sf_coef).to(spat.dtype))
 
 
-def _sf_forward(x, spat, freq_conv, sf_coef, norm):
-    """(1 - sigmoid(sf_coef)) * spat + sigmoid(sf_coef) * pool(irfft2(freq_conv(cat rfft2(x))))."""
+# SURVEY.md §8(f) #1, first step: on CUDA the ~10 elementwise / layout / dtype passes torch makes around the two
+# FFTs and the 1x1 convolution (x.float, real, imag, cat, cast, tensor_split, complex, two muls, add and their
+# backward twins) are replaced by three single-pass kernels (ops.sf_pack / sf_unpack / sf_mix); cuFFT and the
+# convolution stay library calls.
+def _sf_forward_glue(x, spat, freq_conv, sf_coef, norm):
+    from .. import ops
     size = x.shape[-2:]
-    if _dft_gemm_ok(x, spat):
-        return _sf_forward_gemm(x, spat, freq_conv, sf_coef, norm)
-    if USE_OWN_FFT and x.is_cuda and not torch.is_autocast_enabled():
-        from .. import ops
-        planar = freq_conv(ops.rfft2_cat(x.float().contiguous(), norm))
-        y = ops.irfft2_cat(planar.float().contiguous(), size, norm)
-        if tuple(y.shape[-2:]) != tuple(spat.shape[-2:]):
-            y = F.adaptive_avg_pool2d(y, spat.shape[-2:])
-        return ops.sf_mix(spat, y, sf_coef)
-    if USE_GLUE_KERNELS and x.is_cuda:
-        from .. import ops
-        xf = x.to(dtype=torch.float32, memory_format=torch.contiguous_format)
-        with torch.autocast(device_type="cuda", enabled=False):
-            spec = torch.fft.rfft2(xf, norm=norm)
-        cl = spat.dim() == 4 and spat.is_contiguous(memory_format=torch.channels_last) and not spat.is_contiguous()
-        planar = ops.sf_pack(spec, spat.dtype if spat.dtype in (torch.float32, torch.bfloat16) else torch.float32, cl)
-        planar = freq_conv(planar)
-        with torch.autocast(device_type="cuda", enabled=False):
-            y = torch.fft.irfft2(ops.sf_unpack(planar), s=size, norm=norm)
-        if tuple(y.shape[-2:]) != tuple(spat.shape[-2:]):
-            y = F.adaptive_avg_pool2d(y, spat.shape[-2:])
-        return ops.sf_mix(spat, y, sf_coef)
-    freq = _freq_branch(x, freq_conv, spat.shape[-2:], norm)
-    gate = torch.sigmoid(sf_coef)
-    return (1.0 - gate) * spat + gate * freq
+    xf = x.to(dtype=torch.float32, memory_format=torch.contiguous_format)
+    with torch.autocast(device_type="cuda", enabled=False):
+        spec = torch.fft.rfft2(xf, norm=norm)
+    cl = spat.dim() == 4 and spat.is_contiguous(memory_format=torch.channels_last) and not spat.is_contiguous()
+    planar = ops.sf_pack(spec, spat.dtype if spat.dtype in (torch.float32, torch.bfloat16) else torch.float32, cl)
+    planar = freq_conv(planar)
+    with torch.autocast(device_type="cuda", enabled=False):
+        y = torch.fft.irfft2(ops.sf_unpack(planar), s=size, norm=norm)
+    if tuple(y.shape[-2:]) != tuple(spat.shape[-2:]):
+        y = F.adaptive_avg_pool2d(y, spat.shape[-2:])
+    return ops.sf_mix(spat, y, sf_coef)
 
 
-def _freq_branch(x, freq_conv, out_hw, norm):
+# The plain torch composition of the reference: the CPU path (the oracle arm).
+def _sf_forward_plain(x, spat, freq_conv, sf_coef, norm):
     size = x.shape[-2:]
     with torch.autocast(device_type=x.device.type, enabled=False):
         spec = torch.fft.rfft2(x.float(), norm=norm)
@@ -143,9 +121,19 @@ def _freq_branch(x, freq_conv, out_hw, norm):
     with torch.autocast(device_type=x.device.type, enabled=False):
         re, im = torch.tensor_split(planar.float(), 2, dim=1)
         y = torch.fft.irfft2(torch.complex(re, im), s=size, norm=norm)
-    if tuple(y.shape[-2:]) != tuple(out_hw):
-        y = F.adaptive_avg_pool2d(y, out_hw)
-    return y
+    if tuple(y.shape[-2:]) != tuple(spat.shape[-2:]):
+        y = F.adaptive_avg_pool2d(y, spat.shape[-2:])
+    gate = torch.sigmoid(sf_coef)
+    return (1.0 - gate) * spat + gate * y
+
+
+def _sf_forward(x, spat, freq_conv, sf_coef, norm):
+    """(1 - sigmoid(sf_coef)) * spat + sigmoid(sf_coef) * pool(irfft2(freq_conv(cat rfft2(x))))."""
+    if _dft_gemm_ok(x):
+        return _sf_forward_gemm(x, spat, freq_conv, sf_coef, norm)
+    if x.is_cuda:
+        return _sf_forward_glue(x, spat, freq_conv, sf_coef, norm)
+    return _sf_forward_plain(x, spat, freq_conv, sf_coef, norm)
 
 
 class SFConv2d(nn.Conv2d):

@@ -58,17 +58,12 @@ class _ReconTail(torch.autograd.Function):
             gs = (g_spatial if g_spatial is not None else torch.zeros(N, device=x.device)).contiguous().float()
             gf = (g_freq if g_freq is not None else torch.zeros(N, device=x.device)).contiguous().float()
             g_dec = torch.empty_like(dec) if need_dec else None
+            g_x = torch.empty_like(x) if need_x else None
             nws = lib.ud_recon_tail_workspace_bytes(N, C, h, w, H, W)
             ws = L.workspace(nws, x.device)
-            if need_x:
-                g_x = torch.empty_like(x)
-                L.check(lib.ud_recon_tail_bwd2(L.ptr(dec), L.ptr(x), L.ptr(signs), L.ptr(gs), L.ptr(gf), L.ptr(g_dec),
-                                               L.ptr(g_x), L.ptr(ws), ws.numel(), N, C, h, w, H, W, ctx.norm_ortho,
-                                               L.stream()), "recon_tail_bwd2")
-            else:
-                L.check(lib.ud_recon_tail_bwd(L.ptr(dec), L.ptr(x), L.ptr(signs), L.ptr(gs), L.ptr(gf), L.ptr(g_dec),
-                                              L.ptr(ws), ws.numel(), N, C, h, w, H, W, ctx.norm_ortho, L.stream()),
-                        "recon_tail_bwd")
+            L.check(lib.ud_recon_tail_bwd(L.ptr(dec), L.ptr(x), L.ptr(signs), L.ptr(gs), L.ptr(gf), L.ptr(g_dec),
+                                          L.ptr(g_x), L.ptr(ws), ws.numel(), N, C, h, w, H, W, ctx.norm_ortho, L.stream()),
+                    "recon_tail_bwd")
         if g_rec is not None and need_dec:
             # rec = interpolate(dec) is differentiable in the reference (model/unidefense.py:244); the shipped engines
             # never use that gradient, but a loss on out['rec'] gets the transposed resize, not silent zeros
@@ -537,18 +532,12 @@ class _DyfiMask(torch.autograd.Function):
         dz = torch.empty_like(proj)
         g_w2 = torch.empty(2 + D, device=dev, dtype=torch.float32)
         ws = L.workspace(lib.ud_dyfi_mask_bwd_workspace_bytes(N, HW), dev)
-        g_diff = None
-        if ctx.needs_input_grad[5]:          # the error maps carry x's gradient (model/modules.py:101-103, :130-132)
-            g_diff = torch.empty_like(diff)
-            L.check(lib.ud_dyfi_mask_bwd2(L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(gamma), L.ptr(beta), L.ptr(diff),
-                                          L.ptr(w2f), L.ptr(x), L.ptr(mask), L.ptr(pmean), L.ptr(pmax), L.ptr(argmax),
-                                          L.ptr(g_mask), L.ptr(g_out), L.ptr(g_x), L.ptr(dz), L.ptr(g_w2), L.ptr(g_diff),
-                                          L.ptr(ws), ws.numel(), N, Cp, D, Cx, HW, ctx.act, L.stream()), "dyfi_mask_bwd2")
-        else:
-            L.check(lib.ud_dyfi_mask_bwd(L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(gamma), L.ptr(beta), L.ptr(diff),
-                                         L.ptr(w2f), L.ptr(x), L.ptr(mask), L.ptr(pmean), L.ptr(pmax), L.ptr(argmax),
-                                         L.ptr(g_mask), L.ptr(g_out), L.ptr(g_x), L.ptr(dz), L.ptr(g_w2), L.ptr(ws),
-                                         ws.numel(), N, Cp, D, Cx, HW, ctx.act, L.stream()), "dyfi_mask_bwd")
+        # the error maps carry x's gradient (model/modules.py:101-103, :130-132)
+        g_diff = torch.empty_like(diff) if ctx.needs_input_grad[5] else None
+        L.check(lib.ud_dyfi_mask_bwd(L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(gamma), L.ptr(beta), L.ptr(diff),
+                                     L.ptr(w2f), L.ptr(x), L.ptr(mask), L.ptr(pmean), L.ptr(pmax), L.ptr(argmax),
+                                     L.ptr(g_mask), L.ptr(g_out), L.ptr(g_x), L.ptr(dz), L.ptr(g_w2), L.ptr(g_diff),
+                                     L.ptr(ws), ws.numel(), N, Cp, D, Cx, HW, ctx.act, L.stream()), "dyfi_mask_bwd")
         sums = torch.empty(2, Cp, device=dev, dtype=torch.float32)
         L.check(lib.ud_bn_bwd_reduce(L.ptr(dz), L.ptr(proj), L.ptr(mean), L.ptr(rstd), L.ptr(sums[0]), L.ptr(sums[1]),
                                      N, Cp, HW, L.stream()), "bn_bwd_reduce")
