@@ -21,7 +21,7 @@
  *  - reductions are fixed-order (bitwise reproducible) except ud_recon_tail_bwd's g_dec and ud_bilinear_ac_bwd,
  *    whose transposed resize accumulates with float atomics.  The input-gradient outputs (g_x of ud_recon_tail_bwd,
  *    ud_attn_prep_bwd, ud_gaussian_blur5_bwd, ud_downscale_nearest_bwd; g_diff of ud_dyfi_mask_bwd) are gathers
- *    written once per element: bitwise reproducible.
+ *    written once per element: bitwise reproducible.  ud_attack_step's per-sample norms are fixed-order too.
  */
 #ifndef UNIDEFENSE_B200_H
 #define UNIDEFENSE_B200_H
@@ -43,7 +43,7 @@ typedef struct CUstream_st* cudaStream_t;
 #define UD_API
 #endif
 
-#define UD_B200_VERSION 101
+#define UD_B200_VERSION 102
 #define UD_FFT_MAX_N 1024
 
 #define UD_ACT_NONE 0
@@ -293,6 +293,27 @@ UD_API size_t ud_sf_mix_bwd_workspace_bytes(int N, int C, int P);
 UD_API int ud_sf_mix_bwd(const void* g_out, const void* spat, const float* freq, const float* coef, void* g_spat,
                          float* g_freq, float* g_coef, void* ws, size_t ws_bytes, int N, int C, int P, int nhwc,
                          int bf16, cudaStream_t stream);
+
+/* ---- a19: projected-gradient attack step (PGD / FGSM robustness evaluation) ---------------------------------------
+ * One iteration's image-sized work for a batch, per sample n, mirroring oracle/attack.py operation for operation in
+ * fp32 with explicit rounding (no FMA contraction; sign(0) = 0 as torch.sign):
+ *  1. select: if loss[n] > best_loss[n] (strict: a NaN loss never improves), best_loss[n] = loss[n] and
+ *     x_best[n] = x_adv[n] as it was BEFORE this call's step; other samples keep x_best / best_loss bit for bit.
+ *  2. step (skipped when g == NULL: "select only", for the iterate after the last forward):
+ *     UD_NORM_LINF: x_adv = clamp(x0 + clamp((x_adv + alpha*sign(g)) - x0, -eps, eps), lo, hi)
+ *     UD_NORM_L2:   u = g / (||g_n||_2 + 1e-12); d = x_adv + alpha*u - x0; d *= min(1, eps/||d_n||_2) (0/0 -> 1);
+ *                   x_adv = clamp(x0 + d, lo, hi)
+ * x0, x_adv, g, x_best [N, per_sample] (any per_sample >= 1); loss, best_loss, eps, alpha [N], all fp32 device memory
+ * (eps / alpha on the device so one captured graph serves an eps sweep; both may be NULL for a select-only call).
+ * x_adv, best_loss, x_best are updated in place; x_best must not alias x_adv.  The L2 norms are fixed-order sums of
+ * per-CTA partials kept in ws (ud_attack_workspace_bytes): two calls on the same inputs are bitwise identical.
+ * Launches: 2 (L-inf, select only) or 3 (L2).  N <= 65535.                                                         */
+#define UD_NORM_LINF 0
+#define UD_NORM_L2 2
+UD_API size_t ud_attack_workspace_bytes(int N, long long per_sample);
+UD_API int ud_attack_step(const float* x0, float* x_adv, const float* g, const float* loss, float* best_loss,
+                          float* x_best, const float* eps, const float* alpha, float lo, float hi, int norm, int N,
+                          long long per_sample, void* ws, size_t ws_bytes, cudaStream_t stream);
 
 /* ---- §8(e): the exchange step -- SyncBatchNorm statistics over NVLink peer memory ----------------------------------
  * Replaces the two per-layer collectives of torch.nn.SyncBatchNorm (engine/forgery_engine.py:142 converts all 99

@@ -938,3 +938,34 @@ class _SfMix(torch.autograd.Function):
 
 def sf_mix(spat, freq, coef):
     return _SfMix.apply(spat, freq, coef)
+
+
+# ------------------------------------------------------------------------------------------
+# a19: projected-gradient attack step (unidefense_b200/attack.py)
+# ------------------------------------------------------------------------------------------
+ATTACK_NORMS = {"linf": 0, "l2": 2}
+
+
+def attack_step(x0, x_adv, g, loss, best_loss, x_best, eps, alpha, lo, hi, norm="linf"):
+    """One PGD iteration in place (csrc/ud_attack.cu): best-iterate select of x_adv by `loss`, then (unless g is None)
+    the step under `norm` ('linf' | 'l2'), the projection onto the eps-ball around x0 and the clamp to [lo, hi].
+    x0, x_adv, g, x_best: fp32 [N, ...] of one shape; loss, best_loss, eps, alpha: fp32 [N] (eps / alpha may be None
+    for a select-only call).  Updates x_adv, best_loss and x_best; the attack state is not differentiated."""
+    if norm not in ATTACK_NORMS:
+        raise ValueError(f"attack_step: norm must be one of {sorted(ATTACK_NORMS)}, got {norm!r}")
+    L.require_cuda_f32(x0, x_adv, g, loss, best_loss, x_best, eps, alpha)
+    N = x0.shape[0]
+    if x_adv.shape != x0.shape or x_best.shape != x0.shape or (g is not None and g.shape != x0.shape):
+        raise ValueError("attack_step: x0, x_adv, g and x_best must share one shape")
+    for name, t in (("loss", loss), ("best_loss", best_loss), ("eps", eps), ("alpha", alpha)):
+        if t is not None and t.numel() != N:
+            raise ValueError(f"attack_step: {name} has {t.numel()} entries for a batch of {N}")
+    if g is not None and (eps is None or alpha is None):
+        raise ValueError("attack_step: a step needs eps and alpha")
+    per_sample = x0.numel() // max(N, 1)
+    lib = L.lib()
+    nws = lib.ud_attack_workspace_bytes(N, per_sample)
+    ws = L.workspace(nws, x0.device)
+    L.check(lib.ud_attack_step(L.ptr(x0), L.ptr(x_adv), L.ptr(g), L.ptr(loss), L.ptr(best_loss), L.ptr(x_best),
+                               L.ptr(eps), L.ptr(alpha), float(lo), float(hi), ATTACK_NORMS[norm], N, per_sample,
+                               L.ptr(ws), ws.numel(), L.stream()), "attack_step")
