@@ -22,6 +22,7 @@
  *    whose transposed resize accumulates with float atomics.  The input-gradient outputs (g_x of ud_recon_tail_bwd,
  *    ud_attn_prep_bwd, ud_gaussian_blur5_bwd, ud_downscale_nearest_bwd; g_diff of ud_dyfi_mask_bwd) are gathers
  *    written once per element: bitwise reproducible.  ud_attack_step's per-sample norms are fixed-order too.
+ *    ud_corrupt writes every output element once from a fixed-order computation: bitwise reproducible.
  */
 #ifndef UNIDEFENSE_B200_H
 #define UNIDEFENSE_B200_H
@@ -43,7 +44,7 @@ typedef struct CUstream_st* cudaStream_t;
 #define UD_API
 #endif
 
-#define UD_B200_VERSION 102
+#define UD_B200_VERSION 103
 #define UD_FFT_MAX_N 1024
 
 #define UD_ACT_NONE 0
@@ -314,6 +315,46 @@ UD_API size_t ud_attack_workspace_bytes(int N, long long per_sample);
 UD_API int ud_attack_step(const float* x0, float* x_adv, const float* g, const float* loss, float* best_loss,
                           float* x_best, const float* eps, const float* alpha, float lo, float hi, int norm, int N,
                           long long per_sample, void* ws, size_t ws_bytes, cudaStream_t stream);
+
+/* ---- a20: image corruptions (corruption-robustness evaluation; DeeperForensics-1.0 / LipForensics protocol) -----------
+ * y = corruption of x, x and y fp32 [N, 3, H, W] (channels R, G, B, values in [lo, hi]; y must not overlap x).  Each
+ * kind maps x to 8-bit levels p = clamp(rint((x - lo)*s), 0, 255) with s = 255/(hi - lo) (fp64 on the host, used as
+ * fp32), corrupts p, rounds with rint, clamps to [0, 255] and writes y = lo + p'*(1/s): outputs lie on the 8-bit grid.
+ * Colour space: JFIF full-range BT.601 on levels, Y = .299R + .587G + .114B, Cb = -.168736R - .331264G + .5B + 128,
+ * Cr = .5R - .418688G - .081312B + 128; inverse R = Y + 1.402(Cr-128), G = Y - .344136(Cb-128) - .714136(Cr-128),
+ * B = Y + 1.772(Cb-128).  `param` is the severity parameter:
+ *  SATURATION s in [0, 1]: Cb' = 128 + (Cb-128)*s, likewise Cr, back to RGB.
+ *  CONTRAST   c in [0, 1]: p' = p*c.
+ *  BLOCK      k in 0..4096: k 8x8 squares set to level 128 in all channels; square j's top-left corner is
+ *             r = (u0*(H-7)) >> 32, c = (u1*(W-7)) >> 32 (64-bit products) with (u0, u1, ...) = Philox4x32-10(ctr =
+ *             (j, id_lo, id_hi, 0), key = (seed_lo, seed_hi ^ 0x424C4F43)).  H, W >= 8.
+ *  NOISE      sigma^2 in [0, 1]: in YCbCr/255 add sigma*z to Y, Cb, Cr; z0, z1 by Box-Muller from words (a, b) and z2 from
+ *             (c, d) of Philox4x32-10(ctr = (h*W + w, id_lo, id_hi, 0), key = (seed_lo, seed_hi ^ 0x4E4F4953)), with
+ *             u1 = (a + 0.5)*2^-32, u2 = b*2^-32, z0 = sqrt(-2 ln u1) cos(2 pi u2), z1 = ... sin(2 pi u2).
+ *  BLUR       odd k in 1..31: separable Gaussian, w_i ~ exp(-i^2 / (2 sigma^2)), sigma = k/6, normalised, |i| <= (k-1)/2;
+ *             reflect-101 borders (OpenCV's default).  H, W > (k-1)/2.
+ *  PIXELATE   f in 1..64: mean of each f x f cell (partial cells at the bottom / right average their valid pixels),
+ *             rounded, replicated over the cell.
+ *  JPEG       q in 1..100: baseline JPEG round trip, 4:2:0: YCbCr; chroma 2x2 mean (edge replication at odd sizes);
+ *             planes padded to whole 8x8 blocks by edge replication; per block orthonormal DCT-II of v - 128 (JPEG's
+ *             FDCT scaling), quantised rha(F/Q)*Q (rha: round half away from zero) with the ITU-T T.81 Annex K tables
+ *             scaled as libjpeg does (S = 5000/q if q < 50 else 200 - 2q; Q = clamp((T*S + 50) div 100, 1, 255)),
+ *             orthonormal IDCT + 128; chroma upsampled with libjpeg's triangle ("fancy") filter; back to RGB.
+ *             ws = ud_corrupt_workspace_bytes(JPEG, N, H, W) bytes (0 for every other kind).
+ * ids: int64 [N] device array keying the random kinds per sample (id_lo / id_hi its two 32-bit halves), or NULL for
+ * ids 0..N-1, so image i gets the same corruption in any batch.  saturation, contrast, block and pixelate are
+ * bit-identical to oracle/corrupt.py (fp32, explicit rounding); noise, blur and jpeg restate its fp64 definitions in
+ * fp32 (jpeg's forward DCT and quantisation in fp64).  Launches: 1, or 2 for block and jpeg.  N <= 65535, H, W <= 8192. */
+#define UD_CORRUPT_SATURATION 0
+#define UD_CORRUPT_CONTRAST 1
+#define UD_CORRUPT_BLOCK 2
+#define UD_CORRUPT_NOISE 3
+#define UD_CORRUPT_BLUR 4
+#define UD_CORRUPT_PIXELATE 5
+#define UD_CORRUPT_JPEG 6
+UD_API size_t ud_corrupt_workspace_bytes(int kind, int N, int H, int W);
+UD_API int ud_corrupt(const float* x, float* y, const long long* ids, int N, int H, int W, int kind, float param,
+                      unsigned long long seed, float lo, float hi, void* ws, size_t ws_bytes, cudaStream_t stream);
 
 /* ---- §8(e): the exchange step -- SyncBatchNorm statistics over NVLink peer memory ----------------------------------
  * Replaces the two per-layer collectives of torch.nn.SyncBatchNorm (engine/forgery_engine.py:142 converts all 99

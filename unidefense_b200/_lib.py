@@ -93,6 +93,8 @@ SIGNATURES = {
     "ud_kl_div_log_target_fwd": (c_i, [c_p] * 5 + [c_sz, c_i, c_i, c_p]),
     "ud_attack_workspace_bytes": (c_sz, [c_i, ctypes.c_longlong]),
     "ud_attack_step": (c_i, [c_p] * 8 + [c_f, c_f, c_i, c_i, ctypes.c_longlong, c_p, c_sz, c_p]),
+    "ud_corrupt_workspace_bytes": (c_sz, [c_i] * 4),
+    "ud_corrupt": (c_i, [c_p] * 3 + [c_i] * 4 + [c_f, ctypes.c_ulonglong, c_f, c_f, c_p, c_sz, c_p]),
 }
 
 

@@ -969,3 +969,36 @@ def attack_step(x0, x_adv, g, loss, best_loss, x_best, eps, alpha, lo, hi, norm=
     L.check(lib.ud_attack_step(L.ptr(x0), L.ptr(x_adv), L.ptr(g), L.ptr(loss), L.ptr(best_loss), L.ptr(x_best),
                                L.ptr(eps), L.ptr(alpha), float(lo), float(hi), ATTACK_NORMS[norm], N, per_sample,
                                L.ptr(ws), ws.numel(), L.stream()), "attack_step")
+
+
+# ------------------------------------------------------------------------------------------
+# a20: image corruptions (unidefense_b200/corrupt.py)
+# ------------------------------------------------------------------------------------------
+CORRUPT_KINDS = {"saturation": 0, "contrast": 1, "block": 2, "noise": 3, "blur": 4, "pixelate": 5, "jpeg": 6}
+
+
+def corrupt(x, kind, param, ids=None, seed=0, lo=-1.0, hi=1.0):
+    """y = corruption `kind` of x at severity parameter `param` (csrc/ud_corrupt.cu; definitions in
+    include/unidefense_b200.h).  x: contiguous fp32 [N, 3, H, W] in [lo, hi]; ids: int64 [N] per-sample keys of the
+    random kinds (None: 0..N-1); seed: uint64.  No autograd: y has no gradient and x is not differentiated."""
+    if kind not in CORRUPT_KINDS:
+        raise ValueError(f"corrupt: kind must be one of {sorted(CORRUPT_KINDS)}, got {kind!r}")
+    L.require_cuda_f32(x)
+    if x.dim() != 4 or x.shape[1] != 3:
+        raise ValueError(f"corrupt: x must be [N, 3, H, W] RGB, got {tuple(x.shape)}")
+    N, _, H, W = x.shape
+    if ids is not None:
+        if not ids.is_cuda or ids.device != x.device or ids.dtype != torch.int64 or ids.numel() != N:
+            raise ValueError(f"corrupt: ids must be an int64 tensor of {N} entries on {x.device}")
+        ids = ids.contiguous()
+    seed = int(seed)
+    if not 0 <= seed < 2 ** 64:
+        raise ValueError(f"corrupt: seed {seed} is not a uint64")
+    y = torch.empty_like(x)
+    lib = L.lib()
+    k = CORRUPT_KINDS[kind]
+    nws = lib.ud_corrupt_workspace_bytes(k, N, H, W)
+    ws = L.workspace(nws, x.device) if nws else None
+    L.check(lib.ud_corrupt(L.ptr(x.detach()), L.ptr(y), L.ptr(ids), N, H, W, k, float(param), seed, float(lo),
+                           float(hi), L.ptr(ws), nws, L.stream()), "corrupt")
+    return y
