@@ -64,6 +64,8 @@ UD_API int ud_fft_size_any(int n);
  * Replaces model/unidefense.py:244-253 (Eb4), :423-433 (Res18), :618-628 (Res50):
  *   interpolate(dec, x.shape[-2:]) ; abs(rec-x).mean ; rfft2 x2 ; cat ; abs ; tensor_split ; mean.
  * dec [N,C,h,w], x [N,C,H,W] -> rec [N,C,H,W], spatial [N], freq [N].
+ * Any 1 <= H, W <= UD_FFT_MAX_N.  The decoder width w shares shared memory with one row FFT: every w <= 2214 fits
+ * at every W; a wider decoder that does not fit is rejected (UD_ERR_UNSUPPORTED) before any launch.
  * signs (nullable; ud_recon_tail_signs_bytes) receives 1 byte per spectral bin (sign codes of
  * Re/Im dF) and is what backward needs instead of the two saved spectra.                    */
 UD_API size_t ud_recon_tail_workspace_bytes(int N, int C, int h, int w, int H, int W);

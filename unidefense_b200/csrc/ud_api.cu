@@ -248,6 +248,15 @@ static void host_fft_pow2(std::vector<double>& re, std::vector<double>& im) {
   }
 }
 
+int ud_any_line_len(int n) {
+  if (n < 1 || n > UD_FFT_MAX_N) return 0;
+  UdDynPlan p;
+  if (ud_make_dyn_plan(n, &p)) return n;
+  int m = 1;
+  while (m < 2 * n - 1) m <<= 1;
+  return m;
+}
+
 bool ud_make_any_plan(int n, UdAnyPlan* plan) {
   if (n < 1 || n > UD_FFT_MAX_N) {
     ud_set_error("FFT size %d outside [1, %d]", n, UD_FFT_MAX_N);
@@ -262,8 +271,7 @@ bool ud_make_any_plan(int n, UdAnyPlan* plan) {
     plan->tw = ud_twiddles(n);
     return plan->tw != nullptr;
   }
-  int m = 1;
-  while (m < 2 * n - 1) m <<= 1;
+  const int m = ud_any_line_len(n);
   plan->m = m;
   plan->bluestein = 1;
   if (!ud_make_dyn_plan(m, &plan->inner)) {

@@ -39,11 +39,8 @@ static bool f2_static(int n) { return n == 380 || n == 256 || n == 224 || n == 2
   } while (0)
 
 static int f2_lines(const UdAnyPlan& p) {
-  const size_t per = 2ull * (size_t)ud_any_line_stride(p) * sizeof(float2);
-  int L = (int)((96u << 10) / per);
-  if (L > 16) L = 16;
-  if (L < 1) L = 1;
-  return L;
+  const int L = ud_any_lines(p.m, 0, 0, 96u << 10, 16);   // 96 KB of line buffers (the twiddles come on top)
+  return L < 1 ? 1 : L;
 }
 static size_t f2_smem(const UdAnyPlan& p, int L) {
   return sizeof(float2) * ((size_t)p.m + 2ull * L * ud_any_line_stride(p));

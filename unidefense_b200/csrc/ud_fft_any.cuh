@@ -64,5 +64,34 @@ struct UdAnyPlan {
 // Host: fills `plan` for any 1 <= n <= UD_FFT_MAX_N (tables cached per (device, n), created on first use -- not
 // during a CUDA-graph capture).  Returns false (error set) on failure.
 bool ud_make_any_plan(int n, UdAnyPlan* plan);
+// Host: the working length m of n's plan (n, or Bluestein's power of two >= 2n-1) without creating the plan; 0 outside
+// [1, UD_FFT_MAX_N].
+int ud_any_line_len(int n);
 // odd line stride for a plan's line buffers
 static inline int ud_any_line_stride(const UdAnyPlan& p) { return p.m | 1; }
+
+#define UD_SMEM_CTA_MAX (227u << 10)   // dynamic shared memory one CTA may use on sm_100a
+
+// Host: lines per CTA of a kernel that keeps two ping-pong buffers of (m | 1) points per line: the largest L <= lmax for
+// which `fixed` bytes (staged twiddles, tables) plus L * (two line buffers + `per_line` other bytes) fit in `budget`
+// bytes; 0 when not even one line fits.  Every shared-memory line-FFT kernel sizes its lines here.
+static inline int ud_any_lines(int m, size_t fixed, size_t per_line, size_t budget, int lmax) {
+  const size_t line = 2 * sizeof(float2) * (size_t)(m | 1) + per_line;
+  if (budget < fixed + line) return 0;
+  const size_t L = (budget - fixed) / line;
+  return L < (size_t)lmax ? (int)L : lmax;
+}
+// Kernels instantiated at lmax, lmax/2 and lmax/4 lines per CTA: the largest of those <= fit (a ud_any_lines result);
+// 0 when none is.
+static inline int ud_halving_lines(int fit, int lmax) {
+  for (int L = lmax; L >= lmax / 4 && L >= 1; L /= 2)
+    if (L <= fit) return L;
+  return 0;
+}
+// runs the body with `constexpr int LV` bound to L, which is one of X, X/2 and X/4 (a ud_halving_lines result)
+#define UD_LINES_DISPATCH(L, X, LV, ...)                                 \
+  do {                                                                   \
+    if ((L) == (X)) { constexpr int LV = (X); __VA_ARGS__; }             \
+    else if ((L) == (X) / 2) { constexpr int LV = (X) / 2; __VA_ARGS__; } \
+    else { constexpr int LV = (X) / 4; __VA_ARGS__; }                    \
+  } while (0)

@@ -18,10 +18,12 @@
 #define FS_COL_T 320
 #define FS_COL_L 16   // lines per cols CTA: 8 content columns + 8 style columns
 #define FS_COL_K 8
+// Lines longer than shared memory holds at those counts (long Bluestein lines, m = 1024 or 2048) run instantiations
+// with a half or a quarter of them: fs_row_lines / fs_col_k pick the largest that fits.
 
 static inline int fs_whp(int W) { return ((W / 2 + 1) + 7) & ~7; }
 
-template <class Plan>
+template <class Plan, int L>
 __global__ void __launch_bounds__(FS_ROW_T)
 fs_rows_fwd_kernel(Plan plan, const float* __restrict__ a, const float* __restrict__ b, float2* __restrict__ Ya,
                    float2* __restrict__ Yb, const float2* __restrict__ tw_g, int plane0, int H, int W) {
@@ -31,17 +33,17 @@ fs_rows_fwd_kernel(Plan plan, const float* __restrict__ a, const float* __restri
   const int LS = m | 1;
   float2* tw = smem;
   float2* buf0 = tw + m;
-  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + FS_ROW_L * LS;
+  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + L * LS;
   W = n;
   const int Wh = n / 2 + 1;
   const int WhP = (Wh + 7) & ~7;
   const int pl = blockIdx.y;
   const long long plane = plane0 + pl;
-  const int r0 = blockIdx.x * FS_ROW_L;
+  const int r0 = blockIdx.x * L;
   for (int t = threadIdx.x; t < m; t += FS_ROW_T) tw[t] = __ldg(tw_g + t);
   const float* ap = a + plane * (long long)H * W;
   const float* bp = b + plane * (long long)H * W;
-  for (int p = 0; p < FS_ROW_L; ++p) {
+  for (int p = 0; p < L; ++p) {
     const int r = r0 + p;
     float2* line = buf0 + p * LS;
     if (r < H) {
@@ -56,10 +58,10 @@ fs_rows_fwd_kernel(Plan plan, const float* __restrict__ a, const float* __restri
   ud_cp_async_commit();
   ud_cp_async_wait_all();
   __syncthreads();
-  float2* res = plan.run(buf0, buf1, tw, FS_ROW_L, LS);
+  float2* res = plan.run(buf0, buf1, tw, L, LS);
   float2* Yap = Ya + (long long)pl * H * WhP;
   float2* Ybp = Yb + (long long)pl * H * WhP;
-  for (int t = threadIdx.x; t < FS_ROW_L * Wh; t += FS_ROW_T) {
+  for (int t = threadIdx.x; t < L * Wh; t += FS_ROW_T) {
     const int p = t / Wh, k = t - p * Wh;
     const int r = r0 + p;
     if (r >= H) continue;
@@ -70,44 +72,46 @@ fs_rows_fwd_kernel(Plan plan, const float* __restrict__ a, const float* __restri
   }
 }
 
-// Plan16 transforms all FS_COL_L lines (forward), Plan8 the first FS_COL_K lines (inverse of the mix).
-template <class Plan16, class Plan8>
+// K column pairs per CTA (FS_COL_K for every static plan): Plan16 transforms all 2K lines (forward), Plan8 the first K
+// lines (inverse of the mix).
+template <class Plan16, class Plan8, int K>
 __global__ void __launch_bounds__(FS_COL_T)
 fs_cols_kernel(Plan16 plan16, Plan8 plan8, float2* __restrict__ Ya, const float2* __restrict__ Yb,
                const float* __restrict__ lmda, const float2* __restrict__ tw_g, int plane0, int C, int H, int W) {
+  constexpr int NL = 2 * K;   // lines per CTA
   extern __shared__ float2 smem[];
   const int n = plan16.n();
   const int m = plan16.line_len();     // == n except for Bluestein plans
   const int LS = m | 1;
   float2* tw = smem;
   float2* buf0 = tw + m;
-  float2* buf1 = Plan16::kInPlace ? buf0 : buf0 + FS_COL_L * LS;
+  float2* buf1 = Plan16::kInPlace ? buf0 : buf0 + NL * LS;
   H = n;
   const int Wh = W / 2 + 1;
   const int WhP = (Wh + 7) & ~7;
   const int pl = blockIdx.y;
   const long long plane = plane0 + pl;
   const float lam = __ldg(lmda + plane / C);
-  const int k0 = blockIdx.x * FS_COL_K;
-  const int ncols = min(FS_COL_K, Wh - k0);
+  const int k0 = blockIdx.x * K;
+  const int ncols = min(K, Wh - k0);
   for (int t = threadIdx.x; t < m; t += FS_COL_T) tw[t] = __ldg(tw_g + t);
   float2* Yap = Ya + (long long)pl * H * WhP;
   const float2* Ybp = Yb + (long long)pl * H * WhP;
-  for (int t = threadIdx.x; t < H * FS_COL_L; t += FS_COL_T) {
-    const int r = t / FS_COL_L, l = t - r * FS_COL_L;
-    const int cc = l & (FS_COL_K - 1);
-    if (cc < ncols) ud_cp_async8(&buf0[l * LS + r], (l < FS_COL_K ? Yap : Ybp) + (long long)r * WhP + k0 + cc);
+  for (int t = threadIdx.x; t < H * NL; t += FS_COL_T) {
+    const int r = t / NL, l = t - r * NL;
+    const int cc = l & (K - 1);
+    if (cc < ncols) ud_cp_async8(&buf0[l * LS + r], (l < K ? Yap : Ybp) + (long long)r * WhP + k0 + cc);
     else buf0[l * LS + r] = make_float2(0.f, 0.f);
   }
   ud_cp_async_commit();
   ud_cp_async_wait_all();
   __syncthreads();
-  float2* res = plan16.run(buf0, buf1, tw, FS_COL_L, LS);
-  // mix in place into lines [0, FS_COL_K) of buf0 (swapped for the inverse transform)
-  for (int t = threadIdx.x; t < FS_COL_K * H; t += FS_COL_T) {
+  float2* res = plan16.run(buf0, buf1, tw, NL, LS);
+  // mix in place into lines [0, K) of buf0 (swapped for the inverse transform)
+  for (int t = threadIdx.x; t < K * H; t += FS_COL_T) {
     const int cc = t / H, j = t - cc * H;
     const float2 fa = res[cc * LS + j];
-    const float2 fb = res[(FS_COL_K + cc) * LS + j];
+    const float2 fb = res[(K + cc) * LS + j];
     const float am = sqrtf(fa.x * fa.x + fa.y * fa.y);
     const float bm = sqrtf(fb.x * fb.x + fb.y * fb.y);
     const float m = lam * am + (1.f - lam) * bm;
@@ -123,9 +127,9 @@ fs_cols_kernel(Plan16 plan16, Plan8 plan8, float2* __restrict__ Ya, const float2
   __syncthreads();
   // when the forward plan ping-ponged, `res` may be buf1: run the inverse from there
   float2* other = (res == buf0) ? buf1 : buf0;
-  float2* inv = plan8.run(res, other, tw, FS_COL_K, LS);
-  for (int t = threadIdx.x; t < H * FS_COL_K; t += FS_COL_T) {
-    const int r = t / FS_COL_K, cc = t - r * FS_COL_K;
+  float2* inv = plan8.run(res, other, tw, K, LS);
+  for (int t = threadIdx.x; t < H * K; t += FS_COL_T) {
+    const int r = t / K, cc = t - r * K;
     if (cc < ncols) {
       const float2 v = inv[cc * LS + r];
       Yap[(long long)r * WhP + k0 + cc] = make_float2(v.y, v.x);   // T overwrites the content spectrum rows
@@ -133,7 +137,7 @@ fs_cols_kernel(Plan16 plan16, Plan8 plan8, float2* __restrict__ Ya, const float2
   }
 }
 
-template <class Plan>
+template <class Plan, int L>
 __global__ void __launch_bounds__(FS_ROW_T)
 fs_rows_inv_kernel(Plan plan, const float2* __restrict__ T, float* __restrict__ out, const float2* __restrict__ tw_g,
                    int plane0, int H, int W, float scale) {
@@ -143,18 +147,18 @@ fs_rows_inv_kernel(Plan plan, const float2* __restrict__ T, float* __restrict__ 
   const int LS = m | 1;
   float2* tw = smem;
   float2* buf0 = tw + m;
-  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + FS_ROW_L * LS;
+  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + L * LS;
   W = n;
   const int Wh = n / 2 + 1;
   const int WhP = (Wh + 7) & ~7;
   const int pl = blockIdx.y;
   const long long plane = plane0 + pl;
-  const int r0 = blockIdx.x * (2 * FS_ROW_L);
+  const int r0 = blockIdx.x * (2 * L);
   for (int t = threadIdx.x; t < m; t += FS_ROW_T) tw[t] = __ldg(tw_g + t);
   const float2* Tp = T + (long long)pl * H * WhP;
   // X_full[k] = T[k] (k < Wh, imaginary parts of self-paired bins dropped), X_full[n-k] = conj T[k];
   // V = Xa + i Xb, stored swapped for the inverse transform.
-  for (int t = threadIdx.x; t < FS_ROW_L * Wh; t += FS_ROW_T) {
+  for (int t = threadIdx.x; t < L * Wh; t += FS_ROW_T) {
     const int p = t / Wh, k = t - p * Wh;
     const int ra = r0 + 2 * p;
     float2 ta = make_float2(0.f, 0.f), tb = make_float2(0.f, 0.f);
@@ -169,9 +173,9 @@ fs_rows_inv_kernel(Plan plan, const float2* __restrict__ T, float* __restrict__ 
     }
   }
   __syncthreads();
-  float2* res = plan.run(buf0, buf1, tw, FS_ROW_L, LS);   // res[p][c] = (y_b[c], y_a[c])
+  float2* res = plan.run(buf0, buf1, tw, L, LS);   // res[p][c] = (y_b[c], y_a[c])
   float* op = out + plane * (long long)H * W;
-  for (int p = 0; p < FS_ROW_L; ++p) {
+  for (int p = 0; p < L; ++p) {
     const int ra = r0 + 2 * p;
     if (ra >= H) break;
     const bool has_b = ra + 1 < H;
@@ -192,6 +196,18 @@ static int fs_line_len(int n) {
 static size_t fs_smem(int n, int m, int L) {
   return sizeof(float2) * ((size_t)m + (fs_static(n) ? 1 : 2) * (size_t)L * (m | 1));
 }
+// Lines per CTA of the rows kernels (FS_ROW_L, /2 or /4) and column pairs per CTA of the cols kernel (FS_COL_K, /2 or
+// /4): the most whose two line buffers fit in shared memory, 0 when none does.  The in-place static plans always fit.
+static int fs_row_lines(int W) {
+  if (fs_static(W)) return FS_ROW_L;
+  const int m = ud_any_line_len(W);
+  return ud_halving_lines(ud_any_lines(m, sizeof(float2) * (size_t)m, 0, UD_SMEM_CTA_MAX, FS_ROW_L), FS_ROW_L);
+}
+static int fs_col_k(int H) {
+  if (fs_static(H)) return FS_COL_K;
+  const int m = ud_any_line_len(H);
+  return ud_halving_lines(ud_any_lines(m, sizeof(float2) * (size_t)m, 0, UD_SMEM_CTA_MAX, FS_COL_L), FS_COL_L) / 2;
+}
 
 template <class K>
 static int fs_set_smem(K kernel, size_t bytes) {
@@ -207,21 +223,23 @@ static int fs_set_smem(K kernel, size_t bytes) {
   return UD_OK;
 }
 
-#define FS_PLAN1(n, L, THREADS, P, ...)                                                        \
-  do {                                                                                         \
-    if ((n) == 380) { UdStaticPlanIP<380, L, THREADS, 19, 5, 4> P; __VA_ARGS__; }              \
-    else if ((n) == 256) { UdStaticPlanIP<256, L, THREADS, 4, 4, 4, 4> P; __VA_ARGS__; }       \
-    else if ((n) == 224) { UdStaticPlanIP<224, L, THREADS, 7, 4, 4, 2> P; __VA_ARGS__; }       \
-    else if ((n) == 299) { UdStaticPlanIP<299, L, THREADS, 23, 13> P; __VA_ARGS__; }           \
-    else { UdAnyPlan P; if (!ud_make_any_plan((n), &P)) return UD_ERR_UNSUPPORTED; __VA_ARGS__; } \
+// Both run the body with the plan(s) of n and `constexpr int LV` lines per CTA: L for the static plans, Lany (one of L,
+// L/2, L/4) for the run-time plan.
+#define FS_PLAN1(n, L, Lany, THREADS, P, LV, ...)                                                                      \
+  do {                                                                                                                 \
+    if ((n) == 380) { UdStaticPlanIP<380, L, THREADS, 19, 5, 4> P; constexpr int LV = L; __VA_ARGS__; }                \
+    else if ((n) == 256) { UdStaticPlanIP<256, L, THREADS, 4, 4, 4, 4> P; constexpr int LV = L; __VA_ARGS__; }         \
+    else if ((n) == 224) { UdStaticPlanIP<224, L, THREADS, 7, 4, 4, 2> P; constexpr int LV = L; __VA_ARGS__; }         \
+    else if ((n) == 299) { UdStaticPlanIP<299, L, THREADS, 23, 13> P; constexpr int LV = L; __VA_ARGS__; }             \
+    else { UdAnyPlan P; if (!ud_make_any_plan((n), &P)) return UD_ERR_UNSUPPORTED; UD_LINES_DISPATCH(Lany, L, LV, __VA_ARGS__); } \
   } while (0)
-#define FS_PLAN2(n, P16, P8, ...)                                                                                          \
+#define FS_PLAN2(n, Kany, P16, P8, KV, ...)                                                                                \
   do {                                                                                                                     \
-    if ((n) == 380) { UdStaticPlanIP<380, FS_COL_L, FS_COL_T, 19, 5, 4> P16; UdStaticPlanIP<380, FS_COL_K, FS_COL_T, 19, 5, 4> P8; __VA_ARGS__; } \
-    else if ((n) == 256) { UdStaticPlanIP<256, FS_COL_L, FS_COL_T, 4, 4, 4, 4> P16; UdStaticPlanIP<256, FS_COL_K, FS_COL_T, 4, 4, 4, 4> P8; __VA_ARGS__; } \
-    else if ((n) == 224) { UdStaticPlanIP<224, FS_COL_L, FS_COL_T, 7, 4, 4, 2> P16; UdStaticPlanIP<224, FS_COL_K, FS_COL_T, 7, 4, 4, 2> P8; __VA_ARGS__; } \
-    else if ((n) == 299) { UdStaticPlanIP<299, FS_COL_L, FS_COL_T, 23, 13> P16; UdStaticPlanIP<299, FS_COL_K, FS_COL_T, 23, 13> P8; __VA_ARGS__; } \
-    else { UdAnyPlan P16; if (!ud_make_any_plan((n), &P16)) return UD_ERR_UNSUPPORTED; UdAnyPlan P8 = P16; __VA_ARGS__; }  \
+    if ((n) == 380) { UdStaticPlanIP<380, FS_COL_L, FS_COL_T, 19, 5, 4> P16; UdStaticPlanIP<380, FS_COL_K, FS_COL_T, 19, 5, 4> P8; constexpr int KV = FS_COL_K; __VA_ARGS__; } \
+    else if ((n) == 256) { UdStaticPlanIP<256, FS_COL_L, FS_COL_T, 4, 4, 4, 4> P16; UdStaticPlanIP<256, FS_COL_K, FS_COL_T, 4, 4, 4, 4> P8; constexpr int KV = FS_COL_K; __VA_ARGS__; } \
+    else if ((n) == 224) { UdStaticPlanIP<224, FS_COL_L, FS_COL_T, 7, 4, 4, 2> P16; UdStaticPlanIP<224, FS_COL_K, FS_COL_T, 7, 4, 4, 2> P8; constexpr int KV = FS_COL_K; __VA_ARGS__; } \
+    else if ((n) == 299) { UdStaticPlanIP<299, FS_COL_L, FS_COL_T, 23, 13> P16; UdStaticPlanIP<299, FS_COL_K, FS_COL_T, 23, 13> P8; constexpr int KV = FS_COL_K; __VA_ARGS__; } \
+    else { UdAnyPlan P16; if (!ud_make_any_plan((n), &P16)) return UD_ERR_UNSUPPORTED; UdAnyPlan P8 = P16; UD_LINES_DISPATCH(Kany, FS_COL_K, KV, __VA_ARGS__); }  \
   } while (0)
 
 static int fs_chunk(int N, int C, int H, int W) {
@@ -242,6 +260,9 @@ extern "C" int ud_freq_style_transfer(const float* content, const float* style, 
   UD_REQUIRE(N >= 0 && C >= 1 && H >= 1 && W >= 1, UD_ERR_INVALID, "freq_style: bad shape N=%d C=%d H=%d W=%d", N, C, H, W);
   UD_REQUIRE(H <= UD_FFT_MAX_N && W <= UD_FFT_MAX_N, UD_ERR_UNSUPPORTED, "freq_style: FFT size %dx%d unsupported (n <= %d)",
              H, W, UD_FFT_MAX_N);
+  const int LR = fs_row_lines(W), KC = fs_col_k(H);
+  UD_REQUIRE(LR > 0, UD_ERR_UNSUPPORTED, "freq_style: %d-point rows do not fit shared memory", W);
+  UD_REQUIRE(KC > 0, UD_ERR_UNSUPPORTED, "freq_style: %d-point columns do not fit shared memory", H);
   if (N == 0) return UD_OK;
   UD_REQUIRE(content && style && lmda && out && ws, UD_ERR_INVALID, "freq_style: null pointer");
   UD_REQUIRE(ws_bytes >= ud_freq_style_workspace_bytes(N, C, H, W), UD_ERR_WORKSPACE, "freq_style: workspace too small");
@@ -254,28 +275,28 @@ extern "C" int ud_freq_style_transfer(const float* content, const float* style, 
   const float2* twW = ud_twiddles(mW);
   const float2* twH = ud_twiddles(mH);
   if (!twW || !twH) return UD_ERR_CUDA;
-  const size_t smR = fs_smem(W, mW, FS_ROW_L), smC = fs_smem(H, mH, FS_COL_L);
+  const size_t smR = fs_smem(W, mW, LR), smC = fs_smem(H, mH, 2 * KC);
   const float scale = 1.f / ((float)H * (float)W);
   int rc;
   for (int s0 = 0; s0 < N; s0 += chunk) {
     const int ns = (N - s0 < chunk) ? (N - s0) : chunk;
     const int planes = ns * C, plane0 = s0 * C;
-    FS_PLAN1(W, FS_ROW_L, FS_ROW_T, plan, {
-      auto k = fs_rows_fwd_kernel<decltype(plan)>;
+    FS_PLAN1(W, FS_ROW_L, LR, FS_ROW_T, plan, LV, {
+      auto k = fs_rows_fwd_kernel<decltype(plan), LV>;
       if ((rc = fs_set_smem(k, smR)) != UD_OK) return rc;
-      k<<<dim3(ud_cdiv(H, FS_ROW_L), planes), FS_ROW_T, smR, stream>>>(plan, content, style, Ya, Yb, twW, plane0, H, W);
+      k<<<dim3(ud_cdiv(H, LV), planes), FS_ROW_T, smR, stream>>>(plan, content, style, Ya, Yb, twW, plane0, H, W);
     });
     if ((rc = ud_check_launch("fs_rows_fwd")) != UD_OK) return rc;
-    FS_PLAN2(H, p16, p8, {
-      auto k = fs_cols_kernel<decltype(p16), decltype(p8)>;
+    FS_PLAN2(H, KC, p16, p8, KV, {
+      auto k = fs_cols_kernel<decltype(p16), decltype(p8), KV>;
       if ((rc = fs_set_smem(k, smC)) != UD_OK) return rc;
-      k<<<dim3(ud_cdiv(Wh, FS_COL_K), planes), FS_COL_T, smC, stream>>>(p16, p8, Ya, Yb, lmda, twH, plane0, C, H, W);
+      k<<<dim3(ud_cdiv(Wh, KV), planes), FS_COL_T, smC, stream>>>(p16, p8, Ya, Yb, lmda, twH, plane0, C, H, W);
     });
     if ((rc = ud_check_launch("fs_cols")) != UD_OK) return rc;
-    FS_PLAN1(W, FS_ROW_L, FS_ROW_T, plan, {
-      auto k = fs_rows_inv_kernel<decltype(plan)>;
+    FS_PLAN1(W, FS_ROW_L, LR, FS_ROW_T, plan, LV, {
+      auto k = fs_rows_inv_kernel<decltype(plan), LV>;
       if ((rc = fs_set_smem(k, smR)) != UD_OK) return rc;
-      k<<<dim3(ud_cdiv(H, 2 * FS_ROW_L), planes), FS_ROW_T, smR, stream>>>(plan, Ya, out, twW, plane0, H, W, scale);
+      k<<<dim3(ud_cdiv(H, 2 * LV), planes), FS_ROW_T, smR, stream>>>(plan, Ya, out, twW, plane0, H, W, scale);
     });
     if ((rc = ud_check_launch("fs_rows_inv")) != UD_OK) return rc;
   }

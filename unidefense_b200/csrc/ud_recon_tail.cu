@@ -40,8 +40,10 @@ int ud_rt2_bwd(const float* dec, const float* x, const uint8_t* signs, const flo
 #define RT_ROW_L 12    // row PAIRS (complex lines) per CTA of the rows kernels  -> 24 image rows
 #define RT_COL_T 320   // threads of the cols kernels
 #define RT_COL_L 16    // columns per CTA of the cols kernels (16 float2 = one 128-byte line per row)
+// Lines longer than shared memory holds at those counts (long Bluestein lines, m = 1024 or 2048) run instantiations
+// with a half or a quarter of them: rt_row_lines / rt_col_lines pick the largest that fits.
 #define RT_HSTAGE 12   // rows_bwd: max horizontal-transpose items per thread kept in registers
-#define RT_VGRP 3      // row pairs whose vertical lerps are staged per barrier (RT_ROW_L % RT_VGRP == 0)
+#define RT_VGRP 3      // row pairs whose vertical lerps are staged per barrier (every row-pair count % RT_VGRP == 0)
 
 static inline int rt_whp(int W) { return ((W / 2 + 1) + 15) & ~15; }  // padded half width (float2)
 
@@ -75,12 +77,13 @@ __device__ __forceinline__ void rt_vrows(const float* __restrict__ decp, const f
 // forward rows: grid (row_tiles, planes_in_chunk)
 //   shared: tw[n] | xtab[n] | buf0[L*LS] (| buf1[L*LS] when the plan ping-pongs) | vbuf[2][2][w]
 // ------------------------------------------------------------------------------------------
-template <class Plan>
+template <class Plan, int L>
 __global__ void __launch_bounds__(RT_ROW_T)
 rt_rows_fwd_kernel(Plan plan, const float* __restrict__ dec, const float* __restrict__ x,
                    float* __restrict__ rec, float2* __restrict__ Y, float* __restrict__ part_spatial,
                    const float2* __restrict__ tw_g, const float2* __restrict__ ytab_g,
                    const float2* __restrict__ xtab_g, int plane0, int h, int w, int H, int W, int row_tiles) {
+  static_assert(L % RT_VGRP == 0, "row pairs are staged in groups of RT_VGRP");
   extern __shared__ float2 smem[];
   const int n = plan.n();  // == W
   const int m = plan.line_len();     // == n except for Bluestein plans
@@ -88,14 +91,14 @@ rt_rows_fwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
   float2* tw = smem;
   float2* xtab = tw + m;
   float2* buf0 = xtab + n;
-  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + RT_ROW_L * LS;
-  float* vbuf = reinterpret_cast<float*>(buf1 + RT_ROW_L * LS);
+  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + L * LS;
+  float* vbuf = reinterpret_cast<float*>(buf1 + L * LS);
   __shared__ float red[33];
 
   const int tile = blockIdx.x;
   const int pl = blockIdx.y;             // plane within chunk
   const long long plane = plane0 + pl;   // global (n*C + c)
-  const int r0 = tile * (2 * RT_ROW_L);
+  const int r0 = tile * (2 * L);
   W = n;                                 // W == n: lets static plans constant-fold every index below
   const int Wh = n / 2 + 1;
   const int WhP = (Wh + 15) & ~15;
@@ -107,7 +110,7 @@ rt_rows_fwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
   float* recp = rec + plane * (long long)H * W;
 
   // whole x tile in flight first: x[ra][c] -> line[p][c].x, x[ra+1][c] -> .y (overwritten in place by d below)
-  for (int p = 0; p < RT_ROW_L; ++p) {
+  for (int p = 0; p < L; ++p) {
     const int ra = r0 + 2 * p;
     if (ra >= H) break;
     const float* xa_p = xp + (long long)ra * W;
@@ -123,8 +126,8 @@ rt_rows_fwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
   ud_cp_async_wait_all();
   __syncthreads();
   float acc = 0.f;
-  for (int g = 0; g < RT_ROW_L / RT_VGRP; ++g) {
-    if (g + 1 < RT_ROW_L / RT_VGRP) {
+  for (int g = 0; g < L / RT_VGRP; ++g) {
+    if (g + 1 < L / RT_VGRP) {
       float* nv = vbuf + ((g + 1) & 1) * (2 * RT_VGRP) * w;
       for (int q = 0; q < RT_VGRP; ++q)
         rt_vrows(decp, ytab_g, r0 + 2 * ((g + 1) * RT_VGRP + q), h, w, H, nv + 2 * q * w, nv + (2 * q + 1) * w);
@@ -163,11 +166,11 @@ rt_rows_fwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
     }
     __syncthreads();
   }
-  float2* res = plan.run(buf0, buf1, tw, RT_ROW_L, LS);
+  float2* res = plan.run(buf0, buf1, tw, L, LS);
 
   // unpack the two real rows of each pair: A[k] = (Z[k]+conj Z[n-k])/2, B[k] = (Z[k]-conj Z[n-k])/(2i)
   float2* Yp = Y + (long long)pl * H * WhP;
-  for (int t = threadIdx.x; t < RT_ROW_L * Wh; t += RT_ROW_T) {
+  for (int t = threadIdx.x; t < L * Wh; t += RT_ROW_T) {
     const int p = t / Wh, k = t - p * Wh;
     const int ra = r0 + 2 * p;
     if (ra >= H) continue;
@@ -183,7 +186,7 @@ rt_rows_fwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
 // ------------------------------------------------------------------------------------------
 // forward cols: grid (col_tiles, planes_in_chunk).  Column FFT length n = H.
 // ------------------------------------------------------------------------------------------
-template <class Plan>
+template <class Plan, int L>
 __global__ void __launch_bounds__(RT_COL_T)
 rt_cols_fwd_kernel(Plan plan, const float2* __restrict__ Y, float* __restrict__ part_freq,
                    uint8_t* __restrict__ signs, const float2* __restrict__ tw_g, int plane0, int H, int W,
@@ -194,7 +197,7 @@ rt_cols_fwd_kernel(Plan plan, const float2* __restrict__ Y, float* __restrict__ 
   const int LS = m | 1;
   float2* tw = smem;
   float2* buf0 = tw + m;
-  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + RT_COL_L * LS;
+  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + L * LS;
   __shared__ float red[33];
 
   const int tile = blockIdx.x;
@@ -203,20 +206,20 @@ rt_cols_fwd_kernel(Plan plan, const float2* __restrict__ Y, float* __restrict__ 
   H = n;                                 // H == n: constant-folds the index math for static plans
   const int Wh = W / 2 + 1;
   const int WhP = (Wh + 15) & ~15;
-  const int k0 = tile * RT_COL_L;
-  const int ncols = min(RT_COL_L, Wh - k0);
+  const int k0 = tile * L;
+  const int ncols = min(L, Wh - k0);
 
   for (int t = threadIdx.x; t < m; t += RT_COL_T) tw[t] = __ldg(tw_g + t);
   const float2* Yp = Y + (long long)pl * H * WhP;
-  for (int t = threadIdx.x; t < H * RT_COL_L; t += RT_COL_T) {
-    const int r = t / RT_COL_L, cc = t - r * RT_COL_L;
+  for (int t = threadIdx.x; t < H * L; t += RT_COL_T) {
+    const int r = t / L, cc = t - r * L;
     if (cc < ncols) ud_cp_async8(&buf0[cc * LS + r], Yp + (long long)r * WhP + k0 + cc);
     else buf0[cc * LS + r] = make_float2(0.f, 0.f);
   }
   ud_cp_async_commit();
   ud_cp_async_wait_all();
   __syncthreads();
-  float2* res = plan.run(buf0, buf1, tw, RT_COL_L, LS);
+  float2* res = plan.run(buf0, buf1, tw, L, LS);
 
   float acc = 0.f;
   for (int t = threadIdx.x; t < ncols * H; t += RT_COL_T) {
@@ -256,7 +259,7 @@ __global__ void rt_finalize_kernel(const float* __restrict__ part_spatial, const
 // T[r,k] = sum_j S[j,k] e^{+2 pi i j r / H},  S = gf * (sgn Re D + i sgn Im D)
 // inverse via the swap trick: IFFT(z) = swap(FFT(swap(z))).
 // ------------------------------------------------------------------------------------------
-template <class Plan>
+template <class Plan, int L>
 __global__ void __launch_bounds__(RT_COL_T)
 rt_cols_bwd_kernel(Plan plan, const uint8_t* __restrict__ signs, const float* __restrict__ g_freq,
                    float2* __restrict__ T, const float2* __restrict__ tw_g, int plane0, int C, int H, int W,
@@ -267,7 +270,7 @@ rt_cols_bwd_kernel(Plan plan, const uint8_t* __restrict__ signs, const float* __
   const int LS = m | 1;
   float2* tw = smem;
   float2* buf0 = tw + m;
-  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + RT_COL_L * LS;
+  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + L * LS;
 
   const int tile = blockIdx.x;
   const int pl = blockIdx.y;
@@ -278,11 +281,11 @@ rt_cols_bwd_kernel(Plan plan, const uint8_t* __restrict__ signs, const float* __
   H = n;
   const int Wh = W / 2 + 1;
   const int WhP = (Wh + 15) & ~15;
-  const int k0 = tile * RT_COL_L;
-  const int ncols = min(RT_COL_L, Wh - k0);
+  const int k0 = tile * L;
+  const int ncols = min(L, Wh - k0);
 
   for (int t = threadIdx.x; t < m; t += RT_COL_T) tw[t] = __ldg(tw_g + t);
-  for (int t = threadIdx.x; t < RT_COL_L * H; t += RT_COL_T) {
+  for (int t = threadIdx.x; t < L * H; t += RT_COL_T) {
     const int cc = t / H, j = t - cc * H;
     float2 v = make_float2(0.f, 0.f);
     if (cc < ncols) {
@@ -294,10 +297,10 @@ rt_cols_bwd_kernel(Plan plan, const uint8_t* __restrict__ signs, const float* __
     buf0[cc * LS + j] = v;
   }
   __syncthreads();
-  float2* res = plan.run(buf0, buf1, tw, RT_COL_L, LS);
+  float2* res = plan.run(buf0, buf1, tw, L, LS);
   float2* Tp = T + (long long)pl * H * WhP;
-  for (int t = threadIdx.x; t < H * RT_COL_L; t += RT_COL_T) {
-    const int r = t / RT_COL_L, cc = t - r * RT_COL_L;
+  for (int t = threadIdx.x; t < H * L; t += RT_COL_T) {
+    const int r = t / L, cc = t - r * L;
     if (cc < ncols) {
       const float2 v = res[cc * LS + r];
       Tp[(long long)r * WhP + k0 + cc] = make_float2(v.y, v.x);  // swap back
@@ -318,7 +321,7 @@ rt_cols_bwd_kernel(Plan plan, const uint8_t* __restrict__ signs, const float* __
 // GX: also g_x = -g_rec at full resolution from the finished lines (zeros for planes whose sample has gs == gf == 0);
 // g_dec may then be NULL.  GX = false is the training path.
 // ------------------------------------------------------------------------------------------
-template <class Plan, bool GX>
+template <class Plan, bool GX, int L>
 __global__ void __launch_bounds__(RT_ROW_T)
 rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __restrict__ x,
                    const float2* __restrict__ T, const float* __restrict__ g_spatial,
@@ -326,6 +329,7 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
                    const float2* __restrict__ tw_g, const float2* __restrict__ ytab_g,
                    const float2* __restrict__ xtab_g, const int2* __restrict__ jtab_g, int plane0, int C, int h,
                    int w, int H, int W, float sp_scale) {
+  static_assert(L % RT_VGRP == 0, "row pairs are staged in groups of RT_VGRP");
   extern __shared__ float2 smem[];
   const int n = plan.n();  // == W
   const int m = plan.line_len();     // == n except for Bluestein plans
@@ -333,8 +337,8 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
   float2* tw = smem;
   float2* xtab = tw + m;
   float2* buf0 = xtab + n;
-  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + RT_ROW_L * LS;
-  float* vbuf = reinterpret_cast<float*>(buf1 + RT_ROW_L * LS);
+  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + L * LS;
+  float* vbuf = reinterpret_cast<float*>(buf1 + L * LS);
 
   const int tile = blockIdx.x;
   const int pl = blockIdx.y;
@@ -342,11 +346,11 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
   const int smp = (int)(plane / C);
   const float gs = g_spatial[smp] * sp_scale;
   const bool has_f = g_freq[smp] != 0.f;
-  const int r0 = tile * (2 * RT_ROW_L);
+  const int r0 = tile * (2 * L);
   if (gs == 0.f && !has_f) {
     if (GX) {                            // the tile's rows of g_x are zero
       float* gxp = g_x + plane * (long long)H * n;
-      const long long e = (long long)min(H, r0 + 2 * RT_ROW_L) * n;
+      const long long e = (long long)min(H, r0 + 2 * L) * n;
       for (long long i = (long long)r0 * n + threadIdx.x; i < e; i += RT_ROW_T) gxp[i] = 0.f;
     }
     return;
@@ -354,17 +358,17 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
   W = n;
   const int Wh = n / 2 + 1;
   const int WhP = (Wh + 15) & ~15;
-  const int nrows = min(2 * RT_ROW_L, H - r0);
+  const int nrows = min(2 * L, H - r0);
 
   for (int t = threadIdx.x; t < m; t += RT_ROW_T) tw[t] = __ldg(tw_g + t);
   for (int t = threadIdx.x; t < n; t += RT_ROW_T) xtab[t] = __ldg(xtab_g + t);
   // sign(rec - x) of the tile first (2+2 bits per row pair and column), while the buffer is still free:
   // x is prefetched into the lines with cp.async exactly like the forward does.
-  uint8_t* sgn = reinterpret_cast<uint8_t*>(vbuf + 4 * RT_VGRP * w);   // [RT_ROW_L][n]
+  uint8_t* sgn = reinterpret_cast<uint8_t*>(vbuf + 4 * RT_VGRP * w);   // [L][n]
   if (gs != 0.f) {
     const float* decp = dec + plane * (long long)h * w;
     const float* xp = x + plane * (long long)H * W;
-    for (int p = 0; p < RT_ROW_L; ++p) {
+    for (int p = 0; p < L; ++p) {
       const int ra = r0 + 2 * p;
       if (ra >= H) break;
       const float* xa_p = xp + (long long)ra * W;
@@ -379,8 +383,8 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
     for (int q = 0; q < RT_VGRP; ++q) rt_vrows(decp, ytab_g, r0 + 2 * q, h, w, H, vbuf + 2 * q * w, vbuf + (2 * q + 1) * w);
     ud_cp_async_wait_all();
     __syncthreads();
-    for (int g = 0; g < RT_ROW_L / RT_VGRP; ++g) {
-      if (g + 1 < RT_ROW_L / RT_VGRP) {
+    for (int g = 0; g < L / RT_VGRP; ++g) {
+      if (g + 1 < L / RT_VGRP) {
         float* nv = vbuf + ((g + 1) & 1) * (2 * RT_VGRP) * w;
         for (int q = 0; q < RT_VGRP; ++q)
           rt_vrows(decp, ytab_g, r0 + 2 * ((g + 1) * RT_VGRP + q), h, w, H, nv + 2 * q * w, nv + (2 * q + 1) * w);
@@ -419,7 +423,7 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
   if (has_f) {
     const float2* Tp = T + (long long)pl * H * WhP;
     // build V = Th_a + i Th_b (swapped for the inverse) for k in [0, Wh) and its mirror n-k
-    for (int t = threadIdx.x; t < RT_ROW_L * Wh; t += RT_ROW_T) {
+    for (int t = threadIdx.x; t < L * Wh; t += RT_ROW_T) {
       const int p = t / Wh, k = t - p * Wh;
       const int ra = r0 + 2 * p;
       float2 ta = make_float2(0.f, 0.f), tb = make_float2(0.f, 0.f);
@@ -438,13 +442,13 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
       }
     }
     __syncthreads();
-    res = plan.run(buf0, buf1, tw, RT_ROW_L, LS);   // res[p][c] = (g_b[c], g_a[c])
+    res = plan.run(buf0, buf1, tw, L, LS);   // res[p][c] = (g_b[c], g_a[c])
   } else {
-    for (int t = threadIdx.x; t < RT_ROW_L * LS; t += RT_ROW_T) buf0[t] = make_float2(0.f, 0.f);
+    for (int t = threadIdx.x; t < L * LS; t += RT_ROW_T) buf0[t] = make_float2(0.f, 0.f);
     __syncthreads();
   }
   if (gs != 0.f) {  // g += gs * sign(rec - x)
-    for (int t = threadIdx.x; t < RT_ROW_L * n; t += RT_ROW_T) {
+    for (int t = threadIdx.x; t < L * n; t += RT_ROW_T) {
       const int p = t / n, c = t - p * n;
       const uint8_t code = sgn[t];
       float2 g = res[p * LS + c];
@@ -465,7 +469,7 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
     if (g_dec == nullptr) return;        // g_x only: no transposed resize
   }
   float* gd = g_dec + plane * (long long)h * w;
-  const int items = RT_ROW_L * w;
+  const int items = L * w;
   if (items <= RT_HSTAGE * RT_ROW_T && w <= n) {   // staged results are written back over the line (n slots)
     // horizontal transposed lerp, both rows of a pair per item, staged in registers.  jtab[j] = first/last
     // output column whose two taps include dec column j (exact, from the same fp32 table as the forward).
@@ -475,7 +479,7 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
 #pragma unroll
     for (int s = 0; s < RT_HSTAGE; ++s) {
       hv[s] = make_float2(0.f, 0.f);
-      if (p < RT_ROW_L) {
+      if (p < L) {
         const int2 cr = __ldg(jtab_g + j);
         const float2* line = res + p * LS;
         float ax = 0.f, ay = 0.f;
@@ -498,7 +502,7 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
     while (j >= w) { j -= w; ++p; }
 #pragma unroll
     for (int s = 0; s < RT_HSTAGE; ++s) {
-      if (p < RT_ROW_L) res[p * LS + j] = hv[s];
+      if (p < L) res[p * LS + j] = hv[s];
       j += RT_ROW_T;
       while (j >= w) { j -= w; ++p; }
     }
@@ -556,13 +560,31 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
 // host side
 // ------------------------------------------------------------------------------------------
 // m: points per line buffer / staged twiddles (UdAnyPlan::m: n, or the Bluestein length for sizes with a prime factor
-// > 23).  The plans are not in place, so the kernels keep two line buffers.
-static size_t rt_rows_smem(int n, int m, int w) {
-  return sizeof(float2) * ((size_t)m + n + 2ull * RT_ROW_L * (size_t)(m | 1)) + sizeof(float) * 4ull * RT_VGRP * w +
-         (size_t)RT_ROW_L * n;   // + sign bytes of the tile (rows_bwd)
+// > 23).  The plans are not in place, so the kernels keep two line buffers of L lines each.
+static size_t rt_rows_fixed_smem(int n, int m, int w) {   // tw[m] | xtab[n] | vbuf
+  return sizeof(float2) * ((size_t)m + n) + sizeof(float) * 4ull * RT_VGRP * w;
 }
-static size_t rt_cols_smem(int m) {
-  return sizeof(float2) * ((size_t)m + 2ull * RT_COL_L * (size_t)(m | 1));
+static size_t rt_rows_smem(int n, int m, int w, int L) {
+  return rt_rows_fixed_smem(n, m, w) + sizeof(float2) * 2ull * L * (size_t)(m | 1) +
+         (size_t)L * n;   // + sign bytes of the tile (rows_bwd)
+}
+static size_t rt_cols_smem(int m, int L) {
+  return sizeof(float2) * ((size_t)m + 2ull * L * (size_t)(m | 1));
+}
+// Static shared memory of rt_rows_fwd_kernel / rt_cols_fwd_kernel: red[33] as ptxas lays it out.  The per-CTA limit
+// holds static and dynamic bytes together, so the line counts below leave room for it.
+#define RT_STATIC_SMEM 144
+// Row pairs per CTA of the rows kernels (RT_ROW_L, /2 or /4) and columns per CTA of the cols kernels (RT_COL_L, /2 or
+// /4): the most that fit in shared memory, 0 when none does.
+static int rt_row_lines(int W, int w) {
+  const int m = ud_any_line_len(W);
+  return ud_halving_lines(ud_any_lines(m, rt_rows_fixed_smem(W, m, w) + RT_STATIC_SMEM, W, UD_SMEM_CTA_MAX, RT_ROW_L),
+                          RT_ROW_L);
+}
+static int rt_col_lines(int H) {
+  const int m = ud_any_line_len(H);
+  return ud_halving_lines(ud_any_lines(m, sizeof(float2) * (size_t)m + RT_STATIC_SMEM, 0, UD_SMEM_CTA_MAX, RT_COL_L),
+                          RT_COL_L);
 }
 
 static size_t rt_plane_bytes(int H, int W) {
@@ -580,9 +602,11 @@ static int rt_chunk_samples(int N, int C, int H, int W) {
 }
 
 extern "C" size_t ud_recon_tail_workspace_bytes(int N, int C, int h, int w, int H, int W) {
-  (void)h; (void)w;
+  (void)h;
   const int chunk = rt_chunk_samples(N, C, H, W);
-  const int row_tiles = ud_cdiv(H, 2 * RT_ROW_L), col_tiles = ud_cdiv(W / 2 + 1, RT_COL_L);
+  // the first-generation tiles outnumber the second generation's; a size no count fits is rejected by the entry points
+  const int LR = rt_row_lines(W, w), LC = rt_col_lines(H);
+  const int row_tiles = ud_cdiv(H, 2 * (LR > 0 ? LR : 1)), col_tiles = ud_cdiv(W / 2 + 1, LC > 0 ? LC : 1);
   size_t y = ud_align_up((size_t)chunk * C * rt_plane_bytes(H, W), 256);
   size_t ps = ud_align_up((size_t)N * C * row_tiles * sizeof(float), 256);
   size_t pf = ud_align_up((size_t)N * C * col_tiles * sizeof(float), 256);
@@ -613,6 +637,9 @@ static int rt_validate(int N, int C, int h, int w, int H, int W) {
   UD_REQUIRE(H <= UD_FFT_MAX_N && W <= UD_FFT_MAX_N, UD_ERR_UNSUPPORTED,
              "recon_tail: FFT size %dx%d unsupported (n <= %d)", H, W, UD_FFT_MAX_N);
   UD_REQUIRE((long long)N * C <= 65535LL * 64, UD_ERR_UNSUPPORTED, "recon_tail: too many planes");
+  UD_REQUIRE(rt_row_lines(W, w) > 0, UD_ERR_UNSUPPORTED,
+             "recon_tail: %d-point rows with a %d-wide decoder do not fit shared memory", W, w);
+  UD_REQUIRE(rt_col_lines(H) > 0, UD_ERR_UNSUPPORTED, "recon_tail: %d-point columns do not fit shared memory", H);
   return UD_OK;
 }
 
@@ -630,8 +657,9 @@ extern "C" int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, f
   if (chunk * C > 65535) chunk = 65535 / C;
   const int Wh = W / 2 + 1;
   const bool v2 = ud_rt2_supported(h, w, H, W);
-  const int row_tiles = v2 ? ud_cdiv((H + 1) / 2, ud_rt2_rows_lpc()) : ud_cdiv(H, 2 * RT_ROW_L);
-  const int col_tiles = v2 ? ud_cdiv(Wh, RT2_COLS_PER_TILE) : ud_cdiv(Wh, RT_COL_L);
+  const int LR = rt_row_lines(W, w), LC = rt_col_lines(H);
+  const int row_tiles = v2 ? ud_cdiv((H + 1) / 2, ud_rt2_rows_lpc()) : ud_cdiv(H, 2 * LR);
+  const int col_tiles = v2 ? ud_cdiv(Wh, RT2_COLS_PER_TILE) : ud_cdiv(Wh, LC);
   char* p = static_cast<char*>(ws);
   float2* Y = reinterpret_cast<float2*>(p);
   p += ud_align_up((size_t)rt_chunk_samples(N, C, H, W) * C * rt_plane_bytes(H, W), 256);
@@ -643,7 +671,7 @@ extern "C" int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, f
   const float2* ytab = ud_lerp_table(h, H);
   const float2* xtab = ud_lerp_table(w, W);
   if (!ytab || !xtab) return UD_ERR_CUDA;
-  const size_t smW = rt_rows_smem(W, pW.m, w), smH = rt_cols_smem(pH.m);
+  const size_t smW = rt_rows_smem(W, pW.m, w, LR), smH = rt_cols_smem(pH.m, LC);
 
   for (int s0 = 0; s0 < N; s0 += chunk) {
     const int ns = (N - s0 < chunk) ? (N - s0) : chunk;
@@ -653,13 +681,18 @@ extern "C" int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, f
                            stream)) != UD_OK) return rc;
       continue;
     }
-    if ((rc = rt_set_smem(rt_rows_fwd_kernel<UdAnyPlan>, smW)) != UD_OK) return rc;
-    rt_rows_fwd_kernel<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(pW, dec, x, rec, Y, part_sp, pW.tw, ytab, xtab,
-                                                                           plane0, h, w, H, W, row_tiles);
+    UD_LINES_DISPATCH(LR, RT_ROW_L, LV, {
+      auto k = rt_rows_fwd_kernel<UdAnyPlan, LV>;
+      if ((rc = rt_set_smem(k, smW)) != UD_OK) return rc;
+      k<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(pW, dec, x, rec, Y, part_sp, pW.tw, ytab, xtab, plane0, h, w,
+                                                            H, W, row_tiles);
+    });
     if ((rc = ud_check_launch("rt_rows_fwd")) != UD_OK) return rc;
-    if ((rc = rt_set_smem(rt_cols_fwd_kernel<UdAnyPlan>, smH)) != UD_OK) return rc;
-    rt_cols_fwd_kernel<<<dim3(col_tiles, planes), RT_COL_T, smH, stream>>>(pH, Y, part_fr, signs, pH.tw, plane0, H, W,
-                                                                           col_tiles);
+    UD_LINES_DISPATCH(LC, RT_COL_L, LV, {
+      auto k = rt_cols_fwd_kernel<UdAnyPlan, LV>;
+      if ((rc = rt_set_smem(k, smH)) != UD_OK) return rc;
+      k<<<dim3(col_tiles, planes), RT_COL_T, smH, stream>>>(pH, Y, part_fr, signs, pH.tw, plane0, H, W, col_tiles);
+    });
     if ((rc = ud_check_launch("rt_cols_fwd")) != UD_OK) return rc;
   }
   const float nrm = norm_ortho ? 1.f / sqrtf((float)H * (float)W) : 1.f;
@@ -683,8 +716,9 @@ extern "C" int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t
   if (chunk * C > 65535) chunk = 65535 / C;
   const int Wh = W / 2 + 1;
   const bool v2 = ud_rt2_supported(h, w, H, W);
-  const int row_tiles = v2 ? ud_cdiv((H + 1) / 2, ud_rt2_rows_lpc()) : ud_cdiv(H, 2 * RT_ROW_L);
-  const int col_tiles = v2 ? ud_cdiv(Wh, RT2_COLS_PER_TILE) : ud_cdiv(Wh, RT_COL_L);
+  const int LR = rt_row_lines(W, w), LC = rt_col_lines(H);
+  const int row_tiles = v2 ? ud_cdiv((H + 1) / 2, ud_rt2_rows_lpc()) : ud_cdiv(H, 2 * LR);
+  const int col_tiles = v2 ? ud_cdiv(Wh, RT2_COLS_PER_TILE) : ud_cdiv(Wh, LC);
   float2* T = reinterpret_cast<float2*>(ws);
   UdAnyPlan pW, pH;   // line FFTs of the first-generation kernels: mixed radix, or Bluestein for a prime factor > 23
   if (!ud_make_any_plan(W, &pW) || !ud_make_any_plan(H, &pH)) return UD_ERR_UNSUPPORTED;
@@ -693,7 +727,7 @@ extern "C" int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t
   if (!ytab || !xtab) return UD_ERR_CUDA;
   const int2* jtab = ud_lerp_ranges(w, W);
   if (!jtab) return UD_ERR_CUDA;
-  const size_t smH = rt_cols_smem(pH.m), smW = rt_rows_smem(W, pW.m, w);
+  const size_t smH = rt_cols_smem(pH.m, LC), smW = rt_rows_smem(W, pW.m, w, LR);
   // freq[n] = nrm/(C*H*Wh) * sum |D'| with D' the unnormalised spectrum, so the sign spectrum
   // carries nrm/(C*H*Wh) and the adjoint of the unnormalised forward is the unnormalised inverse.
   const float nrm = norm_ortho ? 1.f / sqrtf((float)H * (float)W) : 1.f;
@@ -708,14 +742,18 @@ extern "C" int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t
                            gscale, sp_scale, stream)) != UD_OK) return rc;
       continue;
     }
-    if ((rc = rt_set_smem(rt_cols_bwd_kernel<UdAnyPlan>, smH)) != UD_OK) return rc;
-    rt_cols_bwd_kernel<<<dim3(col_tiles, planes), RT_COL_T, smH, stream>>>(pH, signs, g_freq, T, pH.tw, plane0, C, H, W,
-                                                                           gscale);
+    UD_LINES_DISPATCH(LC, RT_COL_L, LV, {
+      auto k = rt_cols_bwd_kernel<UdAnyPlan, LV>;
+      if ((rc = rt_set_smem(k, smH)) != UD_OK) return rc;
+      k<<<dim3(col_tiles, planes), RT_COL_T, smH, stream>>>(pH, signs, g_freq, T, pH.tw, plane0, C, H, W, gscale);
+    });
     if ((rc = ud_check_launch("rt_cols_bwd")) != UD_OK) return rc;
-    auto k = g_x ? rt_rows_bwd_kernel<UdAnyPlan, true> : rt_rows_bwd_kernel<UdAnyPlan, false>;
-    if ((rc = rt_set_smem(k, smW)) != UD_OK) return rc;
-    k<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(pW, dec, x, T, g_spatial, g_freq, g_dec, g_x, pW.tw, ytab, xtab,
-                                                           jtab, plane0, C, h, w, H, W, sp_scale);
+    UD_LINES_DISPATCH(LR, RT_ROW_L, LV, {
+      auto k = g_x ? rt_rows_bwd_kernel<UdAnyPlan, true, LV> : rt_rows_bwd_kernel<UdAnyPlan, false, LV>;
+      if ((rc = rt_set_smem(k, smW)) != UD_OK) return rc;
+      k<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(pW, dec, x, T, g_spatial, g_freq, g_dec, g_x, pW.tw, ytab,
+                                                             xtab, jtab, plane0, C, h, w, H, W, sp_scale);
+    });
     if ((rc = ud_check_launch("rt_rows_bwd")) != UD_OK) return rc;
   }
   return UD_OK;
