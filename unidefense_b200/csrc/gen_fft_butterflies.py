@@ -52,7 +52,7 @@ def gen(p: int) -> str:
     return "\n".join(o)
 
 
-# Composite radices used by the register-resident two-stage line FFTs (ud_fft2s.cuh): R = Ra * Rb evaluated as
+# Composite radices used by the register-resident two-stage line FFTs (Ud2S, ud_fft.cuh): R = Ra * Rb evaluated as
 # Rb sub-DFTs of size Ra, constant twiddles W_R^(nb*ka) (literals), then Ra sub-DFTs of size Rb.  Natural order in
 # and out:  v[n], n = Rb*na + nb  ->  X[ka + Ra*kb].
 COMPOSITES = [(8, 2, 4), (12, 4, 3), (14, 2, 7), (16, 4, 4), (20, 4, 5)]

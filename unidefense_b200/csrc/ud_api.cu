@@ -110,115 +110,86 @@ static void twiddle_host(int n, std::vector<float2>& out) {
 }
 
 static std::mutex g_tw_mutex;
-static std::map<std::pair<int, int>, float2*> g_tw_cache;
 
-const float2* ud_twiddles(int n) {
+// Device copy of a host-built table, uploaded on the first request for (current device, key) and kept for the process
+// lifetime (mutex-guarded, never freed).  `build` fills the host vector; `what` (a printf format over `args`) names
+// the table in error messages.  nullptr on failure (error set).
+template <class T, class Key, class Build, class... Args>
+static const T* ud_cached_table(std::map<std::pair<int, Key>, T*>& cache, const Key& key, Build build, const char* what,
+                                Args... args) {
   int dev = 0;
   if (cudaGetDevice(&dev) != cudaSuccess) {
     ud_set_error("cudaGetDevice failed");
     return nullptr;
   }
   std::lock_guard<std::mutex> lock(g_tw_mutex);
-  auto key = std::make_pair(dev, n);
-  auto it = g_tw_cache.find(key);
-  if (it != g_tw_cache.end()) return it->second;
-  std::vector<float2> h;
-  twiddle_host(n, h);
-  float2* d = nullptr;
-  if (cudaMalloc(&d, sizeof(float2) * (size_t)n) != cudaSuccess) {
-    ud_set_error("cudaMalloc(twiddles n=%d) failed", n);
+  const auto ck = std::make_pair(dev, key);
+  auto it = cache.find(ck);
+  if (it != cache.end()) return it->second;
+  std::vector<T> h;
+  build(h);
+  char name[96];
+  snprintf(name, sizeof(name), what, args...);
+  T* d = nullptr;
+  if (cudaMalloc(&d, sizeof(T) * h.size()) != cudaSuccess) {
+    ud_set_error("cudaMalloc(%s) failed", name);
     return nullptr;
   }
   // synchronous copy on the legacy stream: tables are immutable afterwards, and any stream
   // that later reads them is ordered after this call returns.
-  if (cudaMemcpy(d, h.data(), sizeof(float2) * (size_t)n, cudaMemcpyHostToDevice) != cudaSuccess) {
-    ud_set_error("cudaMemcpy(twiddles n=%d) failed", n);
+  if (cudaMemcpy(d, h.data(), sizeof(T) * h.size(), cudaMemcpyHostToDevice) != cudaSuccess) {
+    ud_set_error("cudaMemcpy(%s) failed", name);
     cudaFree(d);
     return nullptr;
   }
-  g_tw_cache[key] = d;
+  cache[ck] = d;
   return d;
+}
+
+static std::map<std::pair<int, int>, float2*> g_tw_cache;
+
+const float2* ud_twiddles(int n) {
+  return ud_cached_table(g_tw_cache, n, [&](std::vector<float2>& h) { twiddle_host(n, h); }, "twiddles n=%d", n);
 }
 
 static std::map<std::pair<int, std::pair<int, int>>, float2*> g_lerp_cache;
 
 const float2* ud_lerp_table(int in, int out) {
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) {
-    ud_set_error("cudaGetDevice failed");
-    return nullptr;
-  }
-  std::lock_guard<std::mutex> lock(g_tw_mutex);
-  auto key = std::make_pair(dev, std::make_pair(in, out));
-  auto it = g_lerp_cache.find(key);
-  if (it != g_lerp_cache.end()) return it->second;
-  std::vector<float2> h((size_t)out);
-  const float scale = ud_ac_scale(in, out);
-  for (int d = 0; d < out; ++d) {
-    const float src = scale * (float)d;       // ATen: area_pixel_compute_source_index, align_corners=True
-    const int i0 = (int)src;
-    union { int i; float f; } u;
-    u.i = i0;
-    h[d] = make_float2(u.f, src - (float)i0);
-  }
-  float2* p = nullptr;
-  if (cudaMalloc(&p, sizeof(float2) * (size_t)out) != cudaSuccess) {
-    ud_set_error("cudaMalloc(lerp table %d->%d) failed", in, out);
-    return nullptr;
-  }
-  if (cudaMemcpy(p, h.data(), sizeof(float2) * (size_t)out, cudaMemcpyHostToDevice) != cudaSuccess) {
-    ud_set_error("cudaMemcpy(lerp table %d->%d) failed", in, out);
-    cudaFree(p);
-    return nullptr;
-  }
-  g_lerp_cache[key] = p;
-  return p;
+  auto build = [&](std::vector<float2>& h) {
+    h.resize((size_t)out);
+    const float scale = ud_ac_scale(in, out);
+    for (int d = 0; d < out; ++d) {
+      const float src = scale * (float)d;       // ATen: area_pixel_compute_source_index, align_corners=True
+      const int i0 = (int)src;
+      union { int i; float f; } u;
+      u.i = i0;
+      h[d] = make_float2(u.f, src - (float)i0);
+    }
+  };
+  return ud_cached_table(g_lerp_cache, std::make_pair(in, out), build, "lerp table %d->%d", in, out);
 }
 
 static std::map<std::pair<int, std::pair<int, int>>, int2*> g_range_cache;
 
 const int2* ud_lerp_ranges(int in, int out) {
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) {
-    ud_set_error("cudaGetDevice failed");
-    return nullptr;
-  }
-  std::lock_guard<std::mutex> lock(g_tw_mutex);
-  auto key = std::make_pair(dev, std::make_pair(in, out));
-  auto it = g_range_cache.find(key);
-  if (it != g_range_cache.end()) return it->second;
-  std::vector<int2> h((size_t)in, make_int2(out, -1));
-  const float scale = ud_ac_scale(in, out);
-  for (int d = 0; d < out; ++d) {
-    const float src = scale * (float)d;
-    const int i0 = (int)src;
-    const int i1 = i0 + ((i0 < in - 1) ? 1 : 0);
-    for (int i : {i0, i1}) {
-      if (d < h[i].x) h[i].x = d;
-      if (d > h[i].y) h[i].y = d;
+  auto build = [&](std::vector<int2>& h) {
+    h.assign((size_t)in, make_int2(out, -1));
+    const float scale = ud_ac_scale(in, out);
+    for (int d = 0; d < out; ++d) {
+      const float src = scale * (float)d;
+      const int i0 = (int)src;
+      const int i1 = i0 + ((i0 < in - 1) ? 1 : 0);
+      for (int i : {i0, i1}) {
+        if (d < h[i].x) h[i].x = d;
+        if (d > h[i].y) h[i].y = d;
+      }
     }
-  }
-  int2* p = nullptr;
-  if (cudaMalloc(&p, sizeof(int2) * (size_t)in) != cudaSuccess) {
-    ud_set_error("cudaMalloc(lerp ranges %d->%d) failed", in, out);
-    return nullptr;
-  }
-  if (cudaMemcpy(p, h.data(), sizeof(int2) * (size_t)in, cudaMemcpyHostToDevice) != cudaSuccess) {
-    ud_set_error("cudaMemcpy(lerp ranges %d->%d) failed", in, out);
-    cudaFree(p);
-    return nullptr;
-  }
-  g_range_cache[key] = p;
-  return p;
+  };
+  return ud_cached_table(g_range_cache, std::make_pair(in, out), build, "lerp ranges %d->%d", in, out);
 }
 
-
 // ---- Bluestein tables (ud_fft_any.cuh) -------------------------------------------------------------
-struct BluesteinTables {
-  float2* chirp;
-  float2* bhat;
-};
-static std::map<std::pair<int, int>, BluesteinTables> g_bs_cache;
+static std::map<std::pair<int, int>, float2*> g_chirp_cache, g_bhat_cache;
 
 // in-place radix-2 FFT in double precision (host, table construction only)
 static void host_fft_pow2(std::vector<double>& re, std::vector<double>& im) {
@@ -280,22 +251,26 @@ bool ud_make_any_plan(int n, UdAnyPlan* plan) {
   }
   plan->tw = ud_twiddles(m);
   if (!plan->tw) return false;
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess) {
-    ud_set_error("cudaGetDevice failed");
-    return false;
-  }
-  std::lock_guard<std::mutex> lock(g_tw_mutex);
-  auto key = std::make_pair(dev, n);
-  auto it = g_bs_cache.find(key);
-  if (it == g_bs_cache.end()) {
-    std::vector<double> wr(n), wi(n), br(m, 0.0), bi(m, 0.0);
+  // w[j] = exp(-i pi j^2 / n), the phase pi * j^2 / n reduced mod 2 pi in integer arithmetic
+  auto chirp = [n](std::vector<double>& wr, std::vector<double>& wi) {
+    wr.resize(n);
+    wi.resize(n);
     for (int j = 0; j < n; ++j) {
-      const long long q = ((long long)j * j) % (2LL * n);      // phase pi * j^2 / n reduced mod 2 pi
+      const long long q = ((long long)j * j) % (2LL * n);
       const double ang = M_PI * (double)q / (double)n;
       wr[j] = cos(ang);
-      wi[j] = -sin(ang);                                       // w[j] = exp(-i pi j^2 / n)
+      wi[j] = -sin(ang);
     }
+  };
+  plan->chirp = ud_cached_table(g_chirp_cache, n, [&](std::vector<float2>& hc) {
+    std::vector<double> wr, wi;
+    chirp(wr, wi);
+    hc.resize(n);
+    for (int j = 0; j < n; ++j) hc[j] = make_float2((float)wr[j], (float)wi[j]);
+  }, "Bluestein chirp n=%d", n);
+  if (plan->chirp) plan->bhat = ud_cached_table(g_bhat_cache, n, [&](std::vector<float2>& hb) {
+    std::vector<double> wr, wi, br(m, 0.0), bi(m, 0.0);
+    chirp(wr, wi);
     for (int t = 0; t < n; ++t) {                              // conj(w), even in t, wrapped to length m
       br[t] = wr[t];
       bi[t] = -wi[t];
@@ -305,22 +280,12 @@ bool ud_make_any_plan(int n, UdAnyPlan* plan) {
       }
     }
     host_fft_pow2(br, bi);
-    std::vector<float2> hc(n), hb(m);
-    for (int j = 0; j < n; ++j) hc[j] = make_float2((float)wr[j], (float)wi[j]);
+    hb.resize(m);
     for (int k = 0; k < m; ++k) hb[k] = make_float2((float)(br[k] / m), (float)(bi[k] / m));
-    BluesteinTables t = {nullptr, nullptr};
-    if (cudaMalloc(&t.chirp, sizeof(float2) * (size_t)n) != cudaSuccess ||
-        cudaMalloc(&t.bhat, sizeof(float2) * (size_t)m) != cudaSuccess ||
-        cudaMemcpy(t.chirp, hc.data(), sizeof(float2) * (size_t)n, cudaMemcpyHostToDevice) != cudaSuccess ||
-        cudaMemcpy(t.bhat, hb.data(), sizeof(float2) * (size_t)m, cudaMemcpyHostToDevice) != cudaSuccess) {
-      ud_set_error("Bluestein tables for n=%d: allocation or copy failed", n);
-      if (t.chirp) cudaFree(t.chirp);
-      if (t.bhat) cudaFree(t.bhat);
-      return false;
-    }
-    it = g_bs_cache.emplace(key, t).first;
+  }, "Bluestein bhat n=%d", n);
+  if (!plan->bhat) {
+    ud_set_error("Bluestein tables for n=%d: allocation or copy failed", n);
+    return false;
   }
-  plan->chirp = it->second.chirp;
-  plan->bhat = it->second.bhat;
   return true;
 }

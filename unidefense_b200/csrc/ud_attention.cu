@@ -255,18 +255,6 @@ static int at_check_small(const char* what, int N, int C, int h, int w) {
   return UD_OK;
 }
 
-template <class K>
-static int at_set_smem(K k, size_t bytes) {
-  if (bytes > (48u << 10)) {
-    cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-    if (e != cudaSuccess) {
-      ud_set_error("cudaFuncSetAttribute(%zu) failed: %s", bytes, cudaGetErrorString(e));
-      return UD_ERR_CUDA;
-    }
-  }
-  return UD_OK;
-}
-
 static float at_scale(int h, int w, int norm_ortho, bool inverse) {
   if (norm_ortho) return 1.f / sqrtf((float)h * (float)w);
   return inverse ? 1.f / ((float)h * (float)w) : 1.f;
@@ -280,7 +268,7 @@ int ud_rfft2_small(const float* x, float* xf, int N, int C, int h, int w, int no
   int rc;
   const int P = at_planes_per_cta(h, w);
   const size_t smem = at_smem_bytes(h, w, P);
-  if ((rc = at_set_smem(at_r2c_kernel, smem)) != UD_OK) return rc;
+  if ((rc = ud_set_smem(at_r2c_kernel, smem, "rfft2_cat")) != UD_OK) return rc;
   const int planes = N * C;
   const float scale = at_scale(h, w, norm_ortho, adjoint_of_inverse != 0);
   at_r2c_kernel<<<ud_cdiv(planes, P), AT_THREADS, smem, stream>>>(x, xf, planes, C, h, w, scale, adjoint_of_inverse, P);
@@ -294,7 +282,7 @@ int ud_irfft2_small(const float* xf, const float* mask, float* y, int N, int C, 
   int rc;
   const int P = at_planes_per_cta(h, w);
   const size_t smem = at_smem_bytes(h, w, P);
-  if ((rc = at_set_smem(at_c2r_kernel, smem)) != UD_OK) return rc;
+  if ((rc = ud_set_smem(at_c2r_kernel, smem, "irfft2_cat")) != UD_OK) return rc;
   const int planes = N * C;
   const float scale = at_scale(h, w, norm_ortho, adjoint_of_forward == 0);
   at_c2r_kernel<<<ud_cdiv(planes, P), AT_THREADS, smem, stream>>>(xf, mask, y, planes, C, h, w, scale,
@@ -366,7 +354,7 @@ extern "C" int ud_attn_prep(const float* pred, const float* x, float* spat_diff,
   if (N == 0) return UD_OK;
   UD_REQUIRE(pred && x && spat_diff && freq_diff, UD_ERR_INVALID, "attn_prep: null pointer");
   const size_t smem = at_smem_bytes(h, w, 1);
-  if ((rc = at_set_smem(at_prep_kernel, smem)) != UD_OK) return rc;
+  if ((rc = ud_set_smem(at_prep_kernel, smem, "attn_prep")) != UD_OK) return rc;
   at_prep_kernel<<<N * C, AT_THREADS, smem, stream>>>(pred, x, spat_diff, freq_diff, C, hp, wp, Hx, Wx, h, w,
                                                       ud_ac_scale(hp, h), ud_ac_scale(wp, w), ud_ac_scale(Hx, h),
                                                       ud_ac_scale(Wx, w), at_scale(h, w, norm_ortho, false));
@@ -470,7 +458,7 @@ extern "C" int ud_attn_prep_bwd(const float* pred, const float* x, const float* 
   if (N == 0) return UD_OK;
   UD_REQUIRE(pred && x && g_x, UD_ERR_INVALID, "attn_prep_bwd: null pointer");
   const size_t smem = sizeof(float2) * (size_t)(w + h) + sizeof(float) * (size_t)at_slot_floats(h, w);
-  if ((rc = at_set_smem(at_prep_bwd_kernel, smem)) != UD_OK) return rc;
+  if ((rc = ud_set_smem(at_prep_bwd_kernel, smem, "attn_prep_bwd")) != UD_OK) return rc;
   at_prep_bwd_kernel<<<dim3(ud_cdiv(Hx, AT_BWD_ROWS), N * C), AT_THREADS, smem, stream>>>(
       pred, x, g_spat_diff, g_freq_diff, g_x, C, hp, wp, Hx, Wx, h, w, ud_ac_scale(hp, h), ud_ac_scale(wp, w),
       ud_ac_scale(Hx, h), ud_ac_scale(Wx, w), at_scale(h, w, norm_ortho, false));

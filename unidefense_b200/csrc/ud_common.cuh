@@ -36,6 +36,19 @@ static inline int ud_cdiv(long long a, long long b) { return (int)((a + b - 1) /
 static inline size_t ud_align_up(size_t a, size_t b) { return (a + b - 1) / b * b; }
 
 #define UD_NUM_SMS 148
+#define UD_SMEM_CTA_MAX (227u << 10)   // dynamic shared memory one CTA may use on sm_100a
+
+// Lets `kernel` launch with `bytes` of dynamic shared memory: UD_ERR_UNSUPPORTED above UD_SMEM_CTA_MAX, UD_ERR_CUDA
+// when the attribute cannot be set (dynamic plus static bytes over the limit).  `what` names the op in the message.
+template <class K>
+static int ud_set_smem(K kernel, size_t bytes, const char* what) {
+  UD_REQUIRE(bytes <= UD_SMEM_CTA_MAX, UD_ERR_UNSUPPORTED, "%s: needs %zu bytes of shared memory per CTA (> 227 KB)",
+             what, bytes);
+  const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  UD_REQUIRE(e == cudaSuccess, UD_ERR_CUDA, "%s: cudaFuncSetAttribute(smem=%zu) failed: %s", what, bytes,
+             cudaGetErrorString(e));
+  return UD_OK;
+}
 
 __device__ __forceinline__ float ud_warp_sum(float v) {
 #pragma unroll
@@ -131,6 +144,13 @@ __device__ __forceinline__ UdLerp ud_lerp_ac(int dst, int in_size, float scale) 
   r.l1 = src - (float)r.i0;
   r.l0 = 1.f - r.l1;
   return r;
+}
+// The same taps from an entry t of a host-built table (ud_lerp_table: t = {__int_as_float(i0), l1}).
+__device__ __forceinline__ void ud_lerp_tab(const float2 t, int in_size, int& i0, int& i1, float& l0, float& l1) {
+  i0 = __float_as_int(t.x);
+  i1 = i0 + ((i0 < in_size - 1) ? 1 : 0);
+  l1 = t.y;
+  l0 = 1.f - l1;
 }
 static inline float ud_ac_scale(int in_size, int out_size) {
   return out_size > 1 ? (float)(in_size - 1) / (float)(out_size - 1) : 0.f;

@@ -10,9 +10,9 @@
 // Natural order in, natural order out, ping-pong between two buffers.  Forward sign only;
 // the inverse is obtained by the callers by swapping re/im on load and store.
 //
-// Plans: StaticPlan<N, R0, R1, ...> (all index arithmetic constant-folded) for the sizes the
-// reference's configs use (224, 256, 299, 380; SURVEY.md App. A.1) and DynPlan for any other
-// n whose prime factors are <= 23.
+// Plans: UdStaticPlanIP<N, L, THREADS, R0, R1, ...> (in place, all index arithmetic constant-folded) for the
+// configured lengths (UdConfigured below) and UdDynPlan for any n whose prime factors are <= 23.  The configured
+// lengths also have a register-resident two-stage plan (Ud2S).
 #pragma once
 #include "ud_common.cuh"
 #include "ud_fft_bfly_gen.cuh"
@@ -23,44 +23,17 @@ __device__ __forceinline__ float2 ud_cmul(float2 a, float2 b) {
   return make_float2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x);
 }
 
+// Radix-R butterfly, forward sign, in place: the generated straight-line code of ud_fft_bfly_gen.cuh
 template <int R>
 struct UdBfly;
-template <>
-struct UdBfly<2> {
-  static __device__ __forceinline__ void run(float2 (&v)[2]) {
-    const float2 a = v[0], b = v[1];
-    v[0] = make_float2(a.x + b.x, a.y + b.y);
-    v[1] = make_float2(a.x - b.x, a.y - b.y);
-  }
-};
-template <>
-struct UdBfly<4> {
-  static __device__ __forceinline__ void run(float2 (&v)[4]) {
-    const float2 s02 = make_float2(v[0].x + v[2].x, v[0].y + v[2].y);
-    const float2 d02 = make_float2(v[0].x - v[2].x, v[0].y - v[2].y);
-    const float2 s13 = make_float2(v[1].x + v[3].x, v[1].y + v[3].y);
-    const float2 d13 = make_float2(v[1].x - v[3].x, v[1].y - v[3].y);
-    v[0] = make_float2(s02.x + s13.x, s02.y + s13.y);
-    v[2] = make_float2(s02.x - s13.x, s02.y - s13.y);
-    // forward: X1 = d02 - i*d13, X3 = d02 + i*d13;  -i*(a+bi) = b - ai
-    v[1] = make_float2(d02.x + d13.y, d02.y - d13.x);
-    v[3] = make_float2(d02.x - d13.y, d02.y + d13.x);
-  }
-};
-#define UD_BFLY_PRIME(P)                                                              \
-  template <>                                                                         \
-  struct UdBfly<P> {                                                                  \
-    static __device__ __forceinline__ void run(float2 (&v)[P]) { ud_bfly##P(v); }     \
+#define UD_BFLY(R)                                                                \
+  template <>                                                                     \
+  struct UdBfly<R> {                                                              \
+    static __device__ __forceinline__ void run(float2 (&v)[R]) { ud_bfly##R(v); } \
   };
-UD_BFLY_PRIME(3)
-UD_BFLY_PRIME(5)
-UD_BFLY_PRIME(7)
-UD_BFLY_PRIME(11)
-UD_BFLY_PRIME(13)
-UD_BFLY_PRIME(17)
-UD_BFLY_PRIME(19)
-UD_BFLY_PRIME(23)
-#undef UD_BFLY_PRIME
+UD_BFLY(2) UD_BFLY(3) UD_BFLY(4) UD_BFLY(5) UD_BFLY(7) UD_BFLY(8) UD_BFLY(11) UD_BFLY(12) UD_BFLY(13) UD_BFLY(14)
+UD_BFLY(16) UD_BFLY(17) UD_BFLY(19) UD_BFLY(20) UD_BFLY(23)
+#undef UD_BFLY
 
 // One Stockham stage over L lines.  tw[t] = exp(-2 pi i t / n), t in [0, n).
 template <int R>
@@ -92,34 +65,6 @@ __device__ __forceinline__ void ud_fft_stage(const float2* __restrict__ in, floa
 }
 
 // ---- plans ---------------------------------------------------------------------------
-template <int N, int NS, int... Rs>
-struct UdStaticStages;
-template <int N, int NS>
-struct UdStaticStages<N, NS> {
-  static __device__ __forceinline__ float2* run(float2* a, float2*, const float2*, int, int) { return a; }
-};
-template <int N, int NS, int R0, int... Rest>
-struct UdStaticStages<N, NS, R0, Rest...> {
-  static __device__ __forceinline__ float2* run(float2* a, float2* b, const float2* tw, int L, int LS) {
-    ud_fft_stage<R0>(a, b, tw, N, NS, L, LS);
-    __syncthreads();
-    return UdStaticStages<N, NS * R0, Rest...>::run(b, a, tw, L, LS);
-  }
-};
-
-template <int N, int... Rs>
-struct UdStaticPlan {
-  static constexpr bool kInPlace = false;
-  static constexpr int kN = N;
-  __device__ __forceinline__ int n() const { return N; }
-  __device__ __forceinline__ int line_len() const { return N; }      // points a line buffer must hold
-  // Runs all stages; data must be in `a` and visible (caller synced).  Returns the buffer
-  // holding the result; ends with a __syncthreads().
-  __device__ __forceinline__ float2* run(float2* a, float2* b, const float2* tw, int L, int LS) const {
-    return UdStaticStages<N, 1, Rs...>::run(a, b, tw, L, LS);
-  }
-};
-
 struct UdDynPlan {
   static constexpr bool kInPlace = false;
   int n_;
@@ -220,7 +165,6 @@ struct UdIpStages<N, NS, L, THREADS, R0, Rest...> {
 template <int N, int L, int THREADS, int... Rs>
 struct UdStaticPlanIP {
   static constexpr bool kInPlace = true;
-  static constexpr int kN = N;
   __device__ __forceinline__ int n() const { return N; }
   __device__ __forceinline__ int line_len() const { return N; }
   __device__ __forceinline__ float2* run(float2* a, float2*, const float2* tw, int, int) const {
@@ -229,10 +173,94 @@ struct UdStaticPlanIP {
   }
 };
 
-typedef UdStaticPlan<380, 19, 5, 4> UdPlan380;
-typedef UdStaticPlan<256, 4, 4, 4, 4> UdPlan256;
-typedef UdStaticPlan<224, 7, 4, 4, 2> UdPlan224;
-typedef UdStaticPlan<299, 23, 13> UdPlan299;
+// ---- register-resident two-stage plans -----------------------------------------------------------
+// A line of N = R1 * R2 complex points is owned by TL = max(R1, R2) threads.  Cooley-Tukey, decimation in time:
+//     n = R2*n1 + n2,  k = k1 + R1*k2
+//     stage A: thread n2 (< R2) holds x[n2 + R2*n1], n1 = 0..R1-1 in registers, runs ONE radix-R1 butterfly
+//              (generated straight-line code with literal twiddles), multiplies by W_N^(n2*k1) and writes
+//              S[k1*P + n2] to shared memory (P = R2|1: conflict-free for the column reads that follow);
+//     stage B: thread k1 (< R1) reads S[k1*P + n2], n2 = 0..R2-1, runs ONE radix-R2 butterfly and holds
+//              X[k1 + R1*k2], k2 = 0..R2-1.
+// One shared-memory exchange and one barrier per line instead of one per radix stage, no index arithmetic inside
+// the butterflies (a thread's role is fixed), and global loads/stores happen straight from/to the registers the
+// butterflies use: for a fixed n1 (k2) the TL threads of a line touch R2 (R1) consecutive elements.
+// Forward sign only; callers obtain the inverse with the re/im swap trick.
+template <int N_, int R1_, int R2_>
+struct Ud2S {
+  static_assert(R1_ * R2_ == N_, "N = R1 * R2");
+  static constexpr int N = N_, R1 = R1_, R2 = R2_;
+  static constexpr int TL = R1_ > R2_ ? R1_ : R2_;                     // threads per line
+  static constexpr int P = R2_ | 1;                                    // pitch of the exchange layout
+  static constexpr int LS = ((R1_ * P > N_ ? R1_ * P : N_) | 1);       // float2 slots of one line buffer
+};
+
+// tw2[k1*P + n2] = exp(-2 pi i n2 k1 / N), from the library's global table tw_g[t] = exp(-2 pi i t / N)
+template <class PL>
+__device__ __forceinline__ void ud2s_build_tw(float2* __restrict__ tw2, const float2* __restrict__ tw_g) {
+  for (int t = threadIdx.x; t < PL::R1 * PL::P; t += blockDim.x) {
+    const int k1 = t / PL::P, n2 = t - k1 * PL::P;
+    tw2[t] = (n2 < PL::R2) ? __ldg(tw_g + n2 * k1) : make_float2(0.f, 0.f);
+  }
+}
+
+// stage A on the thread's R1 values (z[n1] = x[n2 + R2*n1]); results go to the line's exchange buffer S
+template <class PL>
+__device__ __forceinline__ void ud2s_stage_a(float2 (&z)[PL::R1], int n2, const float2* __restrict__ tw2,
+                                             float2* __restrict__ S) {
+  UdBfly<PL::R1>::run(z);
+  S[n2] = z[0];
+#pragma unroll
+  for (int k1 = 1; k1 < PL::R1; ++k1) {
+    const float2 t = tw2[k1 * PL::P + n2];
+    S[k1 * PL::P + n2] = make_float2(z[k1].x * t.x - z[k1].y * t.y, z[k1].x * t.y + z[k1].y * t.x);
+  }
+}
+
+// stage B: u[k2] = X[k1 + R1*k2]
+template <class PL>
+__device__ __forceinline__ void ud2s_stage_b(float2 (&u)[PL::R2], int k1, const float2* __restrict__ S) {
+#pragma unroll
+  for (int n2 = 0; n2 < PL::R2; ++n2) u[n2] = S[k1 * PL::P + n2];
+  UdBfly<PL::R2>::run(u);
+}
+
+// ---- configured lengths -------------------------------------------------------------------------------
+// The image sizes of the reference's configs (SURVEY.md App. A.1) get compile-time plans: the in-place Stockham plan
+// IP<L, THREADS> (L lines per CTA) and the two-stage plan TwoStage.  Every other length runs a run-time plan.
+template <int N>
+struct UdConfigured;
+template <>
+struct UdConfigured<380> {
+  template <int L, int T> using IP = UdStaticPlanIP<380, L, T, 19, 5, 4>;
+  using TwoStage = Ud2S<380, 20, 19>;
+};
+template <>
+struct UdConfigured<256> {
+  template <int L, int T> using IP = UdStaticPlanIP<256, L, T, 4, 4, 4, 4>;
+  using TwoStage = Ud2S<256, 16, 16>;
+};
+template <>
+struct UdConfigured<224> {
+  template <int L, int T> using IP = UdStaticPlanIP<224, L, T, 7, 4, 4, 2>;
+  using TwoStage = Ud2S<224, 16, 14>;
+};
+template <>
+struct UdConfigured<299> {
+  template <int L, int T> using IP = UdStaticPlanIP<299, L, T, 23, 13>;
+  using TwoStage = Ud2S<299, 13, 23>;
+};
+// Runs the body with the type `CFG` bound to UdConfigured<n> when n is a configured length, and `other` otherwise.
+#define UD_FFT_CONFIGURED(n, CFG, other, ...)                              \
+  do {                                                                     \
+    if ((n) == 380) { using CFG = UdConfigured<380>; __VA_ARGS__; }        \
+    else if ((n) == 256) { using CFG = UdConfigured<256>; __VA_ARGS__; }   \
+    else if ((n) == 224) { using CFG = UdConfigured<224>; __VA_ARGS__; }   \
+    else if ((n) == 299) { using CFG = UdConfigured<299>; __VA_ARGS__; }   \
+    else { other; }                                                        \
+  } while (0)
+static inline bool ud_fft_configured(int n) {
+  UD_FFT_CONFIGURED(n, CFG, return false, return true);
+}
 
 // ---- host side -----------------------------------------------------------------------
 // Factorises n into supported radices (largest odd primes first, then 4s, then a 2).
@@ -248,5 +276,3 @@ const float2* ud_lerp_table(int in, int out);
 // For the transposed resize: entry j (0 <= j < in) = {first, last} output sample whose taps (i0 or i1)
 // include input sample j; first > last when none does.  Derived from the same fp32 table.
 const int2* ud_lerp_ranges(int in, int out);
-// padded line stride (odd) for n-point lines
-static inline int ud_line_stride(int n) { return n | 1; }

@@ -27,26 +27,12 @@ int ud_irfft2_small(const float* xf, const float* mask, float* y, int N, int C, 
                     int adjoint_of_forward, cudaStream_t stream);
 bool ud_fft2_small_ok(int h, int w);
 
-static bool f2_static(int n) { return n == 380 || n == 256 || n == 224 || n == 299; }
-// runs the body with PL bound to the static in-place plan of n (L = F2_L lines) or to the run-time plan `any`
-#define F2_DISPATCH(n, any, PL, Lvar, ...)                                                                       \
-  do {                                                                                                           \
-    if ((n) == 380) { UdStaticPlanIP<380, F2_L, F2_THREADS, 19, 5, 4> PL; const int Lvar = F2_L; __VA_ARGS__; }   \
-    else if ((n) == 256) { UdStaticPlanIP<256, F2_L, F2_THREADS, 4, 4, 4, 4> PL; const int Lvar = F2_L; __VA_ARGS__; } \
-    else if ((n) == 224) { UdStaticPlanIP<224, F2_L, F2_THREADS, 7, 4, 4, 2> PL; const int Lvar = F2_L; __VA_ARGS__; } \
-    else if ((n) == 299) { UdStaticPlanIP<299, F2_L, F2_THREADS, 23, 13> PL; const int Lvar = F2_L; __VA_ARGS__; } \
-    else { UdAnyPlan PL = (any); const int Lvar = f2_lines(any); __VA_ARGS__; }                                  \
-  } while (0)
-
 static int f2_lines(const UdAnyPlan& p) {
   const int L = ud_any_lines(p.m, 0, 0, 96u << 10, 16);   // 96 KB of line buffers (the twiddles come on top)
   return L < 1 ? 1 : L;
 }
 static size_t f2_smem(const UdAnyPlan& p, int L) {
   return sizeof(float2) * ((size_t)p.m + 2ull * L * ud_any_line_stride(p));
-}
-static size_t f2_smem_n(int n, const UdAnyPlan& p, int L) {      // static plans: m = n, same two-buffer layout
-  return f2_static(n) ? sizeof(float2) * ((size_t)n + 2ull * L * (size_t)(n | 1)) : f2_smem(p, L);
 }
 
 // Plans: UdAnyPlan (any size, run time) or the in-place static plans of the configured image sizes (every index
@@ -199,11 +185,11 @@ f2_rows_c2r_kernel(Plan plan, const float2* __restrict__ tw_g, const float2* __r
   }
 }
 
-template <class K>
-static int f2_set_smem(K k, size_t bytes) {
-  UD_REQUIRE(bytes <= (227u << 10), UD_ERR_UNSUPPORTED, "fft2: needs %zu bytes of shared memory per CTA", bytes);
-  UD_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-  return UD_OK;
+// Runs launch(plan, L) with n's plan: the configured length's in-place plan at F2_L lines per CTA, or the run-time
+// plan `any` (m = n for every configured length, so both share f2_smem).
+template <class F>
+static int f2_run(int n, const UdAnyPlan& any, F launch) {
+  UD_FFT_CONFIGURED(n, CFG, return launch(any, f2_lines(any)), return launch(CFG::IP<F2_L, F2_THREADS>(), F2_L));
 }
 
 static float f2_scale(int h, int w, int norm_ortho, bool inverse) {
@@ -239,20 +225,23 @@ extern "C" int ud_rfft2(const float* x, float* xf, void* ws, size_t ws_bytes, in
   const float scale = f2_scale(h, w, norm_ortho, adjoint_of_inverse != 0);
   for (int p0 = 0; p0 < planes; p0 += F2_MAX_GRID_Y) {            // gridDim.y <= 65535
     const int np = planes - p0 < F2_MAX_GRID_Y ? planes - p0 : F2_MAX_GRID_Y;
-    F2_DISPATCH(w, pw, pl, L, {
+    rc = f2_run(w, pw, [&](auto pl, int L) {
       auto k = f2_rows_r2c_kernel<decltype(pl)>;
-      const size_t sm = f2_smem_n(w, pw, L);
-      if ((rc = f2_set_smem(k, sm)) != UD_OK) return rc;
-      k<<<dim3(ud_cdiv((h + 1) / 2, L), np), F2_THREADS, sm, stream>>>(pl, pw.tw, x, T, h, w, L, p0);
+      const size_t sm = f2_smem(pw, L);
+      const int e = ud_set_smem(k, sm, "fft2");
+      if (e == UD_OK) k<<<dim3(ud_cdiv((h + 1) / 2, L), np), F2_THREADS, sm, stream>>>(pl, pw.tw, x, T, h, w, L, p0);
+      return e;
     });
-    if ((rc = ud_check_launch("rfft2_rows")) != UD_OK) return rc;
-    F2_DISPATCH(h, ph, pl, L, {
+    if (rc != UD_OK || (rc = ud_check_launch("rfft2_rows")) != UD_OK) return rc;
+    rc = f2_run(h, ph, [&](auto pl, int L) {
       auto k = f2_cols_fwd_kernel<decltype(pl)>;
-      const size_t sm = f2_smem_n(h, ph, L);
-      if ((rc = f2_set_smem(k, sm)) != UD_OK) return rc;
-      k<<<dim3(ud_cdiv(wh, L), np), F2_THREADS, sm, stream>>>(pl, ph.tw, T, xf, C, h, w, L, scale, adjoint_of_inverse, p0);
+      const size_t sm = f2_smem(ph, L);
+      const int e = ud_set_smem(k, sm, "fft2");
+      if (e == UD_OK)
+        k<<<dim3(ud_cdiv(wh, L), np), F2_THREADS, sm, stream>>>(pl, ph.tw, T, xf, C, h, w, L, scale, adjoint_of_inverse, p0);
+      return e;
     });
-    if ((rc = ud_check_launch("rfft2_cols")) != UD_OK) return rc;
+    if (rc != UD_OK || (rc = ud_check_launch("rfft2_cols")) != UD_OK) return rc;
   }
   return UD_OK;
 }
@@ -272,20 +261,23 @@ extern "C" int ud_irfft2(const float* xf, const float* mask, float* y, void* ws,
   const float scale = f2_scale(h, w, norm_ortho, adjoint_of_forward == 0);
   for (int p0 = 0; p0 < planes; p0 += F2_MAX_GRID_Y) {
     const int np = planes - p0 < F2_MAX_GRID_Y ? planes - p0 : F2_MAX_GRID_Y;
-    F2_DISPATCH(h, ph, pl, L, {
+    rc = f2_run(h, ph, [&](auto pl, int L) {
       auto k = f2_cols_inv_kernel<decltype(pl)>;
-      const size_t sm = f2_smem_n(h, ph, L);
-      if ((rc = f2_set_smem(k, sm)) != UD_OK) return rc;
-      k<<<dim3(ud_cdiv(wh, L), np), F2_THREADS, sm, stream>>>(pl, ph.tw, xf, mask, T, C, h, w, L, adjoint_of_forward ? 0 : 1, p0);
+      const size_t sm = f2_smem(ph, L);
+      const int e = ud_set_smem(k, sm, "fft2");
+      if (e == UD_OK)
+        k<<<dim3(ud_cdiv(wh, L), np), F2_THREADS, sm, stream>>>(pl, ph.tw, xf, mask, T, C, h, w, L, adjoint_of_forward ? 0 : 1, p0);
+      return e;
     });
-    if ((rc = ud_check_launch("irfft2_cols")) != UD_OK) return rc;
-    F2_DISPATCH(w, pw, pl, L, {
+    if (rc != UD_OK || (rc = ud_check_launch("irfft2_cols")) != UD_OK) return rc;
+    rc = f2_run(w, pw, [&](auto pl, int L) {
       auto k = f2_rows_c2r_kernel<decltype(pl)>;
-      const size_t sm = f2_smem_n(w, pw, L);
-      if ((rc = f2_set_smem(k, sm)) != UD_OK) return rc;
-      k<<<dim3(ud_cdiv(h, L), np), F2_THREADS, sm, stream>>>(pl, pw.tw, T, y, h, w, L, scale, p0);
+      const size_t sm = f2_smem(pw, L);
+      const int e = ud_set_smem(k, sm, "fft2");
+      if (e == UD_OK) k<<<dim3(ud_cdiv(h, L), np), F2_THREADS, sm, stream>>>(pl, pw.tw, T, y, h, w, L, scale, p0);
+      return e;
     });
-    if ((rc = ud_check_launch("irfft2_rows")) != UD_OK) return rc;
+    if (rc != UD_OK || (rc = ud_check_launch("irfft2_rows")) != UD_OK) return rc;
   }
   return UD_OK;
 }

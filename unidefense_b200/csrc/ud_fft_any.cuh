@@ -70,8 +70,6 @@ int ud_any_line_len(int n);
 // odd line stride for a plan's line buffers
 static inline int ud_any_line_stride(const UdAnyPlan& p) { return p.m | 1; }
 
-#define UD_SMEM_CTA_MAX (227u << 10)   // dynamic shared memory one CTA may use on sm_100a
-
 // Host: lines per CTA of a kernel that keeps two ping-pong buffers of (m | 1) points per line: the largest L <= lmax for
 // which `fixed` bytes (staged twiddles, tables) plus L * (two line buffers + `per_line` other bytes) fit in `budget`
 // bytes; 0 when not even one line fits.  Every shared-memory line-FFT kernel sizes its lines here.

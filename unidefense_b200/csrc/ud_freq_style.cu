@@ -10,7 +10,8 @@
 //   rows^-1 : Hermitian extension (c2r semantics: imaginary parts of the DC / Nyquist columns are ignored),
 //          two output rows per complex line, inverse row FFT, 1/(H*W) scaling, coalesced stores.
 #include "../../include/unidefense_b200.h"
-#include "ud_fft.cuh"
+#include <type_traits>
+
 #include "ud_fft_any.cuh"
 
 #define FS_ROW_T 256
@@ -72,7 +73,7 @@ fs_rows_fwd_kernel(Plan plan, const float* __restrict__ a, const float* __restri
   }
 }
 
-// K column pairs per CTA (FS_COL_K for every static plan): Plan16 transforms all 2K lines (forward), Plan8 the first K
+// K column pairs per CTA (FS_COL_K for every configured length): Plan16 transforms all 2K lines (forward), Plan8 the first K
 // lines (inverse of the mix).
 template <class Plan16, class Plan8, int K>
 __global__ void __launch_bounds__(FS_COL_T)
@@ -187,60 +188,33 @@ fs_rows_inv_kernel(Plan plan, const float2* __restrict__ T, float* __restrict__ 
   }
 }
 
-static bool fs_static(int n) { return n == 380 || n == 256 || n == 224 || n == 299; }
-static int fs_line_len(int n) {
-  if (fs_static(n)) return n;
-  UdAnyPlan p;
-  return ud_make_any_plan(n, &p) ? p.m : 0;
-}
 static size_t fs_smem(int n, int m, int L) {
-  return sizeof(float2) * ((size_t)m + (fs_static(n) ? 1 : 2) * (size_t)L * (m | 1));
+  return sizeof(float2) * ((size_t)m + (ud_fft_configured(n) ? 1 : 2) * (size_t)L * (m | 1));
 }
 // Lines per CTA of the rows kernels (FS_ROW_L, /2 or /4) and column pairs per CTA of the cols kernel (FS_COL_K, /2 or
-// /4): the most whose two line buffers fit in shared memory, 0 when none does.  The in-place static plans always fit.
+// /4): the most whose two line buffers fit in shared memory, 0 when none does.  The in-place plans of the configured
+// lengths always fit.
 static int fs_row_lines(int W) {
-  if (fs_static(W)) return FS_ROW_L;
+  if (ud_fft_configured(W)) return FS_ROW_L;
   const int m = ud_any_line_len(W);
   return ud_halving_lines(ud_any_lines(m, sizeof(float2) * (size_t)m, 0, UD_SMEM_CTA_MAX, FS_ROW_L), FS_ROW_L);
 }
 static int fs_col_k(int H) {
-  if (fs_static(H)) return FS_COL_K;
+  if (ud_fft_configured(H)) return FS_COL_K;
   const int m = ud_any_line_len(H);
   return ud_halving_lines(ud_any_lines(m, sizeof(float2) * (size_t)m, 0, UD_SMEM_CTA_MAX, FS_COL_L), FS_COL_L) / 2;
 }
 
-template <class K>
-static int fs_set_smem(K kernel, size_t bytes) {
-  if (bytes > (227u << 10)) {
-    ud_set_error("freq_style: needs %zu bytes of shared memory per CTA (> 227 KB)", bytes);
-    return UD_ERR_UNSUPPORTED;
-  }
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e != cudaSuccess) {
-    ud_set_error("cudaFuncSetAttribute(smem=%zu) failed: %s", bytes, cudaGetErrorString(e));
-    return UD_ERR_CUDA;
-  }
-  return UD_OK;
+// Runs launch(plan, lines) with W's row plan and lines per CTA (a std::integral_constant): the configured length's
+// in-place plan at FS_ROW_L lines, or the run-time plan at LR lines (FS_ROW_L, /2 or /4).
+template <class F>
+static int fs_rows_run(int W, int LR, F launch) {
+  UD_FFT_CONFIGURED(W, CFG, {
+      UdAnyPlan p;
+      if (!ud_make_any_plan(W, &p)) return UD_ERR_UNSUPPORTED;
+      UD_LINES_DISPATCH(LR, FS_ROW_L, LV, return launch(p, std::integral_constant<int, LV>()));
+    }, return launch(CFG::IP<FS_ROW_L, FS_ROW_T>(), std::integral_constant<int, FS_ROW_L>()));
 }
-
-// Both run the body with the plan(s) of n and `constexpr int LV` lines per CTA: L for the static plans, Lany (one of L,
-// L/2, L/4) for the run-time plan.
-#define FS_PLAN1(n, L, Lany, THREADS, P, LV, ...)                                                                      \
-  do {                                                                                                                 \
-    if ((n) == 380) { UdStaticPlanIP<380, L, THREADS, 19, 5, 4> P; constexpr int LV = L; __VA_ARGS__; }                \
-    else if ((n) == 256) { UdStaticPlanIP<256, L, THREADS, 4, 4, 4, 4> P; constexpr int LV = L; __VA_ARGS__; }         \
-    else if ((n) == 224) { UdStaticPlanIP<224, L, THREADS, 7, 4, 4, 2> P; constexpr int LV = L; __VA_ARGS__; }         \
-    else if ((n) == 299) { UdStaticPlanIP<299, L, THREADS, 23, 13> P; constexpr int LV = L; __VA_ARGS__; }             \
-    else { UdAnyPlan P; if (!ud_make_any_plan((n), &P)) return UD_ERR_UNSUPPORTED; UD_LINES_DISPATCH(Lany, L, LV, __VA_ARGS__); } \
-  } while (0)
-#define FS_PLAN2(n, Kany, P16, P8, KV, ...)                                                                                \
-  do {                                                                                                                     \
-    if ((n) == 380) { UdStaticPlanIP<380, FS_COL_L, FS_COL_T, 19, 5, 4> P16; UdStaticPlanIP<380, FS_COL_K, FS_COL_T, 19, 5, 4> P8; constexpr int KV = FS_COL_K; __VA_ARGS__; } \
-    else if ((n) == 256) { UdStaticPlanIP<256, FS_COL_L, FS_COL_T, 4, 4, 4, 4> P16; UdStaticPlanIP<256, FS_COL_K, FS_COL_T, 4, 4, 4, 4> P8; constexpr int KV = FS_COL_K; __VA_ARGS__; } \
-    else if ((n) == 224) { UdStaticPlanIP<224, FS_COL_L, FS_COL_T, 7, 4, 4, 2> P16; UdStaticPlanIP<224, FS_COL_K, FS_COL_T, 7, 4, 4, 2> P8; constexpr int KV = FS_COL_K; __VA_ARGS__; } \
-    else if ((n) == 299) { UdStaticPlanIP<299, FS_COL_L, FS_COL_T, 23, 13> P16; UdStaticPlanIP<299, FS_COL_K, FS_COL_T, 23, 13> P8; constexpr int KV = FS_COL_K; __VA_ARGS__; } \
-    else { UdAnyPlan P16; if (!ud_make_any_plan((n), &P16)) return UD_ERR_UNSUPPORTED; UdAnyPlan P8 = P16; UD_LINES_DISPATCH(Kany, FS_COL_K, KV, __VA_ARGS__); }  \
-  } while (0)
 
 static int fs_chunk(int N, int C, int H, int W) {
   const size_t per = 2ull * C * H * fs_whp(W) * sizeof(float2);
@@ -270,8 +244,7 @@ extern "C" int ud_freq_style_transfer(const float* content, const float* style, 
   const int Wh = W / 2 + 1;
   float2* Ya = reinterpret_cast<float2*>(ws);
   float2* Yb = Ya + (size_t)chunk * C * H * fs_whp(W);
-  const int mW = fs_line_len(W), mH = fs_line_len(H);
-  if (!mW || !mH) return UD_ERR_UNSUPPORTED;
+  const int mW = ud_any_line_len(W), mH = ud_any_line_len(H);
   const float2* twW = ud_twiddles(mW);
   const float2* twH = ud_twiddles(mH);
   if (!twW || !twH) return UD_ERR_CUDA;
@@ -281,24 +254,35 @@ extern "C" int ud_freq_style_transfer(const float* content, const float* style, 
   for (int s0 = 0; s0 < N; s0 += chunk) {
     const int ns = (N - s0 < chunk) ? (N - s0) : chunk;
     const int planes = ns * C, plane0 = s0 * C;
-    FS_PLAN1(W, FS_ROW_L, LR, FS_ROW_T, plan, LV, {
-      auto k = fs_rows_fwd_kernel<decltype(plan), LV>;
-      if ((rc = fs_set_smem(k, smR)) != UD_OK) return rc;
-      k<<<dim3(ud_cdiv(H, LV), planes), FS_ROW_T, smR, stream>>>(plan, content, style, Ya, Yb, twW, plane0, H, W);
+    rc = fs_rows_run(W, LR, [&](auto plan, auto lines) {
+      auto k = fs_rows_fwd_kernel<decltype(plan), decltype(lines)::value>;
+      const int e = ud_set_smem(k, smR, "freq_style");
+      if (e == UD_OK)
+        k<<<dim3(ud_cdiv(H, lines), planes), FS_ROW_T, smR, stream>>>(plan, content, style, Ya, Yb, twW, plane0, H, W);
+      return e;
     });
-    if ((rc = ud_check_launch("fs_rows_fwd")) != UD_OK) return rc;
-    FS_PLAN2(H, KC, p16, p8, KV, {
-      auto k = fs_cols_kernel<decltype(p16), decltype(p8), KV>;
-      if ((rc = fs_set_smem(k, smC)) != UD_OK) return rc;
-      k<<<dim3(ud_cdiv(Wh, KV), planes), FS_COL_T, smC, stream>>>(p16, p8, Ya, Yb, lmda, twH, plane0, C, H, W);
+    if (rc != UD_OK || (rc = ud_check_launch("fs_rows_fwd")) != UD_OK) return rc;
+    auto cols = [&](auto p16, auto p8, auto kc) {
+      auto k = fs_cols_kernel<decltype(p16), decltype(p8), decltype(kc)::value>;
+      const int e = ud_set_smem(k, smC, "freq_style");
+      if (e == UD_OK)
+        k<<<dim3(ud_cdiv(Wh, kc), planes), FS_COL_T, smC, stream>>>(p16, p8, Ya, Yb, lmda, twH, plane0, C, H, W);
+      return e;
+    };
+    UD_FFT_CONFIGURED(H, CFG, {
+        UdAnyPlan p;
+        if (!ud_make_any_plan(H, &p)) return UD_ERR_UNSUPPORTED;
+        UD_LINES_DISPATCH(KC, FS_COL_K, KV, rc = cols(p, p, std::integral_constant<int, KV>()));
+      }, rc = cols(CFG::IP<FS_COL_L, FS_COL_T>(), CFG::IP<FS_COL_K, FS_COL_T>(), std::integral_constant<int, FS_COL_K>()));
+    if (rc != UD_OK || (rc = ud_check_launch("fs_cols")) != UD_OK) return rc;
+    rc = fs_rows_run(W, LR, [&](auto plan, auto lines) {
+      auto k = fs_rows_inv_kernel<decltype(plan), decltype(lines)::value>;
+      const int e = ud_set_smem(k, smR, "freq_style");
+      if (e == UD_OK)
+        k<<<dim3(ud_cdiv(H, 2 * lines), planes), FS_ROW_T, smR, stream>>>(plan, Ya, out, twW, plane0, H, W, scale);
+      return e;
     });
-    if ((rc = ud_check_launch("fs_cols")) != UD_OK) return rc;
-    FS_PLAN1(W, FS_ROW_L, LR, FS_ROW_T, plan, LV, {
-      auto k = fs_rows_inv_kernel<decltype(plan), LV>;
-      if ((rc = fs_set_smem(k, smR)) != UD_OK) return rc;
-      k<<<dim3(ud_cdiv(H, 2 * LV), planes), FS_ROW_T, smR, stream>>>(plan, Ya, out, twW, plane0, H, W, scale);
-    });
-    if ((rc = ud_check_launch("fs_rows_inv")) != UD_OK) return rc;
+    if (rc != UD_OK || (rc = ud_check_launch("fs_rows_inv")) != UD_OK) return rc;
   }
   return UD_OK;
 }

@@ -47,22 +47,15 @@ int ud_rt2_bwd(const float* dec, const float* x, const uint8_t* signs, const flo
 
 static inline int rt_whp(int W) { return ((W / 2 + 1) + 15) & ~15; }  // padded half width (float2)
 
-__device__ __forceinline__ void rt_tab(const float2 t, int in_size, int& i0, int& i1, float& l0, float& l1) {
-  i0 = __float_as_int(t.x);
-  i1 = i0 + ((i0 < in_size - 1) ? 1 : 0);
-  l1 = t.y;
-  l0 = 1.f - l1;
-}
-
 // Vertical lerp of the two image rows (ra, ra+1) of a pair into vA/vB [w] (shared memory).
 __device__ __forceinline__ void rt_vrows(const float* __restrict__ decp, const float2* __restrict__ ytab_g, int ra, int h,
                                          int w, int H, float* __restrict__ vA, float* __restrict__ vB) {
   if (ra >= H) return;
   int a0, a1, b0, b1;
   float la0, la1, lb0, lb1;
-  rt_tab(__ldg(ytab_g + ra), h, a0, a1, la0, la1);
+  ud_lerp_tab(__ldg(ytab_g + ra), h, a0, a1, la0, la1);
   const bool has_b = ra + 1 < H;
-  rt_tab(__ldg(ytab_g + (has_b ? ra + 1 : ra)), h, b0, b1, lb0, lb1);
+  ud_lerp_tab(__ldg(ytab_g + (has_b ? ra + 1 : ra)), h, b0, b1, lb0, lb1);
   const float* pa0 = decp + (long long)a0 * w;
   const float* pa1 = decp + (long long)a1 * w;
   const float* pb0 = decp + (long long)b0 * w;
@@ -75,23 +68,23 @@ __device__ __forceinline__ void rt_vrows(const float* __restrict__ decp, const f
 
 // ------------------------------------------------------------------------------------------
 // forward rows: grid (row_tiles, planes_in_chunk)
-//   shared: tw[n] | xtab[n] | buf0[L*LS] (| buf1[L*LS] when the plan ping-pongs) | vbuf[2][2][w]
+//   shared: tw[m] | xtab[n] | buf0[L*LS] | buf1[L*LS] | vbuf[2][2][w]
 // ------------------------------------------------------------------------------------------
-template <class Plan, int L>
+template <int L>
 __global__ void __launch_bounds__(RT_ROW_T)
-rt_rows_fwd_kernel(Plan plan, const float* __restrict__ dec, const float* __restrict__ x,
+rt_rows_fwd_kernel(UdAnyPlan plan, const float* __restrict__ dec, const float* __restrict__ x,
                    float* __restrict__ rec, float2* __restrict__ Y, float* __restrict__ part_spatial,
                    const float2* __restrict__ tw_g, const float2* __restrict__ ytab_g,
                    const float2* __restrict__ xtab_g, int plane0, int h, int w, int H, int W, int row_tiles) {
   static_assert(L % RT_VGRP == 0, "row pairs are staged in groups of RT_VGRP");
   extern __shared__ float2 smem[];
-  const int n = plan.n();  // == W
+  const int n = plan.n();
   const int m = plan.line_len();     // == n except for Bluestein plans
   const int LS = m | 1;
   float2* tw = smem;
   float2* xtab = tw + m;
   float2* buf0 = xtab + n;
-  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + L * LS;
+  float2* buf1 = buf0 + L * LS;
   float* vbuf = reinterpret_cast<float*>(buf1 + L * LS);
   __shared__ float red[33];
 
@@ -99,7 +92,7 @@ rt_rows_fwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
   const int pl = blockIdx.y;             // plane within chunk
   const long long plane = plane0 + pl;   // global (n*C + c)
   const int r0 = tile * (2 * L);
-  W = n;                                 // W == n: lets static plans constant-fold every index below
+  W = n;
   const int Wh = n / 2 + 1;
   const int WhP = (Wh + 15) & ~15;
 
@@ -148,7 +141,7 @@ rt_rows_fwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
         for (int c = threadIdx.x; c < W; c += RT_ROW_T) {
           int i0, i1;
           float l0, l1;
-          rt_tab(xtab[c], w, i0, i1, l0, l1);
+          ud_lerp_tab(xtab[c], w, i0, i1, l0, l1);
           const float2 xv = line[c];
           const float va = l0 * vA[i0] + l1 * vA[i1];
           __stcs(ra_p + c, va);
@@ -186,24 +179,24 @@ rt_rows_fwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
 // ------------------------------------------------------------------------------------------
 // forward cols: grid (col_tiles, planes_in_chunk).  Column FFT length n = H.
 // ------------------------------------------------------------------------------------------
-template <class Plan, int L>
+template <int L>
 __global__ void __launch_bounds__(RT_COL_T)
-rt_cols_fwd_kernel(Plan plan, const float2* __restrict__ Y, float* __restrict__ part_freq,
+rt_cols_fwd_kernel(UdAnyPlan plan, const float2* __restrict__ Y, float* __restrict__ part_freq,
                    uint8_t* __restrict__ signs, const float2* __restrict__ tw_g, int plane0, int H, int W,
                    int col_tiles) {
   extern __shared__ float2 smem[];
-  const int n = plan.n();  // == H
+  const int n = plan.n();
   const int m = plan.line_len();     // == n except for Bluestein plans
   const int LS = m | 1;
   float2* tw = smem;
   float2* buf0 = tw + m;
-  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + L * LS;
+  float2* buf1 = buf0 + L * LS;
   __shared__ float red[33];
 
   const int tile = blockIdx.x;
   const int pl = blockIdx.y;
   const long long plane = plane0 + pl;
-  H = n;                                 // H == n: constant-folds the index math for static plans
+  H = n;
   const int Wh = W / 2 + 1;
   const int WhP = (Wh + 15) & ~15;
   const int k0 = tile * L;
@@ -259,9 +252,9 @@ __global__ void rt_finalize_kernel(const float* __restrict__ part_spatial, const
 // T[r,k] = sum_j S[j,k] e^{+2 pi i j r / H},  S = gf * (sgn Re D + i sgn Im D)
 // inverse via the swap trick: IFFT(z) = swap(FFT(swap(z))).
 // ------------------------------------------------------------------------------------------
-template <class Plan, int L>
+template <int L>
 __global__ void __launch_bounds__(RT_COL_T)
-rt_cols_bwd_kernel(Plan plan, const uint8_t* __restrict__ signs, const float* __restrict__ g_freq,
+rt_cols_bwd_kernel(UdAnyPlan plan, const uint8_t* __restrict__ signs, const float* __restrict__ g_freq,
                    float2* __restrict__ T, const float2* __restrict__ tw_g, int plane0, int C, int H, int W,
                    float gscale) {
   extern __shared__ float2 smem[];
@@ -270,7 +263,7 @@ rt_cols_bwd_kernel(Plan plan, const uint8_t* __restrict__ signs, const float* __
   const int LS = m | 1;
   float2* tw = smem;
   float2* buf0 = tw + m;
-  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + L * LS;
+  float2* buf1 = buf0 + L * LS;
 
   const int tile = blockIdx.x;
   const int pl = blockIdx.y;
@@ -313,7 +306,7 @@ rt_cols_bwd_kernel(Plan plan, const uint8_t* __restrict__ signs, const float* __
 // g_rec[r,c] = gs*sign(d[r,c]) + Re sum_{k<Wh} T[r,k] e^{+2 pi i k c / W}; then the transposed
 // bilinear resize accumulates into g_dec (pre-zeroed).  Two rows are packed per complex line by
 // folding T into its Hermitian part Th (Re IFFT(T) == IFFT(Th)) and transforming Th_a + i Th_b.
-//   shared: tw[n] | xtab[n] | buf0[L*LS] (| buf1) | vbuf[2][2][w]
+//   shared: tw[m] | xtab[n] | buf0[L*LS] | buf1[L*LS] | vbuf[2][2][w]
 // After the FFT a line holds (g_b[c], g_a[c]) per column.  The transposed resize runs horizontally
 // first (gather through xtab, both rows of a pair at once, results staged in registers and written back
 // over the line), then vertically: one thread per dec column walks the tile's rows in order carrying two
@@ -321,9 +314,9 @@ rt_cols_bwd_kernel(Plan plan, const uint8_t* __restrict__ signs, const float* __
 // GX: also g_x = -g_rec at full resolution from the finished lines (zeros for planes whose sample has gs == gf == 0);
 // g_dec may then be NULL.  GX = false is the training path.
 // ------------------------------------------------------------------------------------------
-template <class Plan, bool GX, int L>
+template <bool GX, int L>
 __global__ void __launch_bounds__(RT_ROW_T)
-rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __restrict__ x,
+rt_rows_bwd_kernel(UdAnyPlan plan, const float* __restrict__ dec, const float* __restrict__ x,
                    const float2* __restrict__ T, const float* __restrict__ g_spatial,
                    const float* __restrict__ g_freq, float* __restrict__ g_dec, float* __restrict__ g_x,
                    const float2* __restrict__ tw_g, const float2* __restrict__ ytab_g,
@@ -331,13 +324,13 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
                    int w, int H, int W, float sp_scale) {
   static_assert(L % RT_VGRP == 0, "row pairs are staged in groups of RT_VGRP");
   extern __shared__ float2 smem[];
-  const int n = plan.n();  // == W
+  const int n = plan.n();
   const int m = plan.line_len();     // == n except for Bluestein plans
   const int LS = m | 1;
   float2* tw = smem;
   float2* xtab = tw + m;
   float2* buf0 = xtab + n;
-  float2* buf1 = Plan::kInPlace ? buf0 : buf0 + L * LS;
+  float2* buf1 = buf0 + L * LS;
   float* vbuf = reinterpret_cast<float*>(buf1 + L * LS);
 
   const int tile = blockIdx.x;
@@ -403,7 +396,7 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
           if (live) {
             int i0, i1;
             float l0, l1;
-            rt_tab(xtab[c], w, i0, i1, l0, l1);
+            ud_lerp_tab(xtab[c], w, i0, i1, l0, l1);
             const float2 xv = line[c];
             const float dA = (l0 * vA[i0] + l1 * vA[i1]) - xv.x;
             code = dA > 0.f ? 1 : (dA < 0.f ? 2 : 0);
@@ -514,7 +507,7 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
       for (int rr = 0; rr < nrows; ++rr) {
         int i0, i1;
         float l0, l1;
-        rt_tab(__ldg(ytab_g + r0 + rr), h, i0, i1, l0, l1);
+        ud_lerp_tab(__ldg(ytab_g + r0 + rr), h, i0, i1, l0, l1);
         while (cur < i0) {
           if (acc0 != 0.f) atomicAdd(gd + (long long)cur * w + j, acc0);
           acc0 = acc1;
@@ -540,14 +533,14 @@ rt_rows_bwd_kernel(Plan plan, const float* __restrict__ dec, const float* __rest
       for (int c = cr.x; c <= cr.y; ++c) {
         int i0, i1;
         float l0, l1;
-        rt_tab(xtab[c], w, i0, i1, l0, l1);
+        ud_lerp_tab(xtab[c], w, i0, i1, l0, l1);
         const float wgt = ((i0 == j) ? l0 : 0.f) + ((i1 == j) ? l1 : 0.f);
         const float2 g = line[c];
         a = fmaf(wgt, (rr & 1) ? g.x : g.y, a);
       }
       int i0, i1;
       float l0, l1;
-      rt_tab(__ldg(ytab_g + r0 + rr), h, i0, i1, l0, l1);
+      ud_lerp_tab(__ldg(ytab_g + r0 + rr), h, i0, i1, l0, l1);
       if (a != 0.f) {
         atomicAdd(gd + (long long)i0 * w + j, l0 * a);
         if (l1 != 0.f) atomicAdd(gd + (long long)i1 * w + j, l1 * a);
@@ -617,20 +610,6 @@ extern "C" size_t ud_recon_tail_signs_bytes(int N, int C, int H, int W) {
   return (size_t)N * C * (W / 2 + 1) * H;
 }
 
-template <class K>
-static int rt_set_smem(K kernel, size_t bytes) {
-  if (bytes > (227u << 10)) {
-    ud_set_error("recon_tail: needs %zu bytes of shared memory per CTA (> 227 KB)", bytes);
-    return UD_ERR_UNSUPPORTED;
-  }
-  cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  if (e != cudaSuccess) {
-    ud_set_error("cudaFuncSetAttribute(smem=%zu) failed: %s", bytes, cudaGetErrorString(e));
-    return UD_ERR_CUDA;
-  }
-  return UD_OK;
-}
-
 static int rt_validate(int N, int C, int h, int w, int H, int W) {
   UD_REQUIRE(N >= 0 && C >= 1 && h >= 1 && w >= 1 && H >= 1 && W >= 1, UD_ERR_INVALID,
              "recon_tail: bad shape N=%d C=%d h=%d w=%d H=%d W=%d", N, C, h, w, H, W);
@@ -640,6 +619,36 @@ static int rt_validate(int N, int C, int h, int w, int H, int W) {
   UD_REQUIRE(rt_row_lines(W, w) > 0, UD_ERR_UNSUPPORTED,
              "recon_tail: %d-point rows with a %d-wide decoder do not fit shared memory", W, w);
   UD_REQUIRE(rt_col_lines(H) > 0, UD_ERR_UNSUPPORTED, "recon_tail: %d-point columns do not fit shared memory", H);
+  return UD_OK;
+}
+
+// Chunking, tiling, plans and resize tables of a call, shared by the forward and the backward
+struct RtSetup {
+  int chunk;                  // samples per pass over the Y/T workspace
+  bool v2;                    // second-generation kernels (ud_recon_tail2.cu)
+  int LR, LC;                 // row pairs / columns per CTA of the first-generation kernels
+  int row_tiles, col_tiles;
+  UdAnyPlan pW, pH;           // line FFTs of the first-generation kernels: mixed radix, or Bluestein for a prime factor > 23
+  const float2* ytab;
+  const float2* xtab;
+  size_t smW, smH;            // dynamic shared memory of the first-generation rows / cols kernels
+};
+
+static int rt_setup(int N, int C, int h, int w, int H, int W, RtSetup& s) {
+  s.chunk = rt_chunk_samples(N, C, H, W);
+  if (s.chunk * C > 65535) s.chunk = 65535 / C;
+  const int Wh = W / 2 + 1;
+  s.v2 = ud_rt2_supported(h, w, H, W);
+  s.LR = rt_row_lines(W, w);
+  s.LC = rt_col_lines(H);
+  s.row_tiles = s.v2 ? ud_cdiv((H + 1) / 2, ud_rt2_rows_lpc()) : ud_cdiv(H, 2 * s.LR);
+  s.col_tiles = s.v2 ? ud_cdiv(Wh, RT2_COLS_PER_TILE) : ud_cdiv(Wh, s.LC);
+  if (!ud_make_any_plan(W, &s.pW) || !ud_make_any_plan(H, &s.pH)) return UD_ERR_UNSUPPORTED;
+  s.ytab = ud_lerp_table(h, H);
+  s.xtab = ud_lerp_table(w, W);
+  if (!s.ytab || !s.xtab) return UD_ERR_CUDA;
+  s.smW = rt_rows_smem(W, s.pW.m, w, s.LR);
+  s.smH = rt_cols_smem(s.pH.m, s.LC);
   return UD_OK;
 }
 
@@ -653,50 +662,41 @@ extern "C" int ud_recon_tail_fwd(const float* dec, const float* x, float* rec, f
   UD_REQUIRE(ws_bytes >= ud_recon_tail_workspace_bytes(N, C, h, w, H, W), UD_ERR_WORKSPACE,
              "recon_tail_fwd: workspace too small (%zu < %zu)", ws_bytes,
              ud_recon_tail_workspace_bytes(N, C, h, w, H, W));
-  int chunk = rt_chunk_samples(N, C, H, W);
-  if (chunk * C > 65535) chunk = 65535 / C;
+  RtSetup s;
+  if ((rc = rt_setup(N, C, h, w, H, W, s)) != UD_OK) return rc;
   const int Wh = W / 2 + 1;
-  const bool v2 = ud_rt2_supported(h, w, H, W);
-  const int LR = rt_row_lines(W, w), LC = rt_col_lines(H);
-  const int row_tiles = v2 ? ud_cdiv((H + 1) / 2, ud_rt2_rows_lpc()) : ud_cdiv(H, 2 * LR);
-  const int col_tiles = v2 ? ud_cdiv(Wh, RT2_COLS_PER_TILE) : ud_cdiv(Wh, LC);
   char* p = static_cast<char*>(ws);
   float2* Y = reinterpret_cast<float2*>(p);
   p += ud_align_up((size_t)rt_chunk_samples(N, C, H, W) * C * rt_plane_bytes(H, W), 256);
   float* part_sp = reinterpret_cast<float*>(p);
-  p += ud_align_up((size_t)N * C * row_tiles * sizeof(float), 256);
+  p += ud_align_up((size_t)N * C * s.row_tiles * sizeof(float), 256);
   float* part_fr = reinterpret_cast<float*>(p);
-  UdAnyPlan pW, pH;   // line FFTs of the first-generation kernels: mixed radix, or Bluestein for a prime factor > 23
-  if (!ud_make_any_plan(W, &pW) || !ud_make_any_plan(H, &pH)) return UD_ERR_UNSUPPORTED;
-  const float2* ytab = ud_lerp_table(h, H);
-  const float2* xtab = ud_lerp_table(w, W);
-  if (!ytab || !xtab) return UD_ERR_CUDA;
-  const size_t smW = rt_rows_smem(W, pW.m, w, LR), smH = rt_cols_smem(pH.m, LC);
 
-  for (int s0 = 0; s0 < N; s0 += chunk) {
-    const int ns = (N - s0 < chunk) ? (N - s0) : chunk;
+  for (int s0 = 0; s0 < N; s0 += s.chunk) {
+    const int ns = (N - s0 < s.chunk) ? (N - s0) : s.chunk;
     const int planes = ns * C, plane0 = s0 * C;
-    if (v2) {
-      if ((rc = ud_rt2_fwd(dec, x, rec, Y, part_sp, part_fr, signs, plane0, planes, h, w, H, W, row_tiles, col_tiles,
-                           stream)) != UD_OK) return rc;
+    if (s.v2) {
+      if ((rc = ud_rt2_fwd(dec, x, rec, Y, part_sp, part_fr, signs, plane0, planes, h, w, H, W, s.row_tiles,
+                           s.col_tiles, stream)) != UD_OK) return rc;
       continue;
     }
-    UD_LINES_DISPATCH(LR, RT_ROW_L, LV, {
-      auto k = rt_rows_fwd_kernel<UdAnyPlan, LV>;
-      if ((rc = rt_set_smem(k, smW)) != UD_OK) return rc;
-      k<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(pW, dec, x, rec, Y, part_sp, pW.tw, ytab, xtab, plane0, h, w,
-                                                            H, W, row_tiles);
+    UD_LINES_DISPATCH(s.LR, RT_ROW_L, LV, {
+      auto k = rt_rows_fwd_kernel<LV>;
+      if ((rc = ud_set_smem(k, s.smW, "recon_tail")) != UD_OK) return rc;
+      k<<<dim3(s.row_tiles, planes), RT_ROW_T, s.smW, stream>>>(s.pW, dec, x, rec, Y, part_sp, s.pW.tw, s.ytab, s.xtab,
+                                                                plane0, h, w, H, W, s.row_tiles);
     });
     if ((rc = ud_check_launch("rt_rows_fwd")) != UD_OK) return rc;
-    UD_LINES_DISPATCH(LC, RT_COL_L, LV, {
-      auto k = rt_cols_fwd_kernel<UdAnyPlan, LV>;
-      if ((rc = rt_set_smem(k, smH)) != UD_OK) return rc;
-      k<<<dim3(col_tiles, planes), RT_COL_T, smH, stream>>>(pH, Y, part_fr, signs, pH.tw, plane0, H, W, col_tiles);
+    UD_LINES_DISPATCH(s.LC, RT_COL_L, LV, {
+      auto k = rt_cols_fwd_kernel<LV>;
+      if ((rc = ud_set_smem(k, s.smH, "recon_tail")) != UD_OK) return rc;
+      k<<<dim3(s.col_tiles, planes), RT_COL_T, s.smH, stream>>>(s.pH, Y, part_fr, signs, s.pH.tw, plane0, H, W,
+                                                                s.col_tiles);
     });
     if ((rc = ud_check_launch("rt_cols_fwd")) != UD_OK) return rc;
   }
   const float nrm = norm_ortho ? 1.f / sqrtf((float)H * (float)W) : 1.f;
-  rt_finalize_kernel<<<N, 128, 0, stream>>>(part_sp, part_fr, spatial, freq, C, row_tiles, col_tiles,
+  rt_finalize_kernel<<<N, 128, 0, stream>>>(part_sp, part_fr, spatial, freq, C, s.row_tiles, s.col_tiles,
                                             1.f / ((float)C * H * W), nrm / ((float)C * H * Wh));
   return ud_check_launch("rt_finalize");
 }
@@ -712,47 +712,37 @@ extern "C" int ud_recon_tail_bwd(const float* dec, const float* x, const uint8_t
              "recon_tail_bwd: null pointer");
   UD_REQUIRE(ws_bytes >= ud_recon_tail_workspace_bytes(N, C, h, w, H, W), UD_ERR_WORKSPACE,
              "recon_tail_bwd: workspace too small");
-  int chunk = rt_chunk_samples(N, C, H, W);
-  if (chunk * C > 65535) chunk = 65535 / C;
+  RtSetup s;
+  if ((rc = rt_setup(N, C, h, w, H, W, s)) != UD_OK) return rc;
   const int Wh = W / 2 + 1;
-  const bool v2 = ud_rt2_supported(h, w, H, W);
-  const int LR = rt_row_lines(W, w), LC = rt_col_lines(H);
-  const int row_tiles = v2 ? ud_cdiv((H + 1) / 2, ud_rt2_rows_lpc()) : ud_cdiv(H, 2 * LR);
-  const int col_tiles = v2 ? ud_cdiv(Wh, RT2_COLS_PER_TILE) : ud_cdiv(Wh, LC);
   float2* T = reinterpret_cast<float2*>(ws);
-  UdAnyPlan pW, pH;   // line FFTs of the first-generation kernels: mixed radix, or Bluestein for a prime factor > 23
-  if (!ud_make_any_plan(W, &pW) || !ud_make_any_plan(H, &pH)) return UD_ERR_UNSUPPORTED;
-  const float2* ytab = ud_lerp_table(h, H);
-  const float2* xtab = ud_lerp_table(w, W);
-  if (!ytab || !xtab) return UD_ERR_CUDA;
   const int2* jtab = ud_lerp_ranges(w, W);
   if (!jtab) return UD_ERR_CUDA;
-  const size_t smH = rt_cols_smem(pH.m, LC), smW = rt_rows_smem(W, pW.m, w, LR);
   // freq[n] = nrm/(C*H*Wh) * sum |D'| with D' the unnormalised spectrum, so the sign spectrum
   // carries nrm/(C*H*Wh) and the adjoint of the unnormalised forward is the unnormalised inverse.
   const float nrm = norm_ortho ? 1.f / sqrtf((float)H * (float)W) : 1.f;
   const float gscale = nrm / ((float)C * H * Wh);
   const float sp_scale = 1.f / ((float)C * H * W);
   if (g_dec) UD_CUDA(cudaMemsetAsync(g_dec, 0, sizeof(float) * (size_t)N * C * h * w, stream));
-  for (int s0 = 0; s0 < N; s0 += chunk) {
-    const int ns = (N - s0 < chunk) ? (N - s0) : chunk;
+  for (int s0 = 0; s0 < N; s0 += s.chunk) {
+    const int ns = (N - s0 < s.chunk) ? (N - s0) : s.chunk;
     const int planes = ns * C, plane0 = s0 * C;
-    if (v2) {
-      if ((rc = ud_rt2_bwd(dec, x, signs, g_spatial, g_freq, g_dec, g_x, T, plane0, planes, C, h, w, H, W, row_tiles, col_tiles,
-                           gscale, sp_scale, stream)) != UD_OK) return rc;
+    if (s.v2) {
+      if ((rc = ud_rt2_bwd(dec, x, signs, g_spatial, g_freq, g_dec, g_x, T, plane0, planes, C, h, w, H, W, s.row_tiles,
+                           s.col_tiles, gscale, sp_scale, stream)) != UD_OK) return rc;
       continue;
     }
-    UD_LINES_DISPATCH(LC, RT_COL_L, LV, {
-      auto k = rt_cols_bwd_kernel<UdAnyPlan, LV>;
-      if ((rc = rt_set_smem(k, smH)) != UD_OK) return rc;
-      k<<<dim3(col_tiles, planes), RT_COL_T, smH, stream>>>(pH, signs, g_freq, T, pH.tw, plane0, C, H, W, gscale);
+    UD_LINES_DISPATCH(s.LC, RT_COL_L, LV, {
+      auto k = rt_cols_bwd_kernel<LV>;
+      if ((rc = ud_set_smem(k, s.smH, "recon_tail")) != UD_OK) return rc;
+      k<<<dim3(s.col_tiles, planes), RT_COL_T, s.smH, stream>>>(s.pH, signs, g_freq, T, s.pH.tw, plane0, C, H, W, gscale);
     });
     if ((rc = ud_check_launch("rt_cols_bwd")) != UD_OK) return rc;
-    UD_LINES_DISPATCH(LR, RT_ROW_L, LV, {
-      auto k = g_x ? rt_rows_bwd_kernel<UdAnyPlan, true, LV> : rt_rows_bwd_kernel<UdAnyPlan, false, LV>;
-      if ((rc = rt_set_smem(k, smW)) != UD_OK) return rc;
-      k<<<dim3(row_tiles, planes), RT_ROW_T, smW, stream>>>(pW, dec, x, T, g_spatial, g_freq, g_dec, g_x, pW.tw, ytab,
-                                                             xtab, jtab, plane0, C, h, w, H, W, sp_scale);
+    UD_LINES_DISPATCH(s.LR, RT_ROW_L, LV, {
+      auto k = g_x ? rt_rows_bwd_kernel<true, LV> : rt_rows_bwd_kernel<false, LV>;
+      if ((rc = ud_set_smem(k, s.smW, "recon_tail")) != UD_OK) return rc;
+      k<<<dim3(s.row_tiles, planes), RT_ROW_T, s.smW, stream>>>(s.pW, dec, x, T, g_spatial, g_freq, g_dec, g_x, s.pW.tw,
+                                                                s.ytab, s.xtab, jtab, plane0, C, h, w, H, W, sp_scale);
     });
     if ((rc = ud_check_launch("rt_rows_bwd")) != UD_OK) return rc;
   }

@@ -2,7 +2,7 @@
 //                                                                     (SURVEY.md §8a row a1)
 // Same math, entry points and saved state as ud_recon_tail.cu (reference: model/unidefense.py:244-253, :423-433,
 // :618-628; backward = torch autograd of those lines), rebuilt around the register-resident two-stage line FFT of
-// ud_fft2s.cuh for H, W in {380, 256, 224, 299}:
+// ud_fft.cuh (Ud2S) for the configured lengths (UdConfigured):
 //   * a line (two packed image rows, or one spectrum column) is owned by 20 (16, 23) threads whose roles never
 //     change, so the butterflies carry no index arithmetic and the pixel work happens in the registers the
 //     radix-R1 butterfly consumes: x is read and rec written straight from/to global memory, 4 bytes per lane,
@@ -18,7 +18,6 @@
 // Sizes without a two-factor plan keep using the shared-memory Stockham kernels of ud_recon_tail.cu.
 #include "../../include/unidefense_b200.h"
 #include "ud_fft.cuh"
-#include "ud_fft2s.cuh"
 
 #define RT2_LPC 16    // columns per CTA step of the cols kernels (16 float2 = one 128-byte line per row)
 #ifndef RT2_RLPC
@@ -28,13 +27,6 @@
 #define RT2_RLPC 16
 #endif
 // row-pair steps per CTA of the rows kernels: a launch parameter (`iters`, derived from the row-tile count the caller chose)
-
-__device__ __forceinline__ void rt2_tab(const float2 t, int in_size, int& i0, int& i1, float& l0, float& l1) {
-  i0 = __float_as_int(t.x);
-  i1 = i0 + ((i0 < in_size - 1) ? 1 : 0);
-  l1 = t.y;
-  l0 = 1.f - l1;
-}
 
 // Vertical lerps of the row pair of line g (vertical first, like ud_recon_tail.cu): V[c] = (row 2p, row 2p+1) of the
 // upsampled image BEFORE the horizontal lerp.  The TL threads of the line stride over the dec columns; the row taps
@@ -48,9 +40,9 @@ __device__ __forceinline__ void rt2_vrows(const float* __restrict__ decp, const 
   }
   int a0, a1, b0, b1;
   float la0, la1, lb0, lb1;
-  rt2_tab(__ldg(ytab_g + ra), h, a0, a1, la0, la1);
+  ud_lerp_tab(__ldg(ytab_g + ra), h, a0, a1, la0, la1);
   const bool has_b = ra + 1 < H;
-  rt2_tab(__ldg(ytab_g + (has_b ? ra + 1 : ra)), h, b0, b1, lb0, lb1);
+  ud_lerp_tab(__ldg(ytab_g + (has_b ? ra + 1 : ra)), h, b0, b1, lb0, lb1);
   if (!has_b) lb0 = lb1 = 0.f;
   const float* pa0 = decp + (long long)a0 * w;
   const float* pa1 = decp + (long long)a1 * w;
@@ -109,7 +101,7 @@ rt2_rows_fwd_kernel(const float* __restrict__ dec, const float* __restrict__ x, 
         const int c = ln + R2 * n1;
         int i0, i1;
         float l0, l1;
-        rt2_tab(xtab[c], w, i0, i1, l0, l1);
+        ud_lerp_tab(xtab[c], w, i0, i1, l0, l1);
         const float2 v0 = Vg[i0], v1 = Vg[i1];
         const float va = l0 * v0.x + l1 * v1.x;
         __stcs(qa + c, va);
@@ -398,7 +390,7 @@ rt2_rows_bwd_kernel(const float* __restrict__ dec, const float* __restrict__ x, 
           const int c = ln + R1 * k2;
           int i0, i1;
           float l0, l1;
-          rt2_tab(xtab[c], w, i0, i1, l0, l1);
+          ud_lerp_tab(xtab[c], w, i0, i1, l0, l1);
           const float2 v0 = Vg[i0], v1 = Vg[i1];
           const float dA = (l0 * v0.x + l1 * v1.x) - __ldcs(xa + c);
           u[k2].y += dA > 0.f ? gs : (dA < 0.f ? -gs : 0.f);
@@ -451,7 +443,7 @@ rt2_rows_bwd_kernel(const float* __restrict__ dec, const float* __restrict__ x, 
       for (int rr = 0; rr < nrows; ++rr) {
         int i0, i1;
         float l0, l1;
-        rt2_tab(__ldg(ytab_g + r0 + rr), h, i0, i1, l0, l1);
+        ud_lerp_tab(__ldg(ytab_g + r0 + rr), h, i0, i1, l0, l1);
         while (cur < i0) {
           if (acc0 != 0.f) atomicAdd(gd + (long long)cur * w + tid, acc0);
           acc0 = acc1;
@@ -476,34 +468,18 @@ rt2_rows_bwd_kernel(const float* __restrict__ dec, const float* __restrict__ x, 
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-#define RT2_DISPATCH(n, PLV, ...)                                          \
-  do {                                                                     \
-    if ((n) == 380) { typedef Ud2S<380, 20, 19> PLV; __VA_ARGS__; }        \
-    else if ((n) == 256) { typedef Ud2S<256, 16, 16> PLV; __VA_ARGS__; }   \
-    else if ((n) == 224) { typedef Ud2S<224, 16, 14> PLV; __VA_ARGS__; }   \
-    else { typedef Ud2S<299, 13, 23> PLV; __VA_ARGS__; }                   \
-  } while (0)
-
 // steps of RT2_RLPC row pairs a rows CTA walks so that `row_tiles` CTAs cover the (H+1)/2 pairs of a plane
 int ud_rt2_rows_lpc(void) { return RT2_RLPC; }
 static int rt2_iters(int H, int row_tiles) { return ud_cdiv(ud_cdiv((H + 1) / 2, RT2_RLPC), row_tiles); }
 
-static bool rt2_size(int n) { return n == 380 || n == 256 || n == 224 || n == 299; }
-
-// decoder planes at most as wide as the widest thread block (the vertical walk uses one thread per dec column)
+// configured lengths only (ud_rt2_fwd / ud_rt2_bwd run only shapes accepted here), and decoder planes at most as wide as
+// the widest thread block (the vertical walk uses one thread per dec column)
 bool ud_rt2_supported(int h, int w, int H, int W) {
   (void)h;
-  if (!rt2_size(H) || !rt2_size(W)) return false;
+  if (!ud_fft_configured(H)) return false;
   int tl = 0;
-  RT2_DISPATCH(W, PLW, tl = PLW::TL);
+  UD_FFT_CONFIGURED(W, CFG, , tl = CFG::TwoStage::TL);
   return w <= tl * RT2_RLPC && w >= 1;
-}
-
-template <class K>
-static int rt2_set_smem(K kernel, size_t bytes) {
-  UD_REQUIRE(bytes <= (227u << 10), UD_ERR_UNSUPPORTED, "recon_tail: needs %zu bytes of shared memory per CTA", bytes);
-  UD_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
-  return UD_OK;
 }
 
 size_t ud_rt2_workspace_plane_bytes(int H, int W) {
@@ -520,18 +496,20 @@ int ud_rt2_fwd(const float* dec, const float* x, float* rec, float2* Z, float* p
   const float2* xtab = ud_lerp_table(w, W);
   if (!twW || !twH || !ytab || !xtab) return UD_ERR_CUDA;
   int rc;
-  RT2_DISPATCH(W, PLW, {
+  UD_FFT_CONFIGURED(W, CFG, return UD_ERR_UNSUPPORTED, {
+    using PLW = CFG::TwoStage;
     auto k = rt2_rows_fwd_kernel<PLW>;
     const size_t sm = sizeof(float2) * ((size_t)PLW::R1 * PLW::P + W + (size_t)RT2_RLPC * PLW::LS + (size_t)RT2_RLPC * w);
-    if ((rc = rt2_set_smem(k, sm)) != UD_OK) return rc;
+    if ((rc = ud_set_smem(k, sm, "recon_tail")) != UD_OK) return rc;
     k<<<dim3(row_tiles, planes), PLW::TL * RT2_RLPC, sm, stream>>>(dec, x, rec, Z, part_sp, twW, ytab, xtab, plane0, h, w, H,
                                                                     row_tiles, rt2_iters(H, row_tiles));
   });
   if ((rc = ud_check_launch("rt2_rows_fwd")) != UD_OK) return rc;
-  RT2_DISPATCH(H, PLH, {
+  UD_FFT_CONFIGURED(H, CFG, return UD_ERR_UNSUPPORTED, {
+    using PLH = CFG::TwoStage;
     auto k = rt2_cols_fwd_kernel<PLH>;
     const size_t sm = sizeof(float2) * ((size_t)PLH::R1 * PLH::P + 2ull * RT2_LPC * Rt2Cols<PLH>::SB);
-    if ((rc = rt2_set_smem(k, sm)) != UD_OK) return rc;
+    if ((rc = ud_set_smem(k, sm, "recon_tail")) != UD_OK) return rc;
     const int total = planes * col_tiles;
     const int grid = total < 2 * UD_NUM_SMS ? total : 2 * UD_NUM_SMS;
     k<<<grid, PLH::TL * RT2_LPC, sm, stream>>>(Z, part_fr, signs, twH, plane0, planes, W, col_tiles);
@@ -549,18 +527,20 @@ int ud_rt2_bwd(const float* dec, const float* x, const uint8_t* signs, const flo
   const int2* jtab = ud_lerp_ranges(w, W);
   if (!twW || !twH || !ytab || !xtab || !jtab) return UD_ERR_CUDA;
   int rc;
-  RT2_DISPATCH(H, PLH, {
+  UD_FFT_CONFIGURED(H, CFG, return UD_ERR_UNSUPPORTED, {
+    using PLH = CFG::TwoStage;
     auto k = rt2_cols_bwd_kernel<PLH>;
     const size_t a = (size_t)RT2_LPC * PLH::LS, b = (size_t)H * (RT2_LPC + 1);
     const size_t sm = sizeof(float2) * ((size_t)PLH::R1 * PLH::P + (a > b ? a : b));
-    if ((rc = rt2_set_smem(k, sm)) != UD_OK) return rc;
+    if ((rc = ud_set_smem(k, sm, "recon_tail")) != UD_OK) return rc;
     k<<<dim3(col_tiles, planes), PLH::TL * RT2_LPC, sm, stream>>>(signs, g_freq, T, twH, plane0, C, W, gscale);
   });
   if ((rc = ud_check_launch("rt2_cols_bwd")) != UD_OK) return rc;
-  RT2_DISPATCH(W, PLW, {
+  UD_FFT_CONFIGURED(W, CFG, return UD_ERR_UNSUPPORTED, {
+    using PLW = CFG::TwoStage;
     auto k = g_x ? rt2_rows_bwd_kernel<PLW, true> : rt2_rows_bwd_kernel<PLW, false>;
     const size_t sm = sizeof(float2) * ((size_t)PLW::R1 * PLW::P + W + (size_t)RT2_RLPC * PLW::LS + (size_t)RT2_RLPC * w);
-    if ((rc = rt2_set_smem(k, sm)) != UD_OK) return rc;
+    if ((rc = ud_set_smem(k, sm, "recon_tail")) != UD_OK) return rc;
     k<<<dim3(row_tiles, planes), PLW::TL * RT2_RLPC, sm, stream>>>(dec, x, T, g_spatial, g_freq, g_dec, g_x, twW, ytab,
                                                                     xtab, jtab, plane0, C, h, w, H, sp_scale,
                                                                     rt2_iters(H, row_tiles));
