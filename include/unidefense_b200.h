@@ -22,7 +22,8 @@
  *    whose transposed resize accumulates with float atomics.  The input-gradient outputs (g_x of ud_recon_tail_bwd,
  *    ud_attn_prep_bwd, ud_gaussian_blur5_bwd, ud_downscale_nearest_bwd; g_diff of ud_dyfi_mask_bwd) are gathers
  *    written once per element: bitwise reproducible.  ud_attack_step's per-sample norms are fixed-order too.
- *    ud_corrupt writes every output element once from a fixed-order computation: bitwise reproducible.
+ *    ud_corrupt, ud_attrib_step, ud_attrib_mask and ud_rank_desc write every output element once from a fixed-order
+ *    computation: bitwise reproducible.
  */
 #ifndef UNIDEFENSE_B200_H
 #define UNIDEFENSE_B200_H
@@ -44,7 +45,7 @@ typedef struct CUstream_st* cudaStream_t;
 #define UD_API
 #endif
 
-#define UD_B200_VERSION 103
+#define UD_B200_VERSION 104
 #define UD_FFT_MAX_N 1024
 
 #define UD_ACT_NONE 0
@@ -357,6 +358,42 @@ UD_API int ud_attack_step(const float* x0, float* x_adv, const float* g, const f
 UD_API size_t ud_corrupt_workspace_bytes(int kind, int N, int H, int W);
 UD_API int ud_corrupt(const float* x, float* y, const long long* ids, int N, int H, int W, int kind, float param,
                       unsigned long long seed, float lo, float hi, void* ws, size_t ws_bytes, cudaStream_t stream);
+
+/* ---- a21: attribution maps (Integrated Gradients, SmoothGrad) and deletion / insertion faithfulness ----------------
+ * Objective F(x) = log p(target | x): log_softmax(cls_out)[target] for two logits; for one logit z, logsigmoid(z) for
+ * target 1 and logsigmoid(-z) for target 0.  The target is the label when given, else the class predicted at x.
+ * Path point k = 0..S-1: p_k = b + alpha_k*(x - b) + sigma*eps_k, in fp32 in that order (subtract, multiply, add, add
+ * the noise term).  Both methods accumulate acc = sum_k w_k * grad F(p_k) in k order in fp32.
+ *  UD_ATTRIB_IG (steps m, S = m + 1): alpha_k = k/m, sigma = 0, trapezoid weights w_0 = w_m = 1/(2m), 1/m otherwise;
+ *    attr = (x - b) * acc; delta = sum(attr) - (F(x) - F(b)) per sample is the completeness error.
+ *  UD_ATTRIB_SMOOTHGRAD (S draws, noise s): b = 0, alpha_k = 1, sigma = s*(hi - lo), w_k = 1/S, attr = acc; no clamp.
+ *    eps_k of element e (index within the sample, C*H*W order) is normal (4q + i) of Philox4x32-10(ctr = (q = e >> 2,
+ *    id_lo, id_hi, k), key = (seed_lo, seed_hi ^ 0x534D5448)): normals 0, 1 by Box-Muller (as ud_corrupt's NOISE) from
+ *    words (a, b), normals 2, 3 from (c, d).  ids: int64 [N] (NULL: 0..N-1), so sample i gets the same noise at any
+ *    batch size.
+ *  map[n, h, w] = sum_c |attr[n, c, h, w]| (fp32, channel order).
+ * ud_attrib_step: one iteration's image-sized work.  x, g, acc, p, attr [N, C, H, W]; base the same or NULL (base_value
+ *   everywhere); map [N, H, W]; k: int on the device; alpha, w: [S] on the device; sigma: float, seed: uint64 on the
+ *   device (SmoothGrad only).  g == NULL (start): acc = 0, p = p_k.  Otherwise acc += w_k*g, then p = p_{k+1} for
+ *   k < S-1, or attr and map for k = S-1; k out of [0, S) does nothing.  k is read, never written: the caller advances
+ *   it, so one captured graph serves every step.  Launches: 1 (start) or 2.
+ * ud_rank_desc: rank[n, i] = position of pixel i of map plane n in the stable descending order (ties by ascending pixel
+ *   index, NaN after every number, -0 == +0): one radix sort per plane through ws of ud_rank_desc_workspace_bytes().
+ * ud_attrib_mask: the input of faithfulness curve point j = *jp (0..points; t: int [points+1] on the device, t_j =
+ *   floor(j*H*W/points)): deletion (insertion = 0) takes the baseline at every channel of the pixels of rank < t_j and x
+ *   elsewhere; insertion the reverse.  j out of [0, points] does nothing.  y must not alias x or base.
+ * Every output element is written once from a fixed-order computation: bitwise reproducible.  N <= 65535.        */
+#define UD_ATTRIB_IG 0
+#define UD_ATTRIB_SMOOTHGRAD 1
+UD_API int ud_attrib_step(const float* x, const float* base, float base_value, const float* g, float* acc, float* p,
+                          float* attr, float* map, const int* k, const float* alpha, const float* w, const float* sigma,
+                          const long long* ids, const unsigned long long* seed, int steps, int method, int N, int C,
+                          int H, int W, cudaStream_t stream);
+UD_API size_t ud_rank_desc_workspace_bytes(int N, int HW);
+UD_API int ud_rank_desc(const float* map, int* rank, int N, int HW, void* ws, size_t ws_bytes, cudaStream_t stream);
+UD_API int ud_attrib_mask(const float* x, const float* base, float base_value, const int* rank, const int* t,
+                          const int* j, int points, float* y, int insertion, int N, int C, int H, int W,
+                          cudaStream_t stream);
 
 /* ---- §8(e): the exchange step -- SyncBatchNorm statistics over NVLink peer memory ----------------------------------
  * Replaces the two per-layer collectives of torch.nn.SyncBatchNorm (engine/forgery_engine.py:142 converts all 99

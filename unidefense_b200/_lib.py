@@ -95,6 +95,10 @@ SIGNATURES = {
     "ud_attack_step": (c_i, [c_p] * 8 + [c_f, c_f, c_i, c_i, ctypes.c_longlong, c_p, c_sz, c_p]),
     "ud_corrupt_workspace_bytes": (c_sz, [c_i] * 4),
     "ud_corrupt": (c_i, [c_p] * 3 + [c_i] * 4 + [c_f, ctypes.c_ulonglong, c_f, c_f, c_p, c_sz, c_p]),
+    "ud_attrib_step": (c_i, [c_p, c_p, c_f] + [c_p] * 11 + [c_i] * 6 + [c_p]),
+    "ud_rank_desc_workspace_bytes": (c_sz, [c_i, c_i]),
+    "ud_rank_desc": (c_i, [c_p, c_p, c_i, c_i, c_p, c_sz, c_p]),
+    "ud_attrib_mask": (c_i, [c_p, c_p, c_f] + [c_p] * 3 + [c_i, c_p] + [c_i] * 5 + [c_p]),
 }
 
 

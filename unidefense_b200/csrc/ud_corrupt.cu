@@ -16,6 +16,7 @@
 
 #include "../../include/unidefense_b200.h"
 #include "ud_common.cuh"
+#include "ud_philox.cuh"
 
 #define CR_THREADS 256
 #define CR_BLOCK_TAG 0x424C4F43u   // "BLOC"
@@ -48,30 +49,6 @@ __device__ __forceinline__ void cr_id(const CrArgs& a, int n, unsigned& lo, unsi
   hi = (unsigned)(id >> 32);
 }
 
-// Philox4x32-10 (Salmon et al., SC'11), as Random123 defines it
-__device__ __forceinline__ uint4 cr_philox(uint4 c, unsigned k0, unsigned k1) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const unsigned hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
-    const unsigned hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
-    c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
-    k0 += 0x9E3779B9u;
-    k1 += 0xBB67AE85u;
-  }
-  return c;
-}
-
-// Box-Muller: u1 = (a + 0.5)*2^-32, u2 = b*2^-32.  ln(u1) goes through log1p(-(1 - u1)) in the upper half, where
-// 1 - u1 = (~a + 0.5)*2^-32 is exact in the integer and u1 itself would lose it to fp32 rounding.
-__device__ __forceinline__ float2 cr_box_muller(unsigned a, unsigned b) {
-  const float l = a < 0x80000000u ? logf(__fmul_rn(__fadd_rn((float)a, 0.5f), 0x1p-32f))
-                                  : log1pf(-__fmul_rn(__fadd_rn((float)(~a), 0.5f), 0x1p-32f));
-  const float r = sqrtf(-2.f * l);
-  float sn, cs;
-  sincospif(__fmul_rn((float)b, 0x1p-31f), &sn, &cs);
-  return make_float2(r * cs, r * sn);
-}
-
 // ---- pointwise kinds: one read and one write per element ------------------------------------------------------------
 #define CR_QUANT (-1)   // level round trip only (the first pass of block)
 
@@ -97,9 +74,9 @@ __device__ __forceinline__ void cr_pixel(const CrArgs& a, float prm, unsigned id
     const float Y = 0.299f * R + 0.587f * G + 0.114f * B;
     const float Cb = -0.168736f * R - 0.331264f * G + 0.5f * B;
     const float Cr = 0.5f * R - 0.418688f * G - 0.081312f * B;
-    const uint4 w = cr_philox(make_uint4((unsigned)pix, idl, idh, 0u), a.seed_lo, a.seed_hi ^ CR_NOISE_TAG);
-    const float2 z01 = cr_box_muller(w.x, w.y);
-    const float z2 = cr_box_muller(w.z, w.w).x;
+    const uint4 w = ud_philox(make_uint4((unsigned)pix, idl, idh, 0u), a.seed_lo, a.seed_hi ^ CR_NOISE_TAG);
+    const float2 z01 = ud_box_muller(w.x, w.y);
+    const float z2 = ud_box_muller(w.z, w.w).x;
     const float Yn = Y + prm * z01.x, Cbn = Cb + prm * z01.y, Crn = Cr + prm * z2;
     r = cr_out(Yn + 1.402f * Crn, a);
     g = cr_out(Yn - 0.344136f * Cbn - 0.714136f * Crn, a);
@@ -146,7 +123,7 @@ __global__ void __launch_bounds__(64) cr_block_kernel(CrArgs a) {
   const int j = blockIdx.x, n = blockIdx.y;
   unsigned idl, idh;
   cr_id(a, n, idl, idh);
-  const uint4 u = cr_philox(make_uint4((unsigned)j, idl, idh, 0u), a.seed_lo, a.seed_hi ^ CR_BLOCK_TAG);
+  const uint4 u = ud_philox(make_uint4((unsigned)j, idl, idh, 0u), a.seed_lo, a.seed_hi ^ CR_BLOCK_TAG);
   const int r = (int)(((unsigned long long)u.x * (unsigned)(a.H - 7)) >> 32);
   const int c = (int)(((unsigned long long)u.y * (unsigned)(a.W - 7)) >> 32);
   const long long o = (long long)(r + (threadIdx.x >> 3)) * a.W + c + (threadIdx.x & 7);

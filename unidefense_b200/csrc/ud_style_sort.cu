@@ -19,6 +19,10 @@
 //     written right there -- no argsort, no gather, no re-read of the content.
 // Ties: equal content values keep their pixel order (stable); torch.sort leaves the order of ties unspecified, so the
 // reference's own output is implementation-defined there (and only there).
+//
+// A third mode ranks attribution maps for the deletion / insertion faithfulness curves (ud_rank_desc): the keys are
+// inverted (descending order), NaN keys sort after every number and -0 is keyed as +0, the pixel index is carried as in
+// the content sort, and the last pass writes rank[idx] = r.
 #include "../../include/unidefense_b200.h"
 #include "ud_common.cuh"
 
@@ -35,20 +39,31 @@ __device__ __forceinline__ float ss_unkey(uint32_t k) {
   return __uint_as_float(k ^ ((k >> 31) ? 0x80000000u : 0xffffffffu));
 }
 
+#define SS_STYLE 0     // keys only, sorted values out
+#define SS_CONTENT 1   // keys + pixel index, blend with the sorted style values out
+#define SS_RANK 2      // descending keys + pixel index, int32 rank per pixel out
+
+template <int MODE>
+__device__ __forceinline__ uint32_t ss_mode_key(float f) {
+  if (MODE != SS_RANK) return ss_key(f);
+  return f != f ? 0xffffffffu : ~ss_key(f == 0.f ? 0.f : f);
+}
+
 // shared: hist[4][256] | tbase[256] | dbase[256] | whist[SS_WARPS][256]
-template <bool CONTENT>
+template <int MODE>
 __global__ void __launch_bounds__(SS_THREADS, 1)
 ss_sort_kernel(const float* __restrict__ src, uint32_t* __restrict__ ws, const float* __restrict__ style_sorted,
-               const float* __restrict__ lmda, float* __restrict__ dst, int E, int C) {
+               const float* __restrict__ lmda, void* __restrict__ dst, int E, int C) {
   __shared__ int hist[4][256];
   __shared__ int tbase[256];
   __shared__ int dbase[256];
   __shared__ int whist[SS_WARPS][256];
+  constexpr bool IDX = MODE != SS_STYLE;      // carries the pixel index
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const long long seg = blockIdx.x;
   const float* sp = src + seg * (long long)E;
   // per-plane workspace: keys ping | keys pong (| idx ping | idx pong)
-  uint32_t* wsp = ws + seg * (long long)E * (CONTENT ? 4 : 2);
+  uint32_t* wsp = ws + seg * (long long)E * (IDX ? 4 : 2);
   uint32_t* kbuf[2] = {wsp, wsp + E};
   uint32_t* ibuf[2] = {wsp + 2 * (long long)E, wsp + 3 * (long long)E};
   const uint32_t lt_mask = (1u << lane) - 1u;
@@ -56,7 +71,7 @@ ss_sort_kernel(const float* __restrict__ src, uint32_t* __restrict__ ws, const f
   for (int i = tid; i < 4 * 256; i += SS_THREADS) (&hist[0][0])[i] = 0;
   __syncthreads();
   for (int i = tid; i < E; i += SS_THREADS) {
-    const uint32_t k = ss_key(__ldg(sp + i));
+    const uint32_t k = ss_mode_key<MODE>(__ldg(sp + i));
     atomicAdd(&hist[0][k & 255], 1);
     atomicAdd(&hist[1][(k >> 8) & 255], 1);
     atomicAdd(&hist[2][(k >> 16) & 255], 1);
@@ -66,8 +81,8 @@ ss_sort_kernel(const float* __restrict__ src, uint32_t* __restrict__ ws, const f
 
   float one_m_l = 0.f;
   const float* ssp = nullptr;
-  float* op = dst + seg * (long long)E;
-  if (CONTENT) {
+  float* op = static_cast<float*>(dst) + seg * (long long)E;
+  if (MODE == SS_CONTENT) {
     one_m_l = 1.f - __ldg(lmda + seg / C);
     ssp = style_sorted + seg * (long long)E;
   }
@@ -114,8 +129,8 @@ ss_sort_kernel(const float* __restrict__ src, uint32_t* __restrict__ ws, const f
         key[j] = 0;
         id[j] = (uint32_t)i;
         if (i < E) {
-          key[j] = (pass == 0) ? ss_key(__ldg(sp + i)) : kin[i];
-          if (CONTENT && pass > 0) id[j] = iin[i];
+          key[j] = (pass == 0) ? ss_mode_key<MODE>(__ldg(sp + i)) : kin[i];
+          if (IDX && pass > 0) id[j] = iin[i];
         }
       }
 #pragma unroll
@@ -154,8 +169,10 @@ ss_sort_kernel(const float* __restrict__ src, uint32_t* __restrict__ ws, const f
           const int pos = tbase[d] + whist[warp][d] + lr[j];
           if (pass < 3) {
             kout[pos] = key[j];
-            if (CONTENT) iout[pos] = id[j];
-          } else if (CONTENT) {
+            if (IDX) iout[pos] = id[j];
+          } else if (MODE == SS_RANK) {
+            static_cast<int*>(dst)[seg * (long long)E + id[j]] = pos;
+          } else if (MODE == SS_CONTENT) {
             // the content pixel id[j] has rank pos:  content + (1-l)*matched - (1-l)*content, in the reference's order
             const float cv = ss_unkey(key[j]);
             const float mv = __ldg(ssp + pos);
@@ -188,9 +205,24 @@ extern "C" int ud_spatial_style_transfer(const float* content, const float* styl
   float* sorted = static_cast<float*>(ws);
   uint32_t* sortws = reinterpret_cast<uint32_t*>(sorted + (size_t)N * C * HW);
   const int segs = N * C;
-  ss_sort_kernel<false><<<segs, SS_THREADS, 0, stream>>>(style, sortws, nullptr, nullptr, sorted, HW, C);
+  ss_sort_kernel<SS_STYLE><<<segs, SS_THREADS, 0, stream>>>(style, sortws, nullptr, nullptr, sorted, HW, C);
   int rc = ud_check_launch("spatial_style_sort_style");
   if (rc != UD_OK) return rc;
-  ss_sort_kernel<true><<<segs, SS_THREADS, 0, stream>>>(content, sortws, sorted, lmda, out, HW, C);
+  ss_sort_kernel<SS_CONTENT><<<segs, SS_THREADS, 0, stream>>>(content, sortws, sorted, lmda, out, HW, C);
   return ud_check_launch("spatial_style_sort_content");
+}
+
+extern "C" size_t ud_rank_desc_workspace_bytes(int N, int HW) {
+  if (N <= 0 || HW <= 0) return 0;
+  return sizeof(uint32_t) * (size_t)N * HW * 4;   // keys and pixel indices, ping and pong
+}
+
+extern "C" int ud_rank_desc(const float* map, int* rank, int N, int HW, void* ws, size_t ws_bytes, cudaStream_t stream) {
+  UD_REQUIRE(N >= 1 && HW >= 1, UD_ERR_INVALID, "rank_desc: bad shape N=%d HW=%d", N, HW);
+  UD_REQUIRE(N <= 65535 && HW <= (1 << 30), UD_ERR_UNSUPPORTED, "rank_desc: N=%d > 65535 or HW=%d > 2^30", N, HW);
+  UD_REQUIRE(map && rank, UD_ERR_INVALID, "rank_desc: null pointer");
+  const size_t need = ud_rank_desc_workspace_bytes(N, HW);
+  UD_REQUIRE(ws && ws_bytes >= need, UD_ERR_WORKSPACE, "rank_desc: workspace of %zu bytes, %zu needed", ws_bytes, need);
+  ss_sort_kernel<SS_RANK><<<N, SS_THREADS, 0, stream>>>(map, static_cast<uint32_t*>(ws), nullptr, nullptr, rank, HW, 1);
+  return ud_check_launch("rank_desc");
 }

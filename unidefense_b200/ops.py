@@ -1002,3 +1002,88 @@ def corrupt(x, kind, param, ids=None, seed=0, lo=-1.0, hi=1.0):
     L.check(lib.ud_corrupt(L.ptr(x.detach()), L.ptr(y), L.ptr(ids), N, H, W, k, float(param), seed, float(lo),
                            float(hi), L.ptr(ws), nws, L.stream()), "corrupt")
     return y
+
+
+# ------------------------------------------------------------------------------------------
+# a21: attribution maps and faithfulness inputs (unidefense_b200/explain.py)
+# ------------------------------------------------------------------------------------------
+ATTRIB_METHODS = {"ig": 0, "smoothgrad": 1}
+
+
+def _baseline_args(baseline, x, what):
+    """-> (tensor or None, scalar) for a float or an fp32 tensor of x's shape."""
+    if torch.is_tensor(baseline):
+        L.require_cuda_f32(baseline)
+        if baseline.shape != x.shape:
+            raise ValueError(f"{what}: baseline {tuple(baseline.shape)} does not match x {tuple(x.shape)}")
+        return baseline, 0.0
+    return None, float(baseline)
+
+
+def _device_scalar(t, dtype, what, name):
+    if t is None or not t.is_cuda or t.dtype != dtype or t.numel() != 1 or t.device.index != torch.cuda.current_device():
+        raise ValueError(f"{what}: {name} must be a one-element {dtype} tensor on the current device")
+
+
+def attrib_step(x, baseline, g, acc, p, attr, amap, k, alpha, w, method, sigma=None, ids=None, seed=None):
+    """One Integrated-Gradients / SmoothGrad iteration in place (csrc/ud_explain.cu; definitions in
+    include/unidefense_b200.h).  x, g, acc, p, attr: fp32 [N, C, H, W]; baseline: a float or a tensor of x's shape;
+    amap: fp32 [N, H, W]; k: int32 [1] step counter (read, never advanced); alpha, w: fp32 [S] step tables;
+    sigma: fp32 [1], seed: int64 [1] (the uint64's bits) and ids: int64 [N] or None, for 'smoothgrad'.
+    g None: acc = 0, p = p_k.  Otherwise acc += w_k*g, then p = p_{k+1}, or attr and amap at k = S-1."""
+    if method not in ATTRIB_METHODS:
+        raise ValueError(f"attrib_step: method must be one of {sorted(ATTRIB_METHODS)}, got {method!r}")
+    L.require_cuda_f32(x, g, acc, p, attr, amap, alpha, w, sigma)
+    if x.dim() != 4:
+        raise ValueError(f"attrib_step: x must be [N, C, H, W], got {tuple(x.shape)}")
+    N, C, H, W = x.shape
+    for name, t in (("g", g), ("acc", acc), ("p", p), ("attr", attr)):
+        if t is not None and t.shape != x.shape:
+            raise ValueError(f"attrib_step: {name} {tuple(t.shape)} does not match x {tuple(x.shape)}")
+    if amap.shape != (N, H, W):
+        raise ValueError(f"attrib_step: map {tuple(amap.shape)} is not {(N, H, W)}")
+    if alpha.dim() != 1 or w.shape != alpha.shape:
+        raise ValueError("attrib_step: alpha and w must be [S] tables of one length")
+    _device_scalar(k, torch.int32, "attrib_step", "k")
+    if method == "smoothgrad":
+        _device_scalar(sigma, torch.float32, "attrib_step", "sigma")
+        _device_scalar(seed, torch.int64, "attrib_step", "seed")
+    if ids is not None and (not ids.is_cuda or ids.device != x.device or ids.dtype != torch.int64 or ids.numel() != N):
+        raise ValueError(f"attrib_step: ids must be an int64 tensor of {N} entries on {x.device}")
+    b, bval = _baseline_args(baseline, x, "attrib_step")
+    L.check(L.lib().ud_attrib_step(L.ptr(x), L.ptr(b), bval, L.ptr(g), L.ptr(acc), L.ptr(p), L.ptr(attr), L.ptr(amap),
+                                   L.ptr(k), L.ptr(alpha), L.ptr(w), L.ptr(sigma), L.ptr(ids), L.ptr(seed),
+                                   alpha.numel(), ATTRIB_METHODS[method], N, C, H, W, L.stream()), "attrib_step")
+
+
+def rank_desc(amap):
+    """rank [N, H, W] int32: the position of each pixel of amap [N, H, W] in its sample's stable descending order
+    (ties by ascending pixel index, NaN after every number); one radix sort per plane (csrc/ud_style_sort.cu)."""
+    L.require_cuda_f32(amap)
+    if amap.dim() != 3:
+        raise ValueError(f"rank_desc: map must be [N, H, W], got {tuple(amap.shape)}")
+    N, H, W = amap.shape
+    rank = torch.empty(amap.shape, dtype=torch.int32, device=amap.device)
+    lib = L.lib()
+    nws = lib.ud_rank_desc_workspace_bytes(N, H * W)
+    ws = L.workspace(nws, amap.device)
+    L.check(lib.ud_rank_desc(L.ptr(amap), L.ptr(rank), N, H * W, L.ptr(ws), ws.numel(), L.stream()), "rank_desc")
+    return rank
+
+
+def attrib_mask(x, baseline, rank, t, j, y, insertion):
+    """y = the deletion (insertion=False) or insertion input of faithfulness point j (int32 [1] on the device) from
+    rank [N, H, W] (rank_desc) and the thresholds t (int32 [K+1] on the device): the pixels of rank < t[j] take the
+    baseline (deletion) or x (insertion), every other pixel the other one."""
+    L.require_cuda_f32(x, y)
+    if x.dim() != 4 or y.shape != x.shape:
+        raise ValueError(f"attrib_mask: x and y must be one [N, C, H, W] shape, got {tuple(x.shape)}, {tuple(y.shape)}")
+    N, C, H, W = x.shape
+    if rank.dtype != torch.int32 or not rank.is_contiguous() or rank.shape != (N, H, W) or rank.device != x.device:
+        raise ValueError(f"attrib_mask: rank must be a contiguous int32 {(N, H, W)} tensor on {x.device}")
+    if t.dtype != torch.int32 or t.dim() != 1 or t.numel() < 2 or t.device != x.device:
+        raise ValueError("attrib_mask: t must be an int32 [K+1] table (K >= 1) on x's device")
+    _device_scalar(j, torch.int32, "attrib_mask", "j")
+    b, bval = _baseline_args(baseline, x, "attrib_mask")
+    L.check(L.lib().ud_attrib_mask(L.ptr(x), L.ptr(b), bval, L.ptr(rank), L.ptr(t), L.ptr(j), t.numel() - 1, L.ptr(y),
+                                   int(bool(insertion)), N, C, H, W, L.stream()), "attrib_mask")
