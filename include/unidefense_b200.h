@@ -22,8 +22,8 @@
  *    whose transposed resize accumulates with float atomics.  The input-gradient outputs (g_x of ud_recon_tail_bwd,
  *    ud_attn_prep_bwd, ud_gaussian_blur5_bwd, ud_downscale_nearest_bwd; g_diff of ud_dyfi_mask_bwd) are gathers
  *    written once per element: bitwise reproducible.  ud_attack_step's per-sample norms are fixed-order too.
- *    ud_corrupt, ud_attrib_step, ud_attrib_mask and ud_rank_desc write every output element once from a fixed-order
- *    computation: bitwise reproducible.
+ *    ud_corrupt, ud_attrib_step, ud_attrib_mask, ud_rank_desc and ud_fourier_perturb write every output element once
+ *    from a fixed-order computation: bitwise reproducible.
  */
 #ifndef UNIDEFENSE_B200_H
 #define UNIDEFENSE_B200_H
@@ -45,7 +45,7 @@ typedef struct CUstream_st* cudaStream_t;
 #define UD_API
 #endif
 
-#define UD_B200_VERSION 104
+#define UD_B200_VERSION 105
 #define UD_FFT_MAX_N 1024
 
 #define UD_ACT_NONE 0
@@ -394,6 +394,29 @@ UD_API int ud_rank_desc(const float* map, int* rank, int N, int HW, void* ws, si
 UD_API int ud_attrib_mask(const float* x, const float* base, float base_value, const int* rank, const int* t,
                           const int* j, int points, float* y, int insertion, int N, int C, int H, int W,
                           cudaStream_t stream);
+
+/* ---- a22: Fourier-basis perturbations (Fourier heat maps; Yin et al., "A Fourier Perspective on Model Robustness in
+ * Computer Vision", NeurIPS 2019) --------------------------------------------------------------------------------------
+ * x, y fp32 [N, C, H, W] (values in [lo, hi]; y must not overlap x); 1 <= C <= 128, 1 <= H, W <= 4096, H*W <= 2^24 (so
+ * the phase numerator below is exact in fp32), N <= 65535.
+ *  Canonical frequency: a signed grid point (u, v) and (-u, -v) give the same image; the canonical pair (uu, vv) is
+ *    the lexicographically smaller of (u mod H, v mod W) and ((-u) mod H, (-v) mod W).  freqs: int [F][2] canonical
+ *    pairs on the device; the kernel takes them as given (a non-canonical mirror pair keys different signs).
+ *  Basis: k(h, w) = (((uu*h) mod H)*W + ((vv*w) mod W)*H) mod (H*W) in integers; t = k / (H*W) as one correctly
+ *    rounded fp32 division; c = cospif(2t).  a = sqrt(1/(H*W)) when 2uu = 0 (mod H) and 2vv = 0 (mod W) (DC and the
+ *    Nyquist corners), sqrt(2/(H*W)) otherwise, computed in fp64 on the host and rounded to fp32.  Each channel plane
+ *    of a*cos(2 pi t) has L2 norm 1 and a 2-D spectrum that is non-zero only at +-(u, v).
+ *  Sign: r_{n,c} = +1 if bit (c & 31) of word (c >> 5) of Philox4x32-10(ctr = ((uu << 16) | vv, id_lo, id_hi, 0),
+ *    key = (seed_lo, seed_hi ^ 0x464F5552)) is 0, else -1.  ids: int64 [N] (NULL: 0..N-1), so sample i gets the same
+ *    perturbation at (u, v) in any batch, grid and rank.
+ *  Output: s = r * __fmul_rn(eps, a); y = clamp(__fadd_rn(x, __fmul_rn(s, c)), lo, hi) = min(max(., lo), hi).  eps is
+ *    the L2 norm of the perturbation of each channel plane in input units; the per-pixel peak is eps*a.
+ * ud_fourier_perturb: f: int, eps: float, seed: uint64, all on the device, so one captured graph serves every
+ *   frequency, eps and seed.  f out of [0, F), or freqs[f] out of [0, H) x [0, W), writes nothing.  One elementwise
+ *   launch (one read of x, one write of y); every element is written once: bitwise reproducible.                  */
+UD_API int ud_fourier_perturb(const float* x, float* y, const int* freqs, int F, const int* f, const float* eps,
+                              const long long* ids, const unsigned long long* seed, float lo, float hi, int N, int C,
+                              int H, int W, cudaStream_t stream);
 
 /* ---- §8(e): the exchange step -- SyncBatchNorm statistics over NVLink peer memory ----------------------------------
  * Replaces the two per-layer collectives of torch.nn.SyncBatchNorm (engine/forgery_engine.py:142 converts all 99

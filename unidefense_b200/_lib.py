@@ -99,6 +99,7 @@ SIGNATURES = {
     "ud_rank_desc_workspace_bytes": (c_sz, [c_i, c_i]),
     "ud_rank_desc": (c_i, [c_p, c_p, c_i, c_i, c_p, c_sz, c_p]),
     "ud_attrib_mask": (c_i, [c_p, c_p, c_f] + [c_p] * 3 + [c_i, c_p] + [c_i] * 5 + [c_p]),
+    "ud_fourier_perturb": (c_i, [c_p] * 3 + [c_i] + [c_p] * 4 + [c_f, c_f] + [c_i] * 4 + [c_p]),
 }
 
 

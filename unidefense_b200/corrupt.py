@@ -69,21 +69,22 @@ def _scores(logits):
 
 def auc(scores, labels):
     """Mann-Whitney AUC with tie-averaged ranks, on the device and without a host synchronisation (NaN when one class
-    is absent).  Label 1 is the positive (fake) class."""
-    n = scores.numel()
-    v, order = torch.sort(scores.double())
+    is absent).  Label 1 is the positive (fake) class.  scores [..., n] against labels [n]: one AUC per row of the
+    last dimension.  Every partial sum is a multiple of 1/2 below 2^53, so a row scores the same alone or batched."""
+    n = scores.shape[-1]
+    v, order = torch.sort(scores.double(), dim=-1)
     pos = (labels[order] == 1).double()
     idx = torch.arange(n, device=scores.device)
-    new = torch.ones(n, dtype=torch.bool, device=scores.device)
-    new[1:] = v[1:] != v[:-1]
+    new = torch.ones(v.shape, dtype=torch.bool, device=scores.device)
+    new[..., 1:] = v[..., 1:] != v[..., :-1]
     end = torch.ones_like(new)
-    end[:-1] = new[1:]
-    first = torch.cummax(torch.where(new, idx, 0), 0).values
-    last = torch.flip(torch.cummin(torch.flip(torch.where(end, idx, n - 1), [0]), 0).values, [0])
+    end[..., :-1] = new[..., 1:]
+    first = torch.cummax(torch.where(new, idx, 0), -1).values
+    last = torch.flip(torch.cummin(torch.flip(torch.where(end, idx, n - 1), [-1]), -1).values, [-1])
     rank = (first + last).double() / 2 + 1
-    n_pos = pos.sum()
+    n_pos = pos.sum(-1)
     n_neg = n - n_pos
-    return ((rank * pos).sum() - n_pos * (n_pos + 1) / 2) / (n_pos * n_neg)
+    return ((rank * pos).sum(-1) - n_pos * (n_pos + 1) / 2) / (n_pos * n_neg)
 
 
 def evaluate(model, batches, kinds=KINDS, severities=(1, 2, 3, 4, 5), seed=0, lo=-1.0, hi=1.0):

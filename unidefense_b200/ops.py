@@ -1087,3 +1087,30 @@ def attrib_mask(x, baseline, rank, t, j, y, insertion):
     b, bval = _baseline_args(baseline, x, "attrib_mask")
     L.check(L.lib().ud_attrib_mask(L.ptr(x), L.ptr(b), bval, L.ptr(rank), L.ptr(t), L.ptr(j), t.numel() - 1, L.ptr(y),
                                    int(bool(insertion)), N, C, H, W, L.stream()), "attrib_mask")
+
+
+# ------------------------------------------------------------------------------------------
+# a22: Fourier-basis perturbations (unidefense_b200/fourier.py)
+# ------------------------------------------------------------------------------------------
+def fourier_perturb(x, y, freqs, f, eps, ids, seed, lo, hi):
+    """y = clamp(x + r*eps*a*cos(2 pi k / (H*W)), lo, hi) at the canonical frequency freqs[f] (csrc/ud_fourier.cu;
+    definitions in include/unidefense_b200.h).  x, y: fp32 [N, C, H, W], y not overlapping x; freqs: int32 [F, 2]
+    canonical (uu, vv) pairs; f: int32 [1]; eps: fp32 [1]; seed: int64 [1] (the uint64's bits), all on the device;
+    ids: int64 [N] per-sample sign keys or None (0..N-1).  f out of [0, F) writes nothing.  No autograd."""
+    L.require_cuda_f32(x, y, eps)
+    if x.dim() != 4 or y.shape != x.shape:
+        raise ValueError(f"fourier_perturb: x and y must be one [N, C, H, W] shape, got {tuple(x.shape)}, "
+                         f"{tuple(y.shape)}")
+    N, C, H, W = x.shape
+    if (freqs.dtype != torch.int32 or freqs.dim() != 2 or freqs.shape[0] < 1 or freqs.shape[1] != 2
+            or not freqs.is_contiguous() or freqs.device != x.device):
+        raise ValueError(f"fourier_perturb: freqs must be a contiguous int32 [F, 2] table (F >= 1) on {x.device}")
+    _device_scalar(f, torch.int32, "fourier_perturb", "f")
+    _device_scalar(eps, torch.float32, "fourier_perturb", "eps")
+    _device_scalar(seed, torch.int64, "fourier_perturb", "seed")
+    if ids is not None and (not ids.is_cuda or ids.device != x.device or ids.dtype != torch.int64 or ids.numel() != N
+                            or not ids.is_contiguous()):
+        raise ValueError(f"fourier_perturb: ids must be a contiguous int64 tensor of {N} entries on {x.device}")
+    L.check(L.lib().ud_fourier_perturb(L.ptr(x), L.ptr(y), L.ptr(freqs), freqs.shape[0], L.ptr(f), L.ptr(eps),
+                                       L.ptr(ids), L.ptr(seed), float(lo), float(hi), N, C, H, W, L.stream()),
+            "fourier_perturb")
