@@ -119,7 +119,7 @@ def _auc_scipy(s, y):
 
 
 def test_batched_auc_matches_scipy_row_by_row():
-    from unidefense_b200.corrupt import auc
+    from unidefense_b200._evaluator import auc
     rng = np.random.default_rng(4)
     y = np.array([0, 1] * 20)
     s = rng.integers(0, 6, (7, 40)).astype(np.float32) / 5           # many ties
@@ -155,7 +155,7 @@ def _auc_parent(scores, labels):
 
 
 def test_one_dimensional_auc_is_unchanged():
-    from unidefense_b200.corrupt import auc
+    from unidefense_b200._evaluator import auc
     rng = np.random.default_rng(5)
     for n in (1, 2, 9, 100, 1001):
         y = torch.from_numpy(rng.integers(0, 2, n))

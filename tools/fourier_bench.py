@@ -62,7 +62,7 @@ def _model():
 
 def per_point(iters, flush):
     from unidefense_b200 import ops
-    from unidefense_b200.corrupt import _scores
+    from unidefense_b200._evaluator import p_fake
     from unidefense_b200.fourier import FourierHeatMap
     model = _model()
     rows = []
@@ -78,7 +78,7 @@ def per_point(iters, flush):
             def eager():                        # the kernel, a no_grad forward, the scores
                 ops.fourier_perturb(x, y, st.freqs, st.f, st.eps, None, st.seed, -1.0, 1.0)
                 with torch.no_grad():
-                    p, pred = _scores(model(y)["cls_out"])
+                    p, pred = p_fake(model(y)["cls_out"])
                 p_buf.copy_(p)
 
             def replay():

@@ -193,6 +193,23 @@ def require_cuda_f32(*tensors, also=()):
             raise RuntimeError("unidefense_b200 kernels need contiguous tensors")
 
 
+def require_ids(ids, x, what):
+    """Per-sample int64 keys of the random kernels: None, or N entries on x's device.  -> None or contiguous [N]."""
+    if ids is None:
+        return None
+    if not torch.is_tensor(ids) or ids.dtype != torch.int64 or ids.device != x.device or ids.numel() != x.shape[0]:
+        raise ValueError(f"{what}: ids must be an int64 tensor of {x.shape[0]} entries on {x.device}")
+    return ids.reshape(-1).contiguous()
+
+
+def seed_bits(seed, what):
+    """-> the int64 with the bits of the uint64 `seed`, as the kernels' seed arguments take it."""
+    seed = int(seed)
+    if not 0 <= seed < 2 ** 64:
+        raise ValueError(f"{what}: seed {seed} is not a uint64")
+    return seed - 2 ** 64 if seed >= 2 ** 63 else seed
+
+
 _ws = {}
 _ws_retired = []
 

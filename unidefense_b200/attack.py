@@ -15,21 +15,12 @@ captured forward plus a select-only step scores the final iterate.  Across resta
 iterate of highest loss.  The caller's torch.autocast context applies (bf16 evaluation needs no option).
 """
 import math
-import types
 
 import torch
 import torch.nn.functional as F
 
 from . import ops
-
-_capture_streams = {}       # one side stream per device: warm-up and capture share it, and with it the op workspaces
-
-
-def _capture_stream(device):
-    idx = device.index if device.index is not None else torch.cuda.current_device()
-    if idx not in _capture_streams:
-        _capture_streams[idx] = torch.cuda.Stream(device=idx)
-    return _capture_streams[idx]
+from ._evaluator import GraphedEvaluator, check_call, predicted
 
 
 def _random_start(x0, eps, norm, lo, hi):
@@ -44,39 +35,35 @@ def _random_start(x0, eps, norm, lo, hi):
     return torch.clamp(x0 + z * (eps * r).view_as(e), lo, hi)
 
 
-class PGD:
+class PGD(GraphedEvaluator):
     """Projected gradient descent (ascent on the loss) with random restarts and best-iterate tracking.  The captured
     graphs live on this object (deleting it frees them); a new eps or alpha on a seen shape reuses them."""
+    name = "PGD"
 
     def __init__(self, model, norm="linf", steps=10, restarts=1, random_start=True, lo=-1.0, hi=1.0):
         if norm not in ops.ATTACK_NORMS:
             raise ValueError(f"PGD: norm must be one of {sorted(ops.ATTACK_NORMS)}, got {norm!r}")
         if int(steps) < 1 or int(restarts) < 1:
             raise ValueError(f"PGD: steps ({steps}) and restarts ({restarts}) must be >= 1")
-        if not float(lo) <= float(hi):
-            raise ValueError(f"PGD: lo={lo} > hi={hi}")
-        self.model, self.norm = model, norm
+        super().__init__(model, lo, hi)
+        self.norm = norm
         self.steps, self.restarts, self.random_start = int(steps), int(restarts), bool(random_start)
-        self.lo, self.hi = float(lo), float(hi)
-        self._graphs = {}
 
     # ---- the objective ------------------------------------------------------------------------------------------
     @staticmethod
     def _loss_and_miss(logits, labels):
         logits = logits.float()
         if logits.shape[1] == 1:
-            z = logits[:, 0]
-            return F.binary_cross_entropy_with_logits(z, labels.float(), reduction="none"), (z > 0).long() != labels
-        return F.cross_entropy(logits, labels, reduction="none"), logits.argmax(dim=1) != labels
+            loss = F.binary_cross_entropy_with_logits(logits[:, 0], labels.float(), reduction="none")
+        else:
+            loss = F.cross_entropy(logits, labels, reduction="none")
+        return loss, predicted(logits) != labels
 
     def _score(self, st, logits, loss, miss):
         """Logits of the best iterate and the fooled flags; runs before ud_attack_step updates best_loss."""
         imp = loss > st.best_loss
         st.best_logits.copy_(torch.where(imp[:, None], logits.float(), st.best_logits))
         st.fooled.logical_or_(miss)
-
-    def _autocast(self, st):
-        return torch.autocast("cuda", dtype=st.amp_dtype, enabled=st.amp_dtype is not None, cache_enabled=False)
 
     def _iteration(self, st):
         with self._autocast(st), torch.enable_grad():
@@ -96,60 +83,31 @@ class PGD:
         self._score(st, logits, loss, miss)
         ops.attack_step(st.x0, st.x_adv, None, loss, st.best_loss, st.x_best, None, None, self.lo, self.hi, self.norm)
 
+    def _best_logits(self, st):
+        """A first forward finds the number of logits K of the best_logits buffer."""
+        with self._autocast(st), torch.no_grad():
+            K = self.model(st.x_adv)["cls_out"].shape[1]
+        st.best_logits = torch.zeros(st.x0.shape[0], K, device=st.x0.device)
+
     # ---- capture --------------------------------------------------------------------------------------------------
-    def _capture(self, x, labels, amp_dtype):
+    def _state(self, st, x, labels):
         N = x.shape[0]
-        st = types.SimpleNamespace(amp_dtype=amp_dtype)
         st.x0, st.x_adv, st.x_best = x.clone(), x.clone(), x.clone()
         st.labels = labels.clone()
         st.eps = torch.zeros(N, device=x.device)
         st.alpha = torch.zeros(N, device=x.device)
         st.best_loss = torch.full((N,), -math.inf, device=x.device)
         st.fooled = torch.zeros(N, dtype=torch.bool, device=x.device)
-        side = _capture_stream(x.device)
-        side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side):
-            # warm-up: first calls build FFT tables with a synchronous copy and grow the op workspaces (header
-            # conventions); none of that may happen inside the capture
-            with self._autocast(st), torch.no_grad():
-                K = self.model(st.x_adv)["cls_out"].shape[1]
-            st.best_logits = torch.zeros(N, K, device=x.device)
-            for _ in range(2):
-                self._iteration(st)
-                self._final(st)
-        torch.cuda.current_stream().wait_stream(side)
-        torch.cuda.synchronize()
-        st.step = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(st.step, stream=side, capture_error_mode="thread_local"):
-            self._iteration(st)
-        st.final = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(st.final, pool=st.step.pool(), stream=side, capture_error_mode="thread_local"):
-            self._final(st)
-        return st
+        st.step, st.final = self._capture(st, self._iteration, self._final, prepare=self._best_logits)
 
     # ---- the attack -------------------------------------------------------------------------------------------------
     def __call__(self, x, labels, eps=16 / 255, alpha=None):
-        if any(m.training for m in self.model.modules()):
-            raise RuntimeError("PGD: the model is in train mode; call model.eval() first (every replay would move the "
-                               "BatchNorm running statistics and draw dropout)")
-        if not torch.is_tensor(x) or not x.is_cuda or x.dtype != torch.float32:
-            raise RuntimeError("PGD: x must be a CUDA fp32 tensor")
-        if x.device.index != torch.cuda.current_device():
-            raise RuntimeError(f"PGD: x is on cuda:{x.device.index} but the current device is "
-                               f"cuda:{torch.cuda.current_device()}")
+        x, labels, key = check_call(self.name, self.model, x, labels)
         eps = float(eps)
         if not eps >= 0.0:
             raise ValueError(f"PGD: eps must be >= 0, got {eps}")
         alpha = 2.5 * eps / self.steps if alpha is None else float(alpha)
-        labels = torch.as_tensor(labels).to(device=x.device, dtype=torch.long).reshape(-1)
-        if x.dim() < 2 or labels.numel() != x.shape[0]:
-            raise ValueError(f"PGD: {labels.numel()} labels for a batch of {x.shape[0] if x.dim() else 0}")
-        x = x.detach().contiguous()
-        amp = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else None
-        key = (tuple(x.shape), amp, x.device.index)
-        st = self._graphs.get(key)
-        if st is None:
-            st = self._graphs[key] = self._capture(x, labels, amp)
+        st = self._graphed(key, x, labels)
         st.x0.copy_(x)
         st.x_best.copy_(x)
         st.labels.copy_(labels)

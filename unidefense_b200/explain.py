@@ -22,63 +22,20 @@ NaN last); point j = 0..K of the deletion curve replaces the first floor(j*H*W/K
 baseline, the insertion curve starts from the baseline and restores them; the score is p(target | input) and the AUC
 the trapezoid over j/K (after Petsiuk et al., RISE).  Exact definitions: include/unidefense_b200.h (ud_attrib_step).
 
-As attack.PGD does, one iteration (forward, F, d F / dx, ud_attrib_step) is captured as a CUDA graph once per input
-shape, autocast state and device and replayed; so is one faithfulness point (the two masked inputs, their no_grad
-forwards, the scores).  Nothing in a call synchronises with the host.  The caller's torch.autocast context applies.
+One iteration (forward, F, d F / dx, ud_attrib_step) is captured as a CUDA graph once per input shape, autocast state
+and device and replayed (_evaluator.GraphedEvaluator); so is one faithfulness point (the two masked inputs, their
+no_grad forwards, the scores).  Nothing in a call synchronises with the host.  The caller's torch.autocast context
+applies.
 """
-import types
-
 import torch
-import torch.nn.functional as F
 
+from . import _lib as L
 from . import ops
-from .attack import _capture_stream
+from ._evaluator import GraphedEvaluator, check_call, log_p as objective, predicted     # noqa: F401  (public)
 
 
-def objective(logits, target):
-    """F = log p(target | logits) per sample, in fp32."""
-    logits = logits.float()
-    if logits.shape[1] == 1:
-        z = logits[:, 0]
-        return F.logsigmoid(torch.where(target == 1, z, -z))
-    return torch.log_softmax(logits, dim=1).gather(1, target[:, None])[:, 0]
-
-
-def _predicted(logits):
-    logits = logits.float()
-    return (logits[:, 0] > 0).long() if logits.shape[1] == 1 else logits.argmax(dim=1)
-
-
-class _Explainer:
+class _Explainer(GraphedEvaluator):
     name = "explain"
-
-    def __init__(self, model, lo, hi):
-        if not float(lo) <= float(hi):
-            raise ValueError(f"{self.name}: lo={lo} > hi={hi}")
-        self.model, self.lo, self.hi = model, float(lo), float(hi)
-        self._graphs = {}
-
-    def _autocast(self, st):
-        return torch.autocast("cuda", dtype=st.amp_dtype, enabled=st.amp_dtype is not None, cache_enabled=False)
-
-    def _check(self, x, labels):
-        """-> (x contiguous, labels as int64 [N] or None, the graph key)"""
-        if any(m.training for m in self.model.modules()):
-            raise RuntimeError(f"{self.name}: the model is in train mode; call model.eval() first (every replay would "
-                               "move the BatchNorm running statistics and draw dropout)")
-        if not torch.is_tensor(x) or not x.is_cuda or x.dtype != torch.float32:
-            raise RuntimeError(f"{self.name}: x must be a CUDA fp32 tensor")
-        if x.device.index != torch.cuda.current_device():
-            raise RuntimeError(f"{self.name}: x is on cuda:{x.device.index} but the current device is "
-                               f"cuda:{torch.cuda.current_device()}")
-        if x.dim() != 4:
-            raise ValueError(f"{self.name}: x must be [N, C, H, W], got {tuple(x.shape)}")
-        if labels is not None:
-            labels = torch.as_tensor(labels).to(device=x.device, dtype=torch.long).reshape(-1)
-            if labels.numel() != x.shape[0]:
-                raise ValueError(f"{self.name}: {labels.numel()} labels for a batch of {x.shape[0]}")
-        amp = torch.get_autocast_dtype("cuda") if torch.is_autocast_enabled("cuda") else None
-        return x.detach().contiguous(), labels, (tuple(x.shape), amp, x.device.index)
 
     def _baseline(self, st, baseline, x):
         """Fill st.b from None (lo), a float or a tensor of x's shape on x's device."""
@@ -92,21 +49,19 @@ class _Explainer:
         else:
             st.b.fill_(float(baseline))
 
-    def _new_state(self, x, amp):
+    def _new_state(self, st, x):
         N = x.shape[0]
-        st = types.SimpleNamespace(amp_dtype=amp)
         st.x = x.clone()
         st.labels = torch.zeros(N, dtype=torch.long, device=x.device)
         st.use_labels = torch.zeros((), dtype=torch.bool, device=x.device)
         st.target = torch.zeros(N, dtype=torch.long, device=x.device)
         st.f_x = torch.zeros(N, device=x.device)
-        return st
 
     def _target(self, st):
         """Forward at x: the target (the label, or the class predicted at x) and F(x)."""
         with self._autocast(st), torch.no_grad():
             logits = self.model(st.x)["cls_out"]
-        st.target.copy_(torch.where(st.use_labels, st.labels, _predicted(logits)))
+        st.target.copy_(torch.where(st.use_labels, st.labels, predicted(logits)))
         st.f_x.copy_(objective(logits, st.target))
 
     def _set_labels(self, st, labels):
@@ -115,24 +70,6 @@ class _Explainer:
         else:
             st.labels.copy_(labels)
             st.use_labels.fill_(True)
-
-    def _capture(self, st, prologue, point, warm=2):
-        """Warm up on the side stream (first calls build tables and grow the op workspaces, which must not happen
-        inside a capture), then capture `prologue` and `point` into graphs sharing one pool."""
-        side = _capture_stream(st.x.device)
-        side.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(side):
-            for _ in range(warm):
-                prologue(st)
-                point(st)
-        torch.cuda.current_stream().wait_stream(side)
-        torch.cuda.synchronize()
-        st.prologue = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(st.prologue, stream=side, capture_error_mode="thread_local"):
-            prologue(st)
-        st.point = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(st.point, pool=st.prologue.pool(), stream=side, capture_error_mode="thread_local"):
-            point(st)
 
 
 class _Attribution(_Explainer):
@@ -159,8 +96,8 @@ class _Attribution(_Explainer):
                         st.sigma, st.ids, st.seed)
         st.k.add_(1)
 
-    def _state(self, x, amp):
-        st = self._new_state(x, amp)
+    def _state(self, st, x):
+        self._new_state(st, x)
         N, C, H, W = x.shape
         dev = x.device
         alpha, w = self._tables()
@@ -177,14 +114,11 @@ class _Attribution(_Explainer):
             st.sigma = torch.tensor([self.noise * (self.hi - self.lo)], dtype=torch.float32, device=dev)
             st.seed = torch.zeros(1, dtype=torch.int64, device=dev)
             st.ids = torch.arange(N, dtype=torch.int64, device=dev)
-        self._capture(st, self._prologue, self._iteration)
-        return st
+        st.prologue, st.point = self._capture(st, self._prologue, self._iteration)
 
     def _run(self, x, labels, setup):
-        x, labels, key = self._check(x, labels)
-        st = self._graphs.get(key)
-        if st is None:
-            st = self._graphs[key] = self._state(x, key[1])
+        x, labels, key = check_call(self.name, self.model, x, labels)
+        st = self._graphed(key, x)
         setup(st)
         st.x.copy_(x)
         self._set_labels(st, labels)
@@ -235,19 +169,15 @@ class SmoothGrad(_Attribution):
         return [1.0] * self.draws, [1.0 / self.draws] * self.draws
 
     def __call__(self, x, labels=None, ids=None, seed=0):
-        seed = int(seed)
-        if not 0 <= seed < 2 ** 64:
-            raise ValueError(f"{self.name}: seed {seed} is not a uint64")
-        if ids is not None and (not torch.is_tensor(ids) or ids.dtype != torch.int64 or ids.device != x.device
-                                or ids.numel() != x.shape[0]):
-            raise ValueError(f"{self.name}: ids must be an int64 tensor of {x.shape[0]} entries on {x.device}")
+        seed = L.seed_bits(seed, self.name)
+        ids = L.require_ids(ids, x, self.name)
 
         def setup(st):
-            st.seed.fill_(seed - 2 ** 64 if seed >= 2 ** 63 else seed)        # the uint64's bits
+            st.seed.fill_(seed)
             if ids is None:
                 torch.arange(st.ids.numel(), out=st.ids)
             else:
-                st.ids.copy_(ids.reshape(-1))
+                st.ids.copy_(ids)
 
         st = self._run(x, labels, setup)
         return {"attr": st.attr.clone(), "map": st.map.clone(), "target": st.target.clone()}
@@ -277,8 +207,8 @@ class Faithfulness(_Explainer):
                 s.index_copy_(1, col, p[:, None])
         st.j.add_(1)
 
-    def _state(self, x, amp):
-        st = self._new_state(x, amp)
+    def _state(self, st, x):
+        self._new_state(st, x)
         N, C, H, W = x.shape
         dev, K = x.device, self.points
         st.b = torch.full_like(x, self.lo)
@@ -288,20 +218,17 @@ class Faithfulness(_Explainer):
         st.y_del, st.y_ins = torch.empty_like(x), torch.empty_like(x)
         st.deletion = torch.zeros(N, K + 1, device=dev)
         st.insertion = torch.zeros(N, K + 1, device=dev)
-        self._capture(st, self._prologue, self._point)
-        return st
+        st.prologue, st.point = self._capture(st, self._prologue, self._point)
 
     def __call__(self, x, amap, labels=None, baseline=None):
-        x, labels, key = self._check(x, labels)
+        x, labels, key = check_call(self.name, self.model, x, labels)
         N, _, H, W = x.shape
         if not torch.is_tensor(amap) or amap.shape != (N, H, W):
             raise ValueError(f"{self.name}: the map must be [N, H, W] = {(N, H, W)}, got "
                              f"{tuple(amap.shape) if torch.is_tensor(amap) else type(amap).__name__}")
         if not amap.is_cuda or amap.dtype != torch.float32 or amap.device != x.device:
             raise RuntimeError(f"{self.name}: the map must be an fp32 tensor on {x.device}")
-        st = self._graphs.get(key)
-        if st is None:
-            st = self._graphs[key] = self._state(x, key[1])
+        st = self._graphed(key, x)
         self._baseline(st, baseline, x)
         st.x.copy_(x)
         self._set_labels(st, labels)

@@ -13,19 +13,18 @@ canonical frequency is evaluated once and its result fills every grid point that
 floor(floor(min(H, W)/2) / R), so the grid reaches toward Nyquist (380^2, R = 15: stride 12, 481 frequencies).
 Exact definitions: include/unidefense_b200.h (ud_fourier_perturb).
 
-As explain does, two graphs are captured per input shape, autocast state and device and replayed: the clean forward,
-then one frequency point (ud_fourier_perturb, a no_grad forward, the scores into row f of [F, N] buffers, f += 1),
-replayed F times per batch.  Nothing synchronises with the host until the one read of the metrics at the end.  The
-caller's torch.autocast context applies.
+Two graphs are captured per input shape, autocast state and device and replayed (_evaluator.GraphedEvaluator): the
+clean forward, then one frequency point (ud_fourier_perturb, a no_grad forward, the scores into row f of [F, N]
+buffers, f += 1), replayed F times per batch.  Nothing synchronises with the host until the one read of the metrics
+at the end.  The caller's torch.autocast context applies.
 """
 import math
-import types
 
 import torch
 
+from . import _lib as L
 from . import ops
-from .corrupt import _scores, auc
-from .explain import _Explainer
+from ._evaluator import GraphedEvaluator, p_fake, tally
 
 
 def canonical(u, v, H, W):
@@ -55,7 +54,7 @@ def grid(H, W, radius, stride):
     return u, v, table, index
 
 
-class FourierHeatMap(_Explainer):
+class FourierHeatMap(GraphedEvaluator):
     """Accuracy and AUC of a binary detector under Fourier-basis perturbations of L2 norm `eps` per channel plane.  The
     captured graphs live on this object (deleting it frees them); a new eps, seed or batch of a seen shape reuses them."""
     name = "FourierHeatMap"
@@ -92,7 +91,7 @@ class FourierHeatMap(_Explainer):
 
     def _prologue(self, st):
         with self._autocast(st), torch.no_grad():
-            p, pred = _scores(self.model(st.x)["cls_out"])
+            p, pred = p_fake(self.model(st.x)["cls_out"])
         st.p_clean.copy_(p)
         st.hit_clean.copy_(pred == st.labels)
         st.f.zero_()
@@ -100,15 +99,14 @@ class FourierHeatMap(_Explainer):
     def _point(self, st):
         ops.fourier_perturb(st.x, st.y, st.freqs, st.f, st.eps, st.ids, st.seed, self.lo, self.hi)
         with self._autocast(st), torch.no_grad():
-            p, pred = _scores(self.model(st.y)["cls_out"])
+            p, pred = p_fake(self.model(st.y)["cls_out"])
         row = st.f.long()
         st.p.index_copy_(0, row, p[None])
         st.hit.index_copy_(0, row, (pred == st.labels)[None])
         st.f.add_(1)
 
-    def _state(self, x, amp, table):
+    def _state(self, st, x, table):
         N, dev, F = x.shape[0], x.device, len(table)
-        st = types.SimpleNamespace(amp_dtype=amp)
         st.x, st.y = x.clone(), torch.empty_like(x)
         st.labels = torch.zeros(N, dtype=torch.long, device=dev)
         st.ids = torch.arange(N, dtype=torch.int64, device=dev)
@@ -120,61 +118,37 @@ class FourierHeatMap(_Explainer):
         st.hit = torch.zeros(F, N, dtype=torch.bool, device=dev)
         st.p_clean = torch.zeros(N, device=dev)
         st.hit_clean = torch.zeros(N, dtype=torch.bool, device=dev)
-        self._capture(st, self._prologue, self._point)
-        return st
+        st.prologue, st.point = self._capture(st, self._prologue, self._point)
 
     def __call__(self, batches, seed=0):
         """batches yields (x, labels) or (x, labels, ids): x CUDA fp32 [N, C, H, W] of one C, H, W, labels {0 real,
         1 fake}, ids int64 [N] (default: the running sample index over the iterable).  The model must be in eval mode."""
-        seed = int(seed)
-        if not 0 <= seed < 2 ** 64:
-            raise ValueError(f"{self.name}: seed {seed} is not a uint64")
-        p, hit, p_clean, hit_clean, all_labels = [], [], [], [], []
-        n, plane, g = 0, None, None
-        for batch in batches:
-            x, labels, key = self._check(batch[0], batch[1])
-            if labels is None:
-                raise ValueError(f"{self.name}: every batch needs labels")
-            ids = batch[2] if len(batch) > 2 else None
-            N = x.shape[0]
+        seed = L.seed_bits(seed, self.name)
+        plane, g = None, None
+
+        def score(x, labels, ids, key):
+            nonlocal plane, g
             if plane is None:
                 plane = tuple(x.shape[1:])
                 g = self._grid(*plane[1:])
             elif tuple(x.shape[1:]) != plane:
                 raise ValueError(f"{self.name}: every batch of a call must be [N, {', '.join(map(str, plane))}], "
                                  f"got {tuple(x.shape)}")
-            if ids is not None and (not torch.is_tensor(ids) or ids.dtype != torch.int64 or ids.device != x.device
-                                    or ids.numel() != N):
-                raise ValueError(f"{self.name}: ids must be an int64 tensor of {N} entries on {x.device}")
-            st = self._graphs.get(key)
-            if st is None:
-                st = self._graphs[key] = self._state(x, key[1], g[2])
+            st = self._graphed(key, x, g[2])
             st.x.copy_(x)
             st.labels.copy_(labels)
-            if ids is None:
-                torch.arange(n, n + N, out=st.ids)
-            else:
-                st.ids.copy_(ids.reshape(-1))
+            st.ids.copy_(ids)
             st.eps.fill_(self.eps)
-            st.seed.fill_(seed - 2 ** 64 if seed >= 2 ** 63 else seed)        # the uint64's bits
+            st.seed.fill_(seed)
             st.prologue.replay()
             for _ in range(len(g[2])):
                 st.point.replay()
-            p.append(st.p.clone())
-            hit.append(st.hit.clone())
-            p_clean.append(st.p_clean.clone())
-            hit_clean.append(st.hit_clean.clone())
-            all_labels.append(labels)
-            n += N
-        if n == 0:
-            raise ValueError(f"{self.name}: no batches")
-        labels = torch.cat(all_labels)
-        F = len(g[2])
-        stats = torch.cat([torch.cat(hit, 1).double().mean(1), auc(torch.cat(p, 1), labels),
-                           torch.cat(hit_clean).double().mean()[None], auc(torch.cat(p_clean), labels)[None]]).cpu()
+            return torch.cat([st.p_clean[None], st.p]), torch.cat([st.hit_clean[None], st.hit])
+
+        (acc, auc), n = tally(self.name, self.model, batches, score)
         index = torch.tensor(g[3])
         H, W = plane[1:]
         return {"u": torch.tensor(g[0], dtype=torch.int64), "v": torch.tensor(g[1], dtype=torch.int64),
-                "acc": stats[:F][index], "auc": stats[F:2 * F][index],
-                "clean": {"acc": float(stats[2 * F]), "auc": float(stats[2 * F + 1]), "n": n},
+                "acc": acc[1:][index], "auc": auc[1:][index],
+                "clean": {"acc": float(acc[0]), "auc": float(auc[0]), "n": n},
                 "eps": self.eps, "peak": self.eps * math.sqrt(2.0 / (H * W))}

@@ -987,13 +987,8 @@ def corrupt(x, kind, param, ids=None, seed=0, lo=-1.0, hi=1.0):
     if x.dim() != 4 or x.shape[1] != 3:
         raise ValueError(f"corrupt: x must be [N, 3, H, W] RGB, got {tuple(x.shape)}")
     N, _, H, W = x.shape
-    if ids is not None:
-        if not ids.is_cuda or ids.device != x.device or ids.dtype != torch.int64 or ids.numel() != N:
-            raise ValueError(f"corrupt: ids must be an int64 tensor of {N} entries on {x.device}")
-        ids = ids.contiguous()
-    seed = int(seed)
-    if not 0 <= seed < 2 ** 64:
-        raise ValueError(f"corrupt: seed {seed} is not a uint64")
+    ids = L.require_ids(ids, x, "corrupt")
+    seed = L.seed_bits(seed, "corrupt")          # ctypes passes the int64's bits as the uint64 unchanged
     y = torch.empty_like(x)
     lib = L.lib()
     k = CORRUPT_KINDS[kind]
@@ -1048,8 +1043,7 @@ def attrib_step(x, baseline, g, acc, p, attr, amap, k, alpha, w, method, sigma=N
     if method == "smoothgrad":
         _device_scalar(sigma, torch.float32, "attrib_step", "sigma")
         _device_scalar(seed, torch.int64, "attrib_step", "seed")
-    if ids is not None and (not ids.is_cuda or ids.device != x.device or ids.dtype != torch.int64 or ids.numel() != N):
-        raise ValueError(f"attrib_step: ids must be an int64 tensor of {N} entries on {x.device}")
+    ids = L.require_ids(ids, x, "attrib_step")
     b, bval = _baseline_args(baseline, x, "attrib_step")
     L.check(L.lib().ud_attrib_step(L.ptr(x), L.ptr(b), bval, L.ptr(g), L.ptr(acc), L.ptr(p), L.ptr(attr), L.ptr(amap),
                                    L.ptr(k), L.ptr(alpha), L.ptr(w), L.ptr(sigma), L.ptr(ids), L.ptr(seed),
@@ -1108,9 +1102,7 @@ def fourier_perturb(x, y, freqs, f, eps, ids, seed, lo, hi):
     _device_scalar(f, torch.int32, "fourier_perturb", "f")
     _device_scalar(eps, torch.float32, "fourier_perturb", "eps")
     _device_scalar(seed, torch.int64, "fourier_perturb", "seed")
-    if ids is not None and (not ids.is_cuda or ids.device != x.device or ids.dtype != torch.int64 or ids.numel() != N
-                            or not ids.is_contiguous()):
-        raise ValueError(f"fourier_perturb: ids must be a contiguous int64 tensor of {N} entries on {x.device}")
+    ids = L.require_ids(ids, x, "fourier_perturb")
     L.check(L.lib().ud_fourier_perturb(L.ptr(x), L.ptr(y), L.ptr(freqs), freqs.shape[0], L.ptr(f), L.ptr(eps),
                                        L.ptr(ids), L.ptr(seed), float(lo), float(hi), N, C, H, W, L.stream()),
             "fourier_perturb")
